@@ -1,7 +1,7 @@
 #!/usr/bin/env python
-"""bench.py -- the hot path's headline benchmark (contract: see the task brief / DESIGN.md).
+"""bench.py -- the hot path's headline benchmark (see DESIGN.md).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 Workload at every N: BASELINE.json configs[1], "batched forward sweep: 1M random 10-layer
 models x 64 sources, fp64" PER GPU (weak scaling: the model axis is sharded, no data-path
@@ -24,6 +24,10 @@ of the hot path over that batch.
           all-gather of (logL, beta) over NCCL is inside the timed region), a config-5 slice per GPU
 
 --impl reference times that CPU oracle alone (rank 0 only).
+
+--dump-outputs DIR writes what the timed device-resident path returned in its last step (logL, one
+per model) as DIR/logL.npy (DIR/logL_rank<r>.npy on N > 1), float64; the inputs are seeded, so two
+builds run with the same arguments can be compared value for value.
 """
 import argparse
 import json
@@ -38,12 +42,14 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the tree as it found it (it may be read-only)
 
 METRIC = "model_source_travel_time_evals_per_s"
 UNIT = "evals/s"
 WORKLOAD = ("config2: batched forward sweep, 1M random 10-layer models x 64 sources per GPU, fp64, "
             "Gaussian logL fused (one logL per model)")
 FP64_PEAK_THEORY_TFLOPS = 37.2     # 148 SMs x 64 DFMA/clk x 2 flop x 1.965 GHz
+DUMP_BUDGET_BYTES = 64 << 20       # --dump-outputs, all ranks together
 
 
 def config_dict(B, S, layers):
@@ -71,7 +77,27 @@ def parse():
     ap.add_argument("--variant", type=int, default=-1, help="kernel variant (debug only)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (debug only)")
     ap.add_argument("--opt", action="append", default=[], help="library option name=value (debug only)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path (--impl ours)")
+    return args
+
+
+def dump_outputs(dirname, arrays, budget):
+    """Write each array as dirname/<name>.npy in float64.  Over `budget` bytes in all, each array is
+    cut to a fixed, seeded sample of its elements (in index order), the same from run to run."""
+    os.makedirs(dirname, exist_ok=True)
+    total = sum(a.size * 8 for a in arrays.values())
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float64).ravel()
+        if total > budget:
+            keep = a.size * budget // total
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 def workload(rank, models):
@@ -492,6 +518,10 @@ def main():
             import traceback
             traceback.print_exc()
             configs = {"error": f"{type(e).__name__}: {e}"}
+
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logL" if world == 1 else f"logL_rank{rank}": logL_resident},
+                     DUMP_BUDGET_BYTES // world)
 
     if rank == 0:
         evals_step = float(B) * S * world

@@ -13,6 +13,11 @@ from raytracerfortran_b200 import _lib, build, workloads
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
+def _cuobjdump():
+    # the toolkit that built the library, which need not be on PATH (build.nvcc_path falls back)
+    return os.path.join(os.path.dirname(build.nvcc_path()), "cuobjdump")
+
+
 @pytest.fixture(scope="module")
 def lib():
     build.build_library()
@@ -37,7 +42,7 @@ def test_header_and_exports_agree(lib):
 
 
 def test_library_is_sm100a_only(lib):
-    out = subprocess.run(["cuobjdump", "-lelf", _lib.LIB_PATH], capture_output=True, text=True).stdout
+    out = subprocess.run([_cuobjdump(), "-lelf", _lib.LIB_PATH], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_\d+a?", out))
     assert archs == {"sm_100a"}, archs
 
@@ -46,7 +51,7 @@ def test_kernels_stage_tiles_with_tma_bulk_copies(lib):
     """The batch kernels bring a tile's rows in with cp.async.bulk + mbarrier: the SASS carries
     UBLKCP (the bulk copy) and SYNCS (mbarrier arrive/wait), and fp64 math only (no tensor-core
     instructions: the path is not a contraction)."""
-    sass = subprocess.run(["cuobjdump", "-sass", _lib.LIB_PATH], capture_output=True, text=True).stdout
+    sass = subprocess.run([_cuobjdump(), "-sass", _lib.LIB_PATH], capture_output=True, text=True).stdout
     assert sass.count("UBLKCP") >= 3 and sass.count("SYNCS") >= 3          # one per kernel variant at least
     assert "DFMA" in sass and "MUFU.RSQ64H" in sass
     assert not re.search(r"\b(HMMA|IMMA|UTCHMMA|UTCMMA|HGMMA)\b", sass)
