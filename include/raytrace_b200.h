@@ -340,9 +340,9 @@ int         rtb200_init(int device);          /* optional; lazy init picks the d
 void        rtb200_shutdown(void);
 const char *rtb200_last_error(void);          /* "" when the last call succeeded               */
 int         rtb200_device_count(void);        /* 0 without a driver / device                   */
-/* options: "variant" (0 plain loops, 1 lane state machine, 3 deep-model kernel, 4 ray-queue kernel
- *          (experimental, up to 62 velocities per model), 5 variant 1 with one segment of the sorted
- *          ray list per warp; < 0 default: by shape -- 3 for deep models; for shallow ones 5 when
+/* options: "variant" (1 lane state machine, 3 deep-model kernel, 5 variant 1 with one segment of
+ *          the sorted ray list per warp; any other value >= 0 means 1;
+ *          < 0 default: by shape -- 3 for deep models; for shallow ones 5 when
  *          the batch is at least six tiles per resident CTA or a single wave of full tiles, 1 in
  *          between; rtb200_get_stat("variant") reports 9 for the one-model
  *          latency kernel),

@@ -21,10 +21,10 @@ rays = mism = batches = 0
 kinds = {}
 while time.time() - t0 < args.seconds:
     kind = ["shallow", "deep-critical", "ragged", "kmode", "one-model"][batches % 5]
-    # round 2: the batches rotate over the default choice (variant 1, 3 or 5 by shape), variant 5
-    # (one list segment per warp), the opt-in queue kernel (variant 4; deep models fall back to
-    # their own kernel) and variant 1; a kind of its own for the one-model latency kernel
-    rt.set_option("variant", [-1, 5, 4, 1][batches % 4])
+    # the batches rotate over the default choice (variant 1, 3 or 5 by shape), variant 5 (one list
+    # segment per warp), variant 3 (the deep-model kernel, on every depth) and variant 1; a kind of
+    # its own for the one-model latency kernel
+    rt.set_option("variant", [-1, 5, 3, 1][batches % 4])
     seed = int(rng.integers(1, 2**31))
     if kind == "shallow":
         L, S, B = int(rng.integers(1, 13)), int(rng.integers(8, 129)), 60000

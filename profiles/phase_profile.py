@@ -3,7 +3,7 @@
 
 Usage: phase_profile.py <ncu source csv> <nvdisasm --print-line-info listing> <mangled kernel>
 Phases are delimited by marker comments in rt_kernels.cu; inlined helpers (the fp64 primitives,
-sqrt_rsqrt, div_seeded, layer_pair_ffp, div_unchecked, eval_time) are reported by helper name."""
+sqrt_rsqrt, div_seeded, layer_pair_ffp, div_unchecked) are reported by helper name."""
 import csv, re, sys, collections
 src_csv, listing, kern = sys.argv[1:4]
 cu = open("/root/repo/raytracerfortran_b200/csrc/rt_kernels.cu").read().splitlines()
@@ -12,22 +12,20 @@ def find(pat, start=0):
         if pat in cu[i]: return i + 1
     raise SystemExit(f"marker not found: {pat}")
 kstart = find("rt_batch_kernel(const BatchArgs a")
-v4 = find("// ---- variant 4: the solve as level-synchronous", kstart)     # variant 4's block sits between variant 0 and 1
-v1 = find("constexpr bool kDeep = (VARIANT == 3);", v4)
+v1 = find("constexpr bool kDeep = (VARIANT == 3);", kstart)
 marks = [("kernel prologue", kstart), ("A stage+tables", find("// ---------------- A:", kstart)),
          ("B per-ray setup", find("// ---------------- B:", kstart)), ("sort", find("// ---------------- counting sort", kstart)),
-         ("C variant0", find("// ---------------- C: solve", kstart)), ("C variant4 (queues)", v4),
+         ("C setup", find("// ---------------- C: solve", kstart)),
          ("C refill", find("// ---- refill idle lanes", v1)),
          ("C eval loop ctl", find("// ---- f and f' at x", v1)), ("C transition", find("// ---- advance the ray", v1)),
          ("C' travel times", find("// ---- travel times at the final p", v1)), ("D outputs", find("// ---------------- D:", v1)),
          ("end", find("// \"next\" row N1: INTERPLAYER_novar", v1))]
 helpers = [("fp64 prims (dmul..dsqrt builtins)", find("double dmul(double a"), find("double dsqrt(double a") + 1),
-           ("eval_time/eval_ffp (builtin path)", find("struct Tables"), find("// rsqrt-seeded square root")),
            ("sqrt_rsqrt", find("double sqrt_rsqrt("), find("double div_seeded(")),
            ("div_seeded", find("double div_seeded("), find("// a / b by exactly")),
            ("div_unchecked", find("// a / b by exactly"), find("// 32-bit shared-memory addressing")),
-           ("lds/sts helpers", find("// 32-bit shared-memory addressing"), find("// Two consecutive layers")),
-           ("layer_pair_ffp", find("// Two consecutive layers"), find("// variant 0: the solver"))]
+           ("lds/sts helpers", find("// 32-bit shared-memory addressing"), find("// One solver pass evaluates")),
+           ("layer_pair_ffp", find("// One solver pass evaluates"), find("// variant 1: the solver"))]
 def phase_of(ln):
     if ln is None: return "?"
     for name, a, b in helpers:

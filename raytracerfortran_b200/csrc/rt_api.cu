@@ -31,10 +31,6 @@ constexpr double kPi = 3.141592653589793238462643383279502884197;  // data_type.
 constexpr int    kMaxChunks = 64;
 constexpr int    kSchedSlots = 256;  // tile-scheduler counter pairs, one per launch in flight
 constexpr int    kGraphSlots = 512;  // further pairs owned by the kernel nodes of a captured graph (two graphs)
-#ifndef RTB_SHALLOW_VARIANT
-#define RTB_SHALLOW_VARIANT 1
-#endif
-constexpr int    kShallowVariant = RTB_SHALLOW_VARIANT;   // kernel variant for models below kDeepLdv
 constexpr int    kDeepLdv = 40;     // models with this many velocities or more use the deep-model kernel
 
 struct DevBuf {
@@ -217,11 +213,11 @@ int *next_sched() {
 // Tile geometry for one launch (DESIGN.md "tiling").
 int choose_cfg(int B, int ldv, int ldz, int nsrc, bool aligned, TileCfg &c) {
     if (ldv > 255) return fail("more than 254 interfaces per model are not supported");
-    // variant: 0 plain loops; 1 lane state machine; 3 the same with branch-free, two-step-unrolled
-    // layer loops for deep models (more registers, 2 CTAs/SM); default: by depth
-    c.variant = g.opt_variant < 0 ? (ldv >= kDeepLdv ? 3 : kShallowVariant)
-                                  : (g.opt_variant >= 3 && g.opt_variant <= 5 ? g.opt_variant : (g.opt_variant ? 1 : 0));
-    if (c.variant == 4 && ldv > 62) c.variant = 1;      // variant 4 keeps the layer count in 6 bits
+    // variant: 1 lane state machine; 3 the same with branch-free, unrolled layer loops for deep
+    // models (more registers, 2 CTAs/SM); 5 is chosen below.  Default: by depth; the option forces
+    // 3 or 5, and any other value means 1
+    c.variant = g.opt_variant < 0 ? (ldv >= kDeepLdv ? 3 : 1)
+                                  : (g.opt_variant == 3 || g.opt_variant == 5 ? g.opt_variant : 1);
     c.threads = g.opt_threads > 0 ? std::min(256, (g.opt_threads + 31) / 32 * 32) : 256;
     c.LP = std::max(ldv, 2) | 1;
     c.SC = std::min(nsrc, g.opt_tile_sources > 0 ? g.opt_tile_sources : 256);
@@ -231,7 +227,7 @@ int choose_cfg(int B, int ldv, int ldz, int nsrc, bool aligned, TileCfg &c) {
     const int rays_target = c.threads * 8;
     int M = g.opt_tile_models > 0 ? g.opt_tile_models : std::max(2, rays_target / c.SC);
     M = g.opt_tile_models > 0 ? std::max(1, std::min(M, B)) : even_up(std::min(M, even_up(B)));
-    const int want_ctas = g.opt_ctas > 0 ? g.opt_ctas : (c.variant == 3 ? 2 : c.variant == 4 ? 4 : 3);
+    const int want_ctas = g.opt_ctas > 0 ? g.opt_ctas : (c.variant == 3 ? 2 : 3);
     const size_t budget  = (size_t)g.smem_optin;
     const size_t per_cta = std::min<size_t>(budget, (size_t)(227 * 1024) / want_ctas - 1024);
     for (;;) {

@@ -42,16 +42,6 @@ struct BatchArgs {
     int          *sched;
 };
 
-// Variant 4's shared-memory geometry, precomputed by the host (launch_batch) so that the kernel
-// reads every offset as a constant-bank operand: byte offsets from the dynamic smem base.
-struct QGeom {
-    uint32_t tab, src, T, q, st, ctr;    // tables, sources, travel-time slots, ray queues, ray state, counters
-    uint32_t rowB, lp8;                  // bytes per model row of the tables, per sub-table
-    uint32_t oHV, oZ, oVV, oIVM;         // sub-table offsets inside a model row
-    uint32_t oD;                         // source depths after the offsets
-    uint32_t qbytes;                     // bytes per queue buffer
-};
-
 // Tile geometry chosen by the host for one launch.
 struct TileCfg {
     int M;        // models per tile (even unless forced by the tile_models option)
@@ -60,16 +50,15 @@ struct TileCfg {
     int TS;       // row stride of the travel-time tile (odd)
     int threads;  // CTA size
     int grid;     // persistent CTAs
-    int variant;  // 0: plain per-thread loops, 1: lane state machine with refill, 3: the same for deep models,
-                  // 4: level-synchronous ray queues (opt-in), 5: variant 1 with one list segment per warp
+    int variant;  // 1: lane state machine with refill, 3: the same for deep models,
+                  // 5: variant 1 with one list segment per warp
     int use_tma;  // rows are 16-byte aligned: stage with cp.async.bulk
     int logl_shuffle;  // reduce the residuals with warp shuffles (tree order) instead of source order
     size_t smem;  // dynamic shared memory bytes
-    QGeom  q;     // filled in by launch_batch
-    double kc[6]; // the solver's constants (filled in by launch_batch).  Read only when the kernels are
-                  // built with -DRTB_CONST_BANK (constants as kernel parameters instead of immediates
-                  // built in registers on every pass: six LDC against ten moves, measured 0.8 % slower,
-                  // profiles/r02_phase_ab.txt), so the shipped kernels do not touch it
+    // Unused.  It keeps the batch kernel's parameter block at the 1200 bytes its register allocation
+    // was tuned with: 104 bytes smaller, ptxas allocates the kernels differently, and on a B200 at
+    // 1000 W config 2 took 9.127 ms against 9.044 and config 3 0.1360 ms against 0.1338.
+    double reserved[13];
 };
 
 // Prior and proposal scales of the fixed-dimension MH move (read_input.f90:207-214).

@@ -98,12 +98,13 @@ def test_readme_example(golden):
 
 
 # ---------------------------------------------------------------------------------------------
-# batched sweeps against the oracle, both kernel variants
+# batched sweeps against the oracle, every kernel variant.  The "variant" option forces 3 or 5;
+# every other value runs variant 1, so the sweeps below that also pass 0 and 4 check that too.
 # ---------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("variant", [0, 1, 3, 4, 5])
-@pytest.mark.parametrize("B,nlayers,nsrc,seed", [(1500, 10, 64, 2), (257, 4, 20, 11), (64, 29, 256, 3),
-                                                 (33, 1, 7, 5)])
-def test_dff_batch_bitexact(variant, B, nlayers, nsrc, seed):
+BATCH_SHAPES = [(1500, 10, 64, 2), (257, 4, 20, 11), (64, 29, 256, 3), (33, 1, 7, 5)]
+
+
+def _dff_batch_bitexact(variant, B, nlayers, nsrc, seed):
     rt.set_option("variant", variant)
     v, z, nl = workloads.make_models(B, nlayers, seed)
     so, sd = workloads.make_sources(nsrc, seed)
@@ -114,7 +115,21 @@ def test_dff_batch_bitexact(variant, B, nlayers, nsrc, seed):
     assert_bitexact(got["timeP"], ref["timeP"], "timeP")
     assert_bitexact(got["p"], ref["p"], "p")
     assert_logl_close(got["logL"], ref["logL"], nsrc, sigma)
+
+
+@pytest.mark.parametrize("variant", [1, 3, 5])
+@pytest.mark.parametrize("B,nlayers,nsrc,seed", BATCH_SHAPES)
+def test_dff_batch_bitexact(variant, B, nlayers, nsrc, seed):
+    _dff_batch_bitexact(variant, B, nlayers, nsrc, seed)
     assert rt.get_stat("variant") == variant
+
+
+@pytest.mark.parametrize("variant", [0, 2, 4])
+@pytest.mark.parametrize("B,nlayers,nsrc,seed", BATCH_SHAPES)
+def test_dff_batch_bitexact_other_variant_values(variant, B, nlayers, nsrc, seed):
+    """Option values other than 3 and 5 run variant 1, with the oracle's bits."""
+    _dff_batch_bitexact(variant, B, nlayers, nsrc, seed)
+    assert rt.get_stat("variant") == 1
 
 
 @pytest.mark.parametrize("variant", [0, 1, 3, 4, 5])
