@@ -113,6 +113,17 @@ void dff_batch_status_(const double *vels, const double *depths, const int *nlay
                        const double *sigma, double *logL, double *p_out, const int *want,
                        int *status);
 
+/* dff_batch and the gradient of its travel times in one call (host pointers, scalars by
+ * reference): the forward, then rtb200_dff_grad_device's vector-Jacobian product with weights
+ * w [B][NSrc].  gvels [B][ldv] and gdepths [B][ldz] receive sum_s w dT/dV and sum_s w dT/dz;
+ * timeP, p_out, dtdr and dtdd [B][NSrc] may each be NULL.  Returns 0, or a non-zero status
+ * (see rtb200_last_error()). */
+int dff_batch_grad(const double *vels, const double *depths, const int *nlayers,
+                   const int *B, const int *ldv, const int *ldz,
+                   const double *src_offset, const double *src_depth, const int *NSrc,
+                   const double *w, double *timeP, double *p_out,
+                   double *gvels, double *gdepths, double *dtdr, double *dtdd);
+
 /* LOGLHOOD / LOGLHOOD_RT (loglhood.f90:3-32,35-211) over B chain states, with the model
  * mapping of :127-146: state b has k[b] Voronoi nodes, vp[b][0..k-1] = voro(1:k,2),
  * ziface[b][0..k-2] = ziface(1:k-1); k == 1 becomes two equal velocities over one fake
@@ -158,6 +169,29 @@ int rtb200_dff_batch_device(const double *d_vels, const double *d_depths, const 
                             const double *d_src_offset, const double *d_src_depth, int NSrc,
                             double *d_timeP, const double *d_tobs, const double *d_sigma,
                             double *d_logL, double *d_p_out, int kmode, void *stream);
+
+/* Gradient of the travel times with respect to the layered model and the sources, as a
+ * vector-Jacobian product over B models x NSrc sources (DESIGN.md section 11).  Device pointers,
+ * model and source arrays as for rtb200_dff_batch_device (same kmode mapping), plus what that
+ * entry returned for them:
+ *   timeP, p   [B][NSrc]   the forward's travel times and ray parameters (d_timeP, d_p_out)
+ *   w          [B][NSrc]   weights, e.g. dL/dT of a loss L
+ * Out:
+ *   gvels      [B][ldv]    gvels[b][i]   = sum_s w[b][s] dT_bs/dV_i
+ *   gdepths    [B][ldz]    gdepths[b][j] = sum_s w[b][s] dT_bs/dz_j   (kmode: ziface)
+ *   dtdr, dtdd [B][NSrc]   or NULL: dT_bs/d(src_offset[s]), dT_bs/d(src_depth[s])
+ * The derivatives are those of the exact travel-time function at the returned p (Fermat:
+ * dT/dR = p); rays with timeP = -999 (not converged) contribute 0.  Columns past a model's layers
+ * are 0; at k = 1 both layers are vp(1) and the fake interface gets 0.  Each sum runs in source
+ * order without atomics, so the result is reproducible bit for bit.  Rows must hold nlayers[b]+1
+ * velocities and nlayers[b] interfaces, as for the forward.  Stream semantics of
+ * rtb200_dff_batch_device. */
+int rtb200_dff_grad_device(const double *d_vels, const double *d_depths, const int *d_nlayers,
+                           int B, int ldv, int ldz,
+                           const double *d_src_offset, const double *d_src_depth, int NSrc,
+                           const double *d_timeP, const double *d_p, const double *d_w,
+                           double *d_gvels, double *d_gdepths, double *d_dtdr, double *d_dtdd,
+                           int kmode, void *stream);
 
 /* One fixed-dimension Metropolis-Hastings move of B independent chains, entirely on the device:
  * PROPOSAL (prjmh_temper_rf.f90:1386-1447, ENOS = 0: Cauchy step on voro(ivo,iwhich), |.| for a

@@ -61,8 +61,8 @@ struct Ctx {
     cudaEvent_t  ev_h2d[kMaxChunks], ev_d2h[kMaxChunks], ev_k0[kMaxChunks], ev_k1[kMaxChunks];
     cudaEvent_t  ev_t0 = nullptr, ev_t1 = nullptr;
     DevBuf vels, depths, nl, off, dep, tobs, sigma, timeP, pout, logL, arena, voro, vsorted,
-        idxar, arparb, sched, mh_ll, mh_out, mh_kp, mh_lpr;
-    // The scratch buffers below (vels ... mh_lpr) are shared by every entry.  Entries that return
+        idxar, arparb, sched, mh_ll, mh_out, mh_kp, mh_lpr, gw, ggv, ggz, gdr, gdd;
+    // The scratch buffers below (vels ... gdd) are shared by every entry.  Entries that return
     // without synchronising (a caller stream was given) leave an event behind; any later entry that
     // uses the scratch from another stream first makes that stream wait for it.
     cudaEvent_t  ev_scratch = nullptr;
@@ -1017,6 +1017,143 @@ int rtb200_dff_batch_device(const double *d_vels, const double *d_depths, const 
 
 namespace {
 
+// The argument checks both gradient entries share (the shape rules of dff_batch).
+int check_grad_args(int ldv, int ldz, const void *vels, const void *nlayers, const void *off,
+                    const void *dep, int nsrc, const void *w, const void *gvels, const void *gdepths) {
+    if (ldv < 1) return fail("ldv must be >= 1");
+    if (ldv > 255) return fail("more than 254 interfaces per model are not supported");
+    if (!vels || !nlayers || !gvels || (ldz > 0 && !gdepths))
+        return fail("the gradient needs vels, nlayers, gvels and (ldz > 0) gdepths");
+    if (nsrc > 0 && (!off || !dep || !w)) return fail("the gradient needs src_offset, src_depth and w");
+    return 0;
+}
+
+rtb::GradArgs grad_args(const double *vels, const double *depths, const int *nlayers, int B, int ldv,
+                        int ldz, const double *off, const double *dep, int nsrc, const double *timeP,
+                        const double *p, const double *w, double *gvels, double *gdepths,
+                        double *dtdr, double *dtdd, int kmode) {
+    rtb::GradArgs a{};
+    a.vels = vels; a.depths = depths; a.nlayers = nlayers;
+    a.B = B; a.ldv = ldv; a.ldz = ldz; a.kmode = kmode;
+    a.src_offset = off; a.src_depth = dep; a.nsrc = nsrc;
+    a.timeP = timeP; a.p = p; a.w = w;
+    a.gvels = gvels; a.gdepths = gdepths; a.dtdr = dtdr; a.dtdd = dtdd;
+    return a;
+}
+
+}  // namespace
+
+int rtb200_dff_grad_device(const double *d_vels, const double *d_depths, const int *d_nlayers,
+                           int B, int ldv, int ldz, const double *d_src_offset,
+                           const double *d_src_depth, int NSrc, const double *d_timeP,
+                           const double *d_p, const double *d_w, double *d_gvels,
+                           double *d_gdepths, double *d_dtdr, double *d_dtdd, int kmode,
+                           void *stream) {
+    ApiLock api_lock_;
+    if (int rc = ensure_init()) return rc;
+    g.err.clear();
+    if (B <= 0) return 0;
+    ldz = std::max(ldz, 0);
+    NSrc = std::max(NSrc, 0);
+    if (int rc = check_grad_args(ldv, ldz, d_vels, d_nlayers, d_src_offset, d_src_depth, NSrc, d_w,
+                                 d_gvels, d_gdepths))
+        return rc;
+    if (NSrc > 0 && (!d_timeP || !d_p)) return fail("the gradient needs the forward's timeP and p");
+    cudaStream_t st = stream ? (cudaStream_t)stream : g.s_comp;
+    const rtb::GradArgs a = grad_args(d_vels, d_depths, d_nlayers, B, ldv, ldz, d_src_offset,
+                                      d_src_depth, NSrc, d_timeP, d_p, d_w, d_gvels, d_gdepths,
+                                      d_dtdr, d_dtdd, kmode);
+    CK(cudaEventRecord(g.ev_k0[0], st));
+    CK(rtb::launch_grad(a, st));
+    CK(cudaEventRecord(g.ev_k1[0], st));
+    g.launches++;
+    if (!stream) {
+        CK(cudaStreamSynchronize(st));
+        float ms = 0.f;
+        CK(cudaEventElapsedTime(&ms, g.ev_k0[0], g.ev_k1[0]));
+        g.kernel_ms = g.total_ms = ms;
+    }
+    return 0;
+}
+
+int dff_batch_grad(const double *vels, const double *depths, const int *nlayers, const int *B,
+                   const int *ldv, const int *ldz, const double *src_offset,
+                   const double *src_depth, const int *NSrc, const double *w, double *timeP,
+                   double *p_out, double *gvels, double *gdepths, double *dtdr, double *dtdd) {
+    ApiLock api_lock_;
+    if (int rc = ensure_init()) return rc;
+    g.err.clear();
+    g.kernel_ms = g.total_ms = 0.0;
+    const int nb = *B, lv = *ldv, lz = std::max(*ldz, 0), ns = std::max(*NSrc, 0);
+    if (nb <= 0) return 0;
+    if (int rc = check_grad_args(lv, lz, vels, nlayers, src_offset, src_depth, ns, w, gvels, gdepths))
+        return rc;
+    const size_t Bz = (size_t)nb, S = (size_t)ns;
+    TileCfg cfg{};
+    if (ns > 0)
+        if (int rc = choose_cfg(nb, lv, lz, ns, true, cfg)) return rc;
+    // copy in, forward, gradient, copy out; our buffers are padded to whole tiles as in run_host
+    const size_t M = ns > 0 ? (size_t)cfg.M : 1, Bpad = (Bz + M - 1) / M * M + M;
+    CK(g.vels.reserve(Bpad * lv * 8));
+    CK(g.depths.reserve(Bpad * std::max(lz, 1) * 8));
+    CK(g.nl.reserve(Bpad * 4));
+    CK(g.off.reserve(std::max<size_t>(S, 1) * 8));
+    CK(g.dep.reserve(std::max<size_t>(S, 1) * 8));
+    CK(g.timeP.reserve(std::max<size_t>(Bz * S, 1) * 8));
+    CK(g.pout.reserve(std::max<size_t>(Bz * S, 1) * 8));
+    CK(g.gw.reserve(std::max<size_t>(Bz * S, 1) * 8));
+    CK(g.ggv.reserve(Bz * lv * 8));
+    CK(g.ggz.reserve(std::max<size_t>(Bz * lz, 1) * 8));
+    if (dtdr) CK(g.gdr.reserve(std::max<size_t>(Bz * S, 1) * 8));
+    if (dtdd) CK(g.gdd.reserve(std::max<size_t>(Bz * S, 1) * 8));
+    cudaStream_t st = g.s_comp;
+    if (int rc = scratch_acquire(st)) return rc;
+    CK(cudaMemcpyAsync(g.vels.p, vels, Bz * lv * 8, cudaMemcpyHostToDevice, st));
+    if (lz > 0) CK(cudaMemcpyAsync(g.depths.p, depths, Bz * lz * 8, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(g.nl.p, nlayers, Bz * 4, cudaMemcpyHostToDevice, st));
+    if (ns > 0) {
+        CK(cudaMemcpyAsync(g.off.p, src_offset, S * 8, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(g.dep.p, src_depth, S * 8, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(g.gw.p, w, Bz * S * 8, cudaMemcpyHostToDevice, st));
+    }
+    CK(cudaEventRecord(g.ev_k0[0], st));
+    if (ns > 0) {
+        BatchArgs a{};
+        a.vels = g.vels.as<double>(); a.depths = g.depths.as<double>(); a.nlayers = g.nl.as<int>();
+        a.B = nb; a.ldv = lv; a.ldz = lz; a.kmode = 0;
+        a.src_offset = g.off.as<double>(); a.src_depth = g.dep.as<double>(); a.nsrc = ns;
+        a.timeP = g.timeP.as<double>(); a.p_out = g.pout.as<double>();
+        a.padded = 1;
+        a.sched = next_sched();
+        CK(rtb::launch_batch(a, cfg, st));
+        g.launches++;
+        g.last = cfg;
+    }
+    const rtb::GradArgs ga = grad_args(g.vels.as<double>(), g.depths.as<double>(), g.nl.as<int>(), nb, lv,
+                                       lz, g.off.as<double>(), g.dep.as<double>(), ns, g.timeP.as<double>(),
+                                       g.pout.as<double>(), g.gw.as<double>(), g.ggv.as<double>(),
+                                       g.ggz.as<double>(), dtdr ? g.gdr.as<double>() : nullptr,
+                                       dtdd ? g.gdd.as<double>() : nullptr, 0);
+    CK(rtb::launch_grad(ga, st));
+    CK(cudaEventRecord(g.ev_k1[0], st));
+    g.launches++;
+    CK(cudaMemcpyAsync(gvels, g.ggv.p, Bz * lv * 8, cudaMemcpyDeviceToHost, st));
+    if (lz > 0) CK(cudaMemcpyAsync(gdepths, g.ggz.p, Bz * lz * 8, cudaMemcpyDeviceToHost, st));
+    if (ns > 0) {
+        if (timeP) CK(cudaMemcpyAsync(timeP, g.timeP.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
+        if (p_out) CK(cudaMemcpyAsync(p_out, g.pout.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
+        if (dtdr) CK(cudaMemcpyAsync(dtdr, g.gdr.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
+        if (dtdd) CK(cudaMemcpyAsync(dtdd, g.gdd.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
+    }
+    CK(cudaStreamSynchronize(st));
+    if (int rc = scratch_release(st, true)) return rc;
+    float ms = 0.f;
+    if (cudaEventElapsedTime(&ms, g.ev_k0[0], g.ev_k1[0]) == cudaSuccess) g.kernel_ms = g.total_ms = ms;
+    return 0;
+}
+
+namespace {
+
 rtb::MhPrior make_prior(const double *prior, int enos = 0) {
     rtb::MhPrior pr;
     pr.enos = enos ? 1 : 0;
@@ -1581,7 +1718,8 @@ void rtb200_shutdown(void) {
     for (auto &e : g.ev_slot) { if (e) cudaEventDestroy(e); e = nullptr; }
     for (DevBuf *b : {&g.vels, &g.depths, &g.nl, &g.off, &g.dep, &g.tobs, &g.sigma,
                       &g.timeP, &g.pout, &g.logL, &g.arena, &g.voro, &g.vsorted, &g.idxar, &g.arparb,
-                      &g.sched, &g.mh_ll, &g.mh_out, &g.mh_kp, &g.mh_lpr})
+                      &g.sched, &g.mh_ll, &g.mh_out, &g.mh_kp, &g.mh_lpr, &g.gw, &g.ggv, &g.ggz,
+                      &g.gdr, &g.gdd})
         b->release();
     for (int i = 0; i < kMaxChunks; ++i) {
         cudaEventDestroy(g.ev_h2d[i]);

@@ -42,6 +42,26 @@ struct BatchArgs {
     int          *sched;
 };
 
+// One launch of the gradient kernel (the vector-Jacobian product of the travel times, DESIGN.md
+// section 11).  Every pointer is a device pointer; model and source arrays as in BatchArgs.
+struct GradArgs {
+    const double *vels;        // [B][ldv]
+    const double *depths;      // [B][ldz]
+    const int    *nlayers;     // [B]; kmode: node counts k
+    int           B, ldv, ldz;
+    int           kmode;
+    const double *src_offset;  // [nsrc]
+    const double *src_depth;   // [nsrc]
+    int           nsrc;
+    const double *timeP;       // [B][nsrc] the batch kernel's travel times
+    const double *p;           // [B][nsrc] and ray parameters
+    const double *w;           // [B][nsrc] weights of the product
+    double       *gvels;       // [B][ldv]  sum_s w dT/dV_i
+    double       *gdepths;     // [B][ldz]  sum_s w dT/dz_j
+    double       *dtdr;        // [B][nsrc] or null: dT/d(offset)
+    double       *dtdd;        // [B][nsrc] or null: dT/d(depth)
+};
+
 // Tile geometry chosen by the host for one launch.
 struct TileCfg {
     int M;        // models per tile (even unless forced by the tile_models option)
@@ -110,6 +130,7 @@ cudaError_t launch_mcmc_finish(unsigned long long *counter, const int *k, int *p
 
 size_t      tile_smem_bytes(const TileCfg &c, int ldv, int ldz);
 cudaError_t launch_batch(const BatchArgs &a, const TileCfg &c, cudaStream_t st);
+cudaError_t launch_grad(const GradArgs &a, cudaStream_t st);
 cudaError_t launch_prep_voro(const int *k, const double *voro, int B, int ldk, double *vels,
                              double *depths, double *sorted, cudaStream_t st);
 cudaError_t launch_propose_voro(const int *k, const double *voro, int B, int ldk, const int *ivo,

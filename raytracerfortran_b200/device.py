@@ -1,7 +1,8 @@
 """The ray-tracing path on tensors that already live in HBM.
 
 torch is used for device memory and streams only; the work is done by the sm_100a kernels in
-libraytrace_b200.so through rtb200_dff_batch_device (include/raytrace_b200.h).
+libraytrace_b200.so through rtb200_dff_batch_device and, for gradients, rtb200_dff_grad_device
+(include/raytrace_b200.h).
 """
 import torch
 
@@ -62,3 +63,59 @@ def _legacy_stream_handle():
     # torch's default stream is the legacy stream (handle 0).  The C ABI reads NULL as "use the
     # library's own stream and synchronise", so name the legacy stream explicitly instead.
     return 1  # cudaStreamLegacy
+
+
+def _check_grad_shapes(vels, depths, nlayers, src_offset, src_depth, per_ray):
+    """Shapes of a gradient call, checked before anything touches the GPU.  Returns (B, ldv, ldz, S)."""
+    if vels.dim() != 2 or depths.dim() != 2 or vels.shape[0] != depths.shape[0]:
+        raise ValueError("vels and depths must be [B, ldv] and [B, ldz]")
+    B, ldv = vels.shape
+    ldz = depths.shape[1]
+    if not 1 <= ldv <= 255:
+        raise ValueError("ldv must be 1..255 (at most 254 interfaces)")
+    if nlayers.dim() != 1 or nlayers.shape[0] != B:
+        raise ValueError("nlayers must be [B]")
+    if src_offset.dim() != 1 or src_depth.shape != src_offset.shape:
+        raise ValueError("src_offset and src_depth must both be [NSrc]")
+    S = src_offset.shape[0]
+    for name, t in per_ray.items():
+        if t is not None and tuple(t.shape) != (B, S):
+            raise ValueError(f"{name} must be [B, NSrc] = [{B}, {S}], got {list(t.shape)}")
+    return B, ldv, ldz, S
+
+
+def dff_grad_device(vels, depths, nlayers, src_offset, src_depth, timeP, p, w, gvels=None,
+                    gdepths=None, want_src=False, dtdr=None, dtdd=None, kmode=False, stream=None):
+    """Vector-Jacobian product of the travel times dff_batch_device returned (timeP, p [B, NSrc])
+    with weights w [B, NSrc], on the GPU (rtb200_dff_grad_device; DESIGN.md section 11).
+
+    Returns {"gvels" [B, ldv], "gdepths" [B, ldz], "dtdr", "dtdd" [B, NSrc] or None}:
+    gvels[b, i] = sum_s w[b, s] dT[b, s]/dV_i, gdepths likewise for the interfaces (kmode: ziface),
+    dtdr / dtdd the per-ray derivatives with respect to the source offset and depth (want_src).
+    Asynchronous on `stream` (default: torch's current stream)."""
+    B, ldv, ldz, S = _check_grad_shapes(vels, depths, nlayers, src_offset, src_depth,
+                                        {"timeP": timeP, "p": p, "w": w, "dtdr": dtdr, "dtdd": dtdd})
+    for name, t, shape in (("gvels", gvels, (B, ldv)), ("gdepths", gdepths, (B, ldz))):
+        if t is not None and tuple(t.shape) != shape:
+            raise ValueError(f"{name} must be {list(shape)}, got {list(t.shape)}")
+    if not vels.is_cuda:
+        raise ValueError("dff_grad_device needs CUDA tensors (there is no CPU path)")
+    dev = vels.device
+    _ensure_device(dev.index if dev.index is not None else torch.cuda.current_device())
+    f64 = torch.float64
+    if gvels is None:
+        gvels = torch.empty((B, ldv), dtype=f64, device=dev)
+    if gdepths is None:
+        gdepths = torch.empty((B, ldz), dtype=f64, device=dev)
+    if want_src and dtdr is None:
+        dtdr = torch.empty((B, S), dtype=f64, device=dev)
+    if want_src and dtdd is None:
+        dtdd = torch.empty((B, S), dtype=f64, device=dev)
+    st = stream if stream is not None else torch.cuda.current_stream(dev)
+    rc = _lib.load().rtb200_dff_grad_device(
+        _ptr(vels, f64), _ptr(depths, f64) if ldz else None, _ptr(nlayers, torch.int32), B, ldv, ldz,
+        _ptr(src_offset, f64), _ptr(src_depth, f64), S, _ptr(timeP, f64), _ptr(p, f64), _ptr(w, f64),
+        _ptr(gvels, f64), _ptr(gdepths, f64) if ldz else None, _ptr(dtdr, f64), _ptr(dtdd, f64),
+        1 if kmode else 0, st.cuda_stream if st.cuda_stream != 0 else _legacy_stream_handle())
+    _lib.check(rc)
+    return {"gvels": gvels, "gdepths": gdepths, "dtdr": dtdr, "dtdd": dtdd}

@@ -107,6 +107,42 @@ def dff_batch(vels, depths, nlayers, src_offset, src_depth, tobs=None, sigma=Non
     return {"timeP": t, "p": p, "logL": ll}
 
 
+def dff_batch_grad(vels, depths, nlayers, src_offset, src_depth, w, want_times=False, want_p=False,
+                   want_src=False):
+    """dff_batch and the gradient of its travel times in one call (DESIGN.md section 11).
+
+    w [B, NSrc] weights the rays.  Returns a dict with "gvels" [B, ldv] = sum_s w dT/dV,
+    "gdepths" [B, ldz] = sum_s w dT/dz, and, on request, "timeP" / "p" [B, NSrc] of the forward
+    and "dtdr" / "dtdd" [B, NSrc], the per-ray derivatives with respect to the source offset and
+    depth (None otherwise)."""
+    v = _d(vels)
+    z = _d(depths)
+    if v.ndim != 2 or z.ndim != 2 or v.shape[0] != z.shape[0]:
+        raise ValueError("vels and depths must be [B, ldv] and [B, ldz]")
+    nl = np.ascontiguousarray(nlayers, dtype=np.int32)
+    so, sd = _d(src_offset), _d(src_depth)
+    B, ldv, ldz, nsrc = v.shape[0], v.shape[1], z.shape[1], so.size
+    if nl.shape != (B,) or so.ndim != 1 or sd.shape != so.shape:
+        raise ValueError("nlayers must be [B], src_offset and src_depth [NSrc]")
+    if not 1 <= ldv <= 255:
+        raise ValueError("ldv must be 1..255 (at most 254 interfaces)")
+    if B and (nl.min() < 0 or int(nl.max()) + 1 > ldv or int(nl.max()) > ldz):
+        raise ValueError("nlayers exceeds the row length of vels / depths")
+    ww = _d(w)
+    if ww.shape != (B, nsrc):
+        raise ValueError(f"w must be [B, NSrc] = [{B}, {nsrc}], got {list(ww.shape)}")
+    gv, gz = np.empty((B, ldv)), np.empty((B, ldz))
+    t = np.empty((B, nsrc)) if want_times else None
+    p = np.empty((B, nsrc)) if want_p else None
+    dr = np.empty((B, nsrc)) if want_src else None
+    dd = np.empty((B, nsrc)) if want_src else None
+    rc = _lib.load().dff_batch_grad(_p(v), _p(z), nl.ctypes.data_as(_IP), _ci(B), _ci(ldv), _ci(ldz),
+                                    _p(so), _p(sd), _ci(nsrc), _p(ww), _p(t), _p(p), _p(gv), _p(gz),
+                                    _p(dr), _p(dd))
+    _lib.check(rc)
+    return {"gvels": gv, "gdepths": gz, "timeP": t, "p": p, "dtdr": dr, "dtdd": dd}
+
+
 def loglhood_batch(k, voro_vp, ziface, src_offset, src_depth, DobsRT, sdparRT, want_pred=False):
     """LOGLHOOD / LOGLHOOD_RT (loglhood.f90:3-32,35-211) over B chain states.
 
