@@ -235,7 +235,8 @@ int rtb200_mh_step_device_ev(const int *d_k, double *d_voro, double *d_logL, int
 /* n_moves consecutive calls of rtb200_mh_step_device in one: move m uses row m of d_ivo, d_iwhich,
  * d_cauchy, d_uacc and writes row m of d_accept (all [n_moves][B]).  The run is captured once into
  * a CUDA graph and replayed for as long as the caller passes the same buffers and sizes (refill
- * them in place), which removes the launch gaps between the three kernels of every move.
+ * them in place) and the options stay as they were, which removes the launch gaps between the
+ * three kernels of every move; a changed option or tile geometry takes effect on the next call.
  * n_moves <= 512. */
 int rtb200_mh_moves_device(const int *d_k, double *d_voro, double *d_logL, int B, int ldk,
                            int n_moves, const int *d_ivo, const int *d_iwhich,

@@ -17,7 +17,36 @@ import numpy as np
 import torch
 
 from . import _lib
-from .device import _ensure_device, _legacy_stream_handle, _ptr
+from .device import _ensure_device, _ptr, _stream_handle
+
+
+def _move_prologue(name, voro, stream=None, accept=False):
+    """The start every chain-move wrapper shares: voro [B, 2, ldk] a CUDA tensor, the library
+    initialised on its device, and the C ABI's handle of `stream` (default: torch's current stream).
+    `accept` is the caller's [B] i32 output of a single move, None to allocate one; the wrappers that
+    have no such output leave it False.  Returns (dev, B, ldk, stream handle, accept)."""
+    if not voro.is_cuda:
+        raise ValueError(f"{name} needs CUDA tensors (there is no CPU path)")
+    dev = voro.device
+    _ensure_device(dev.index if dev.index is not None else torch.cuda.current_device())
+    B, two, ldk = voro.shape
+    if two != 2:
+        raise ValueError("voro must be [B, 2, ldk]")
+    if accept is None:
+        accept = torch.empty((B,), dtype=torch.int32, device=dev)
+    return dev, B, ldk, _stream_handle(stream, dev), accept
+
+
+def _host_doubles(a, n, message):
+    """A host array of exactly n doubles, contiguous for the C ABI."""
+    arr = np.ascontiguousarray(a, dtype=np.float64)
+    if arr.size != n:
+        raise ValueError(message)
+    return arr
+
+
+_PRIOR_SIZE = "prior must hold 7 doubles (see prior_array)"
+_AR_PRIOR_SIZE = "ar_prior must hold 4 doubles (see ar_prior_array)"
 
 
 def prior_array(hmin=100.1, hmx=10000.1, vmin=1500.0, vmax=10000.0, pertsdsc=30.0, fact=1.0,
@@ -59,26 +88,14 @@ def mh_step_device(k, voro, logL, ivo, iwhich, cauchy, u_acc, beta, sigma, prior
     order statistics prior, PROPOSAL :1418-1431): a depth move then takes the uniform itself in
     `cauchy` (see `move_deviates`).  Returns accept [B] i32: 1 accepted, 0 rejected, -1 outside
     the bounds."""
-    if not voro.is_cuda:
-        raise ValueError("mh_step_device needs CUDA tensors (there is no CPU path)")
-    dev = voro.device
-    _ensure_device(dev.index if dev.index is not None else torch.cuda.current_device())
-    B, two, ldk = voro.shape
-    if two != 2:
-        raise ValueError("voro must be [B, 2, ldk]")
+    _, B, ldk, st, accept = _move_prologue("mh_step_device", voro, stream, accept)
+    pr = _host_doubles(prior, 7, _PRIOR_SIZE)
     f64, i32 = torch.float64, torch.int32
-    if accept is None:
-        accept = torch.empty((B,), dtype=i32, device=dev)
-    pr = np.ascontiguousarray(prior, dtype=np.float64)
-    if pr.size != 7:
-        raise ValueError("prior must hold 7 doubles (see prior_array)")
-    st = stream if stream is not None else torch.cuda.current_stream(dev)
     rc = _lib.load().rtb200_mh_step_device_ev(
         _ptr(k, i32), _ptr(voro, f64), _ptr(logL, f64), B, ldk, _ptr(ivo, i32), _ptr(iwhich, i32),
         _ptr(cauchy, f64), _ptr(u_acc, f64), _ptr(beta, f64), _ptr(sigma, f64),
         pr.ctypes.data_as(C.POINTER(C.c_double)), _ptr(src_offset, f64), _ptr(src_depth, f64),
-        _ptr(tobs, f64), src_offset.numel(), _ptr(accept, i32),
-        st.cuda_stream if st.cuda_stream != 0 else _legacy_stream_handle(),
+        _ptr(tobs, f64), src_offset.numel(), _ptr(accept, i32), st,
         beta_ready.cuda_event if beta_ready is not None else None, 1 if enos else 0)
     _lib.check(rc)
     return accept
@@ -98,19 +115,9 @@ def bd_step_device(k, voro, logL, u_k, idel, u_z, u_v, u_acc, beta, sigma, prior
     """The birth/death move of every chain (rtb200_bd_step_device), in place on k, voro, logL.
     u_k/u_z/u_v/u_acc [B] f64 uniforms, idel [B] i32 (node a death removes, 2..k), pk: host array
     (poisson_pk) or None.  Returns accept [B] i32: 1 / 0 / -1 outside / 2 no move proposed."""
-    if not voro.is_cuda:
-        raise ValueError("bd_step_device needs CUDA tensors (there is no CPU path)")
-    dev = voro.device
-    _ensure_device(dev.index if dev.index is not None else torch.cuda.current_device())
-    B, two, ldk = voro.shape
-    if two != 2:
-        raise ValueError("voro must be [B, 2, ldk]")
+    _, B, ldk, st, accept = _move_prologue("bd_step_device", voro, stream, accept)
+    pr = _host_doubles(prior, 7, _PRIOR_SIZE)
     f64, i32 = torch.float64, torch.int32
-    if accept is None:
-        accept = torch.empty((B,), dtype=i32, device=dev)
-    pr = np.ascontiguousarray(prior, dtype=np.float64)
-    if pr.size != 7:
-        raise ValueError("prior must hold 7 doubles (see prior_array)")
     dp = C.POINTER(C.c_double)
     pkp = None
     if pk is not None:
@@ -118,13 +125,11 @@ def bd_step_device(k, voro, logL, u_k, idel, u_z, u_v, u_acc, beta, sigma, prior
         if pka.size < kmax:
             raise ValueError("pk must hold kmax values")
         pkp = pka.ctypes.data_as(dp)
-    st = stream if stream is not None else torch.cuda.current_stream(dev)
     rc = _lib.load().rtb200_bd_step_device_ex(
         _ptr(k, i32), _ptr(voro, f64), _ptr(logL, f64), B, ldk, _ptr(u_k, f64), _ptr(idel, i32),
         _ptr(u_z, f64), _ptr(u_v, f64), _ptr(u_acc, f64), _ptr(beta, f64), _ptr(sigma, f64),
         pr.ctypes.data_as(dp), pkp, int(kmin), int(kmax), _ptr(src_offset, f64),
-        _ptr(src_depth, f64), _ptr(tobs, f64), src_offset.numel(), _ptr(accept, i32),
-        st.cuda_stream if st.cuda_stream != 0 else _legacy_stream_handle(), 1 if enos else 0)
+        _ptr(src_depth, f64), _ptr(tobs, f64), src_offset.numel(), _ptr(accept, i32), st, 1 if enos else 0)
     _lib.check(rc)
     return accept
 
@@ -140,23 +145,13 @@ def sd_step_device(k, voro, logL, sigma, u_gate, gauss, u_acc, beta, sd_prior, s
                    tobs, accept=None, stream=None):
     """The data-error move of every chain (rtb200_sd_step_device), in place on sigma and logL.
     Returns accept [B] i32: 1 / 0 / -1 outside / 2 no move proposed."""
-    if not voro.is_cuda:
-        raise ValueError("sd_step_device needs CUDA tensors (there is no CPU path)")
-    dev = voro.device
-    _ensure_device(dev.index if dev.index is not None else torch.cuda.current_device())
-    B, two, ldk = voro.shape
+    _, B, ldk, st, accept = _move_prologue("sd_step_device", voro, stream, accept)
+    sp = _host_doubles(sd_prior, 3, "sd_prior must hold 3 doubles (see sd_prior_array)")
     f64, i32 = torch.float64, torch.int32
-    if accept is None:
-        accept = torch.empty((B,), dtype=i32, device=dev)
-    sp = np.ascontiguousarray(sd_prior, dtype=np.float64)
-    if sp.size != 3:
-        raise ValueError("sd_prior must hold 3 doubles (see sd_prior_array)")
-    st = stream if stream is not None else torch.cuda.current_stream(dev)
     rc = _lib.load().rtb200_sd_step_device(
         _ptr(k, i32), _ptr(voro, f64), _ptr(logL, f64), _ptr(sigma, f64), B, ldk, _ptr(u_gate, f64),
         _ptr(gauss, f64), _ptr(u_acc, f64), _ptr(beta, f64), sp.ctypes.data_as(C.POINTER(C.c_double)),
-        _ptr(src_offset, f64), _ptr(src_depth, f64), _ptr(tobs, f64), src_offset.numel(),
-        _ptr(accept, i32), st.cuda_stream if st.cuda_stream != 0 else _legacy_stream_handle())
+        _ptr(src_offset, f64), _ptr(src_depth, f64), _ptr(tobs, f64), src_offset.numel(), _ptr(accept, i32), st)
     _lib.check(rc)
     return accept
 
@@ -182,24 +177,14 @@ def ar_step_device(k, voro, logL, sigma, idxar, arpar, u_choice, u_prop, gauss, 
                    src_offset, src_depth, tobs, accept=None, stream=None):
     """The AR(1) move of every chain (rtb200_ar_step_device, IAR = 1), in place on idxar [B] i32,
     arpar [B] f64 and logL.  Returns accept [B] i32: 1 / 0 / -1 outside."""
-    if not voro.is_cuda:
-        raise ValueError("ar_step_device needs CUDA tensors (there is no CPU path)")
-    dev = voro.device
-    _ensure_device(dev.index if dev.index is not None else torch.cuda.current_device())
-    B, two, ldk = voro.shape
+    _, B, ldk, st, accept = _move_prologue("ar_step_device", voro, stream, accept)
+    ap = _host_doubles(ar_prior, 4, _AR_PRIOR_SIZE)
     f64, i32 = torch.float64, torch.int32
-    if accept is None:
-        accept = torch.empty((B,), dtype=i32, device=dev)
-    ap = np.ascontiguousarray(ar_prior, dtype=np.float64)
-    if ap.size != 4:
-        raise ValueError("ar_prior must hold 4 doubles (see ar_prior_array)")
-    st = stream if stream is not None else torch.cuda.current_stream(dev)
     rc = _lib.load().rtb200_ar_step_device(
         _ptr(k, i32), _ptr(voro, f64), _ptr(logL, f64), _ptr(sigma, f64), _ptr(idxar, i32),
         _ptr(arpar, f64), B, ldk, _ptr(u_choice, f64), _ptr(u_prop, f64), _ptr(gauss, f64),
         _ptr(u_acc, f64), _ptr(beta, f64), ap.ctypes.data_as(C.POINTER(C.c_double)),
-        _ptr(src_offset, f64), _ptr(src_depth, f64), _ptr(tobs, f64), src_offset.numel(),
-        _ptr(accept, i32), st.cuda_stream if st.cuda_stream != 0 else _legacy_stream_handle())
+        _ptr(src_offset, f64), _ptr(src_depth, f64), _ptr(tobs, f64), src_offset.numel(), _ptr(accept, i32), st)
     _lib.check(rc)
     return accept
 
@@ -242,9 +227,8 @@ def mh_moves_device(k, voro, logL, pos, n_moves, beta, sigma, prior, src_offset,
     advanced in place.  The schedule and all random numbers are generated up front into buffers
     that persist between calls, and the run of moves goes to rtb200_mh_moves_device, which replays
     it as one CUDA graph.  Returns the number of accepted moves per chain [B]."""
-    dev = voro.device
-    _ensure_device(dev.index if dev.index is not None else torch.cuda.current_device())
-    B, two, ldk = voro.shape
+    dev, B, ldk, st, _ = _move_prologue("mh_moves_device", voro)
+    pr = _host_doubles(prior, 7, _PRIOR_SIZE)
     f64, i32 = torch.float64, torch.int32
     key = (dev, B, int(n_moves))
     buf = _moves_buffers.get(key)
@@ -265,16 +249,12 @@ def mh_moves_device(k, voro, logL, pos, n_moves, beta, sigma, prior, src_offset,
     torch.tan(math.pi * (buf["u"][0] - 0.5), out=buf["cauchy"])
     if enos:
         buf["cauchy"].copy_(torch.where(buf["iwhich"] == 1, buf["u"][0], buf["cauchy"]))
-    pr = np.ascontiguousarray(prior, dtype=np.float64)
-    if pr.size != 7:
-        raise ValueError("prior must hold 7 doubles (see prior_array)")
-    st = torch.cuda.current_stream(dev)
     rc = _lib.load().rtb200_mh_moves_device_ex(
         _ptr(k, i32), _ptr(voro, f64), _ptr(logL, f64), B, ldk, int(n_moves), _ptr(buf["ivo"], i32),
         _ptr(buf["iwhich"], i32), _ptr(buf["cauchy"], f64), _ptr(buf["u"][1], f64), _ptr(beta, f64),
         _ptr(sigma, f64), pr.ctypes.data_as(C.POINTER(C.c_double)), _ptr(src_offset, f64),
-        _ptr(src_depth, f64), _ptr(tobs, f64), src_offset.numel(), _ptr(buf["accept"], i32),
-        st.cuda_stream if st.cuda_stream != 0 else _legacy_stream_handle(), 1 if enos else 0)
+        _ptr(src_depth, f64), _ptr(tobs, f64), src_offset.numel(), _ptr(buf["accept"], i32), st,
+        1 if enos else 0)
     _lib.check(rc)
     pos.copy_(((pos.to(torch.int64) + n_moves) % period).to(i32))
     return (buf["accept"] == 1).sum(dim=0)
@@ -370,17 +350,13 @@ class McmcGraph:
 
     def __init__(self, k, voro, logL, sigma, beta, n_moves, prior, sd_prior, pk, kmin, kmax,
                  src_offset, src_depth, tobs, seed=1, enos=False, counter0=0, ar=None):
-        dev = voro.device
-        _ensure_device(dev.index if dev.index is not None else torch.cuda.current_device())
+        dev, self.B, self.ldk, _, _ = _move_prologue("McmcGraph", voro)
         self.k, self.voro, self.logL, self.sigma, self.beta = k, voro, logL, sigma, beta
         self.src = (src_offset, src_depth, tobs)
-        self.B, _, self.ldk = voro.shape
         self.M = int(n_moves)
-        self.prior = np.ascontiguousarray(prior, dtype=np.float64)
-        self.sd_prior = np.ascontiguousarray(sd_prior, dtype=np.float64)
+        both = "prior must hold 7 doubles and sd_prior 3 (prior_array, sd_prior_array)"
+        self.prior, self.sd_prior = _host_doubles(prior, 7, both), _host_doubles(sd_prior, 3, both)
         self.pk = None if pk is None else np.ascontiguousarray(pk, dtype=np.float64)
-        if self.prior.size != 7 or self.sd_prior.size != 3:
-            raise ValueError("prior must hold 7 doubles and sd_prior 3 (prior_array, sd_prior_array)")
         if self.pk is not None and self.pk.size < kmax:
             raise ValueError("pk must hold kmax values")
         self.kmin, self.kmax, self.seed, self.enos = int(kmin), int(kmax), int(seed), bool(enos)
@@ -391,18 +367,12 @@ class McmcGraph:
         self.tally = torch.zeros((5, self.B), dtype=torch.int64, device=dev)
         # IAR = 1: ar = (idxar [B] i32, arpar [B] f64, ar_prior (ar_prior_array)); the iteration then
         # ends with the AR(1) move and every likelihood uses the chains' AR state
-        self.ar = None
-        if ar is not None:
-            ap = np.ascontiguousarray(ar[2], dtype=np.float64)
-            if ap.size != 4:
-                raise ValueError("ar_prior must hold 4 doubles (see ar_prior_array)")
-            self.ar = (ar[0], ar[1], ap)
+        self.ar = None if ar is None else (ar[0], ar[1], _host_doubles(ar[2], 4, _AR_PRIOR_SIZE))
         self.views = mcmc_workspace_views(self.workspace, self.B, self.M)
 
     def run(self, n_iterations=1, stream=None):
         f64, i32 = torch.float64, torch.int32
         dp = C.POINTER(C.c_double)
-        st = stream if stream is not None else torch.cuda.current_stream(self.voro.device)
         so, sd, ob = self.src
         rc = _lib.load().rtb200_mcmc_iterations_device(
             _ptr(self.k, i32), _ptr(self.voro, f64), _ptr(self.logL, f64), _ptr(self.sigma, f64),
@@ -414,6 +384,5 @@ class McmcGraph:
             self.tally.data_ptr(), int(n_iterations),
             None if self.ar is None else _ptr(self.ar[0], i32),
             None if self.ar is None else _ptr(self.ar[1], f64),
-            None if self.ar is None else self.ar[2].ctypes.data_as(dp),
-            st.cuda_stream if st.cuda_stream != 0 else _legacy_stream_handle())
+            None if self.ar is None else self.ar[2].ctypes.data_as(dp), _stream_handle(stream, self.voro.device))
         _lib.check(rc)

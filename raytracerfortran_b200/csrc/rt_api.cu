@@ -17,6 +17,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <vector>
 #if defined(__x86_64__)
 #include <emmintrin.h>
@@ -54,6 +55,17 @@ struct DevBuf {
     template <class T> T *as() const { return static_cast<T *>(p); }
 };
 
+// A captured CUDA graph and the key of everything its capture baked in.
+struct GraphCache {
+    cudaGraphExec_t     exec = nullptr;
+    std::vector<size_t> key;
+    void reset() {
+        if (exec) cudaGraphExecDestroy(exec);
+        exec = nullptr;
+        key.clear();
+    }
+};
+
 struct Ctx {
     bool inited = false, ok = false;
     int  device = 0, sms = 0, smem_optin = 0;
@@ -70,13 +82,9 @@ struct Ctx {
     bool         scratch_pending = false;
     unsigned sched_seq = 0;        // launches take scheduler slots round robin
     bool     sched_dirty = false;  // a CUDA call failed: a kernel may have left counters behind
-    // one cached CUDA graph of a run of MH moves (rtb200_mh_moves_device)
-    cudaGraphExec_t     mv_exec = nullptr;
-    std::vector<size_t> mv_key;
-    // one cached CUDA graph of a whole MCMC iteration (rtb200_mcmc_iterations_device)
-    cudaGraphExec_t     mc_exec = nullptr;
-    std::vector<size_t> mc_key;
-    cudaStream_t        s_cap = nullptr;
+    GraphCache   mv;               // a run of MH moves (rtb200_mh_moves_device)
+    GraphCache   mc;               // a whole MCMC iteration (rtb200_mcmc_iterations_device)
+    cudaStream_t s_cap = nullptr;
     // IAR = 1: the chains' AR(1) state, used by every likelihood evaluation of the move entries
     const int    *chain_idxar = nullptr;
     const double *chain_arpar = nullptr;
@@ -1152,6 +1160,7 @@ int dff_batch_grad(const double *vels, const double *depths, const int *nlayers,
     return 0;
 }
 
+extern "C++" {   // the helpers below include templates
 namespace {
 
 rtb::MhPrior make_prior(const double *prior, int enos = 0) {
@@ -1164,31 +1173,89 @@ rtb::MhPrior make_prior(const double *prior, int enos = 0) {
     return pr;
 }
 
-// Scratch of a chain move: the proposal as (vp, ziface) rows for the batch kernel, its node count,
-// its sorted nodes, its logL and the outside / no-move code.
-int reserve_move_scratch(int B, int ldk, const TileCfg &cfg) {
-    const size_t Bz = (size_t)B, Bpad = (Bz + cfg.M - 1) / cfg.M * cfg.M + cfg.M;
-    CK(g.vels.reserve(Bpad * ldk * 8));
-    CK(g.depths.reserve(Bpad * ldk * 8));
+rtb::BdPrior make_bd_prior(const double *pk, int kmin, int kmax) {
+    rtb::BdPrior bd{};
+    bd.kmin = kmin; bd.kmax = kmax; bd.use_pk = pk ? 1 : 0;
+    for (int i = kmin; pk && i <= kmax; ++i) bd.logpk[i - 1] = std::log(pk[i - 1]);   // LOG(pk(i)), libm
+    return bd;
+}
+
+// What every chain move reads: the chains' state (k [B], voro [B][2][ldk], logL, sigma, beta [B]),
+// the data and the likelihood's tile geometry.  The entries' const qualifiers say which state they
+// leave alone; one struct serves every move.
+struct MoveCtx {
+    int          *k;
+    double       *voro, *logL, *sigma;
+    const double *beta;
+    int           B, ldk;
+    const double *src_offset, *src_depth, *tobs;
+    int           NSrc;
+    TileCfg       cfg;
+};
+
+MoveCtx move_ctx(const int *k, const double *voro, double *logL, const double *sigma, const double *beta,
+                 int B, int ldk, const double *src_offset, const double *src_depth, const double *tobs,
+                 int NSrc) {
+    return {const_cast<int *>(k), const_cast<double *>(voro), logL, const_cast<double *>(sigma), beta, B,
+            ldk, src_offset, src_depth, tobs, NSrc, TileCfg{}};
+}
+
+// The argument checks every chain-move entry makes; `name` starts the refusal.
+int check_move_args(const char *name, int NSrc, int ldk) {
+    if (NSrc <= 0) return fail(std::string(name) + " needs at least one source");
+    if (ldk < 1 || ldk > 64) return fail(std::string(name) + " supports 1..64 nodes per state");
+    return 0;
+}
+
+// The start every chain-move entry shares after its checks: the stream (the caller's or the
+// library's own), the likelihood's tile geometry and the scratch of a move -- the proposal as
+// (vp, ziface) rows for the batch kernel, its node count, its sorted nodes, its logL and the
+// outside / no-move code; with `ar` also the AR move's proposal (a graph's key holds its address,
+// so it is reserved before any capture) -- with the stream ordered behind the scratch's last user.
+int begin_move(MoveCtx &m, void *stream, bool ar, cudaStream_t &st) {
+    st = stream ? (cudaStream_t)stream : g.s_comp;
+    if (int rc = choose_cfg(m.B, m.ldk, m.ldk, m.NSrc, true, m.cfg)) return rc;
+    const size_t Bz = (size_t)m.B, Bpad = (Bz + m.cfg.M - 1) / m.cfg.M * m.cfg.M + m.cfg.M;
+    CK(g.vels.reserve(Bpad * m.ldk * 8));
+    CK(g.depths.reserve(Bpad * m.ldk * 8));
     CK(g.nl.reserve(Bpad * 4));
-    CK(g.vsorted.reserve(Bz * 2 * ldk * 8));
+    CK(g.vsorted.reserve(Bz * 2 * m.ldk * 8));
     CK(g.mh_ll.reserve(Bz * 8));
     CK(g.mh_out.reserve(Bz * 4));
     CK(g.mh_kp.reserve(Bz * 4));
     CK(g.mh_lpr.reserve(Bz * 8));
-    return 0;
+    if (ar) {
+        CK(g.idxar.reserve(Bz * 4));
+        CK(g.arparb.reserve(Bz * 8));
+    }
+    return scratch_acquire(st);
+}
+
+// The end every chain-move entry shares: `launches` kernels counted; without a caller stream the
+// work is waited for (`timed`: the likelihood's time goes to kernel_ms), then the scratch released.
+int end_move(const MoveCtx &m, long long launches, bool timed, void *stream, cudaStream_t st) {
+    g.launches += launches;
+    g.last = m.cfg;
+    if (!stream) {
+        CK(cudaStreamSynchronize(st));
+        if (timed) {
+            float ms = 0.f;
+            CK(cudaEventElapsedTime(&ms, g.ev_k0[0], g.ev_k1[0]));
+            g.kernel_ms = g.total_ms = ms;
+        }
+    }
+    return scratch_release(st, stream == nullptr);
 }
 
 // The batch kernel's arguments for evaluating the scratch rows in k-mode; logL goes to g.mh_ll.
-BatchArgs move_eval_args(int B, int ldk, const double *d_src_offset, const double *d_src_depth,
-                         const double *d_tobs, int NSrc, const double *d_sigma, int *sched) {
+BatchArgs move_eval_args(const MoveCtx &m, const double *sigma, int *sched) {
     BatchArgs a{};
     a.vels = g.vels.as<double>(); a.depths = g.depths.as<double>(); a.nlayers = g.nl.as<int>();
-    a.B = B; a.ldv = ldk; a.ldz = ldk; a.kmode = 1;
-    a.src_offset = d_src_offset; a.src_depth = d_src_depth;
-    a.tobs = d_tobs; a.nsrc = NSrc; a.sigma = d_sigma;
+    a.B = m.B; a.ldv = m.ldk; a.ldz = m.ldk; a.kmode = 1;
+    a.src_offset = m.src_offset; a.src_depth = m.src_depth;
+    a.tobs = m.tobs; a.nsrc = m.NSrc; a.sigma = sigma;
     a.logL = g.mh_ll.as<double>();
-    a.logc = log_norm_const(NSrc);
+    a.logc = log_norm_const(m.NSrc);
     a.padded = 1;
     a.sched = sched;
     a.idxar = g.chain_idxar;         // IAR = 1 (rtb200_set_chain_ar); null otherwise
@@ -1199,12 +1266,141 @@ BatchArgs move_eval_args(int B, int ldk, const double *d_src_offset, const doubl
 
 // The likelihood of a move's proposals: the batch kernel, or LOGLHOOD2's constant when the
 // sampler draws from the prior (ISMPPRIOR = 1, prjmh_temper_rf.f90:693-694, :739-740, ...).
-cudaError_t launch_move_eval(const BatchArgs &a, const TileCfg &cfg, cudaStream_t st) {
-    if (g.opt_ismpprior) return rtb::launch_fill_f64(a.logL, a.B, 1.0, st);
-    return rtb::launch_batch(a, cfg, st);
+// `timed`: between ev_k0 and ev_k1 (events are not recorded inside a graph capture).
+cudaError_t launch_move_eval(const MoveCtx &m, const BatchArgs &a, bool timed, cudaStream_t st) {
+    cudaError_t e = timed ? cudaEventRecord(g.ev_k0[0], st) : cudaSuccess;
+    if (e == cudaSuccess)
+        e = g.opt_ismpprior ? rtb::launch_fill_f64(a.logL, a.B, 1.0, st) : rtb::launch_batch(a, m.cfg, st);
+    if (e == cudaSuccess && timed) e = cudaEventRecord(g.ev_k1[0], st);
+    return e;
+}
+
+// The enqueue_* functions issue one move of every chain on `st`: propose -> launch_move_eval ->
+// accept, the likelihood on tile-scheduler slot `sched`.
+// The fixed-dimension MH move.  The proposal and its likelihood do not read beta; only the accept
+// test does, and it waits for `beta_ready` when one is given.
+cudaError_t enqueue_mh(const MoveCtx &m, const rtb::MhPrior &pr, const int *ivo, const int *iwhich,
+                       const double *dev, const double *u_acc, int *accept, cudaEvent_t beta_ready,
+                       int *sched, bool timed, cudaStream_t st) {
+    cudaError_t e = rtb::launch_propose_voro(m.k, m.voro, m.B, m.ldk, ivo, iwhich, dev, pr, g.vels.as<double>(),
+                                             g.depths.as<double>(), g.nl.as<int>(), g.vsorted.as<double>(),
+                                             g.mh_lpr.as<double>(), g.mh_out.as<int>(), st);
+    if (e == cudaSuccess) e = launch_move_eval(m, move_eval_args(m, m.sigma, sched), timed, st);
+    if (e == cudaSuccess && beta_ready) e = cudaStreamWaitEvent(st, beta_ready, 0);
+    if (e == cudaSuccess)
+        e = rtb::launch_mh_accept(m.k, m.voro, g.vsorted.as<double>(), m.logL, g.mh_ll.as<double>(),
+                                  g.mh_lpr.as<double>(), g.mh_out.as<int>(), u_acc, m.beta, m.B, m.ldk, accept, st);
+    return e;
+}
+
+// The birth/death move.
+cudaError_t enqueue_bd(const MoveCtx &m, const rtb::MhPrior &pr, const rtb::BdPrior &bd, const double *u_k,
+                       const int *idel, const double *u_z, const double *u_v, const double *u_acc, int *accept,
+                       int *sched, bool timed, cudaStream_t st) {
+    cudaError_t e = rtb::launch_propose_bd(m.k, m.voro, m.B, m.ldk, u_k, idel, u_z, u_v, pr, bd,
+                                           g.vels.as<double>(), g.depths.as<double>(), g.nl.as<int>(),
+                                           g.mh_kp.as<int>(), g.vsorted.as<double>(), g.mh_lpr.as<double>(),
+                                           g.mh_out.as<int>(), st);
+    if (e == cudaSuccess) e = launch_move_eval(m, move_eval_args(m, m.sigma, sched), timed, st);
+    if (e == cudaSuccess)
+        e = rtb::launch_bd_accept(m.k, m.voro, g.vsorted.as<double>(), g.mh_kp.as<int>(), g.mh_lpr.as<double>(),
+                                  m.logL, g.mh_ll.as<double>(), g.mh_out.as<int>(), u_acc, m.beta, m.B, m.ldk,
+                                  accept, st);
+    return e;
+}
+
+// The data-error move; its likelihood uses the proposed sigma.
+cudaError_t enqueue_sd(const MoveCtx &m, const double *sd_prior, const double *u_gate, const double *gauss,
+                       const double *u_acc, int *accept, int *sched, bool timed, cudaStream_t st) {
+    cudaError_t e = rtb::launch_propose_sd(m.k, m.voro, m.B, m.ldk, m.sigma, u_gate, gauss, sd_prior[0],
+                                           sd_prior[1], sd_prior[2], g.vels.as<double>(), g.depths.as<double>(),
+                                           g.nl.as<int>(), g.mh_lpr.as<double>(), g.mh_out.as<int>(), st);
+    if (e == cudaSuccess) e = launch_move_eval(m, move_eval_args(m, g.mh_lpr.as<double>(), sched), timed, st);
+    if (e == cudaSuccess)
+        e = rtb::launch_sd_accept(m.sigma, g.mh_lpr.as<double>(), m.logL, g.mh_ll.as<double>(),
+                                  g.mh_out.as<int>(), u_acc, m.beta, m.B, accept, st);
+    return e;
+}
+
+// The AR(1) move; its likelihood uses the proposed (idxar, arpar) and armx = ar_prior[3].
+cudaError_t enqueue_ar(const MoveCtx &m, int *idxar, double *arpar, const double *ar_prior,
+                       const double *u_choice, const double *u_prop, const double *gauss, const double *u_acc,
+                       int *accept, int *sched, bool timed, cudaStream_t st) {
+    cudaError_t e = rtb::launch_propose_ar(m.k, m.voro, m.B, m.ldk, idxar, arpar, u_choice, u_prop, gauss,
+                                           ar_prior[0], ar_prior[1], ar_prior[2], std::log(0.5), std::log(2.0),
+                                           g.vels.as<double>(), g.depths.as<double>(), g.nl.as<int>(),
+                                           g.idxar.as<int>(), g.arparb.as<double>(), g.mh_lpr.as<double>(),
+                                           g.mh_out.as<int>(), st);
+    BatchArgs a = move_eval_args(m, m.sigma, sched);
+    a.idxar = g.idxar.as<int>();
+    a.arpar = g.arparb.as<double>();
+    a.armx  = ar_prior[3];
+    if (e == cudaSuccess) e = launch_move_eval(m, a, timed, st);
+    if (e == cudaSuccess)
+        e = rtb::launch_ar_accept(idxar, arpar, g.idxar.as<int>(), g.arparb.as<double>(), g.mh_lpr.as<double>(),
+                                  m.logL, g.mh_ll.as<double>(), g.mh_out.as<int>(), u_acc, m.beta, m.B, accept, st);
+    return e;
+}
+
+// The tile-scheduler slot kernel node `i` of a captured graph owns (past the round-robin slots).
+int *graph_slot(int i) { return g.opt_static_tiles ? nullptr : g.sched.as<int>() + 2 * (kSchedSlots + i); }
+
+// Appends integers and pointers to a graph's key as they are, doubles by their bits.
+template <class... T> void key_add(std::vector<size_t> &key, T... xs) {
+    auto add = [&key](auto x) {
+        if constexpr (std::is_floating_point_v<decltype(x)>) {
+            size_t bits;
+            memcpy(&bits, &x, sizeof bits);
+            key.push_back(bits);
+        } else {
+            key.push_back((size_t)x);
+        }
+    };
+    (add(xs), ...);
+}
+
+// The part of a move graph's key every such graph shares: the chain state and data, every field
+// of the tile geometry (by name: TileCfg has padding and an unused member), the likelihood
+// constant, the scratch, the options and the registered AR state.
+std::vector<size_t> move_key(const MoveCtx &m) {
+    std::vector<size_t> key;
+    const TileCfg &c = m.cfg;
+    key_add(key, m.k, m.voro, m.logL, m.sigma, m.beta, m.B, m.ldk, m.src_offset, m.src_depth, m.tobs, m.NSrc);
+    key_add(key, c.M, c.SC, c.LP, c.TS, c.threads, c.grid, c.variant, c.use_tma, c.logl_shuffle, c.smem,
+            log_norm_const(m.NSrc));
+    key_add(key, g.vels.p, g.depths.p, g.nl.p, g.vsorted.p, g.mh_ll.p, g.mh_out.p, g.mh_kp.p, g.mh_lpr.p,
+            g.idxar.p, g.arparb.p, g.opt_static_tiles, g.opt_ismpprior, g.chain_idxar, g.chain_arpar,
+            g.chain_armx);
+    return key;
+}
+
+// Replays the graph cached in `c` n times on `st`.  When `key` differs from the cached graph's,
+// the graph is first captured anew from `enqueue(stream)` on the capture stream; `what` names the
+// capture in a failure.
+template <class Enqueue>
+int run_graph(GraphCache &c, std::vector<size_t> &key, const TileCfg &cfg, const char *what, Enqueue enqueue,
+              int n, cudaStream_t st) {
+    if (!c.exec || key != c.key) {
+        c.reset();
+        if (!g.s_cap) CK(cudaStreamCreateWithFlags(&g.s_cap, cudaStreamNonBlocking));
+        if (rtb::max_ctas_per_sm(cfg) < 1) return fail("batch kernel cannot be resident");   // sets the smem attribute
+        CK(cudaStreamBeginCapture(g.s_cap, cudaStreamCaptureModeThreadLocal));
+        cudaError_t e = enqueue(g.s_cap);
+        cudaGraph_t graph = nullptr;
+        const cudaError_t e2 = cudaStreamEndCapture(g.s_cap, &graph);
+        if (e != cudaSuccess) { if (graph) cudaGraphDestroy(graph); return fail(what, e); }
+        if (e2 != cudaSuccess) return fail("cudaStreamEndCapture", e2);
+        e = cudaGraphInstantiate(&c.exec, graph, 0);
+        cudaGraphDestroy(graph);
+        if (e != cudaSuccess) { c.exec = nullptr; return fail("cudaGraphInstantiate", e); }
+        c.key.swap(key);
+    }
+    for (int i = 0; i < n; ++i) CK(cudaGraphLaunch(c.exec, st));
+    return 0;
 }
 
 }  // namespace
+}  // extern "C++"
 
 int rtb200_mh_step_device(const int *d_k, double *d_voro, double *d_logL, int B, int ldk,
                           const int *d_ivo, const int *d_iwhich, const double *d_cauchy,
@@ -1228,43 +1424,21 @@ int rtb200_mh_step_device_ev(const int *d_k, double *d_voro, double *d_logL, int
     if (int rc = ensure_init()) return rc;
     g.err.clear();
     if (B <= 0) return 0;
-    if (NSrc <= 0) return fail("rtb200_mh_step_device needs at least one source");
-    if (ldk < 1 || ldk > 64) return fail("rtb200_mh_step_device supports 1..64 nodes per state");
+    if (int rc = check_move_args("rtb200_mh_step_device", NSrc, ldk)) return rc;
     if (!prior) return fail("rtb200_mh_step_device needs the prior array");
-    cudaStream_t st = stream ? (cudaStream_t)stream : g.s_comp;
-    TileCfg cfg;
-    if (int rc = choose_cfg(B, ldk, ldk, NSrc, true, cfg)) return rc;
-    if (int rc = reserve_move_scratch(B, ldk, cfg)) return rc;
-    if (int rc = scratch_acquire(st)) return rc;
-    const rtb::MhPrior pr = make_prior(prior, enos);
-    CK(rtb::launch_propose_voro(d_k, d_voro, B, ldk, d_ivo, d_iwhich, d_cauchy, pr,
-                                g.vels.as<double>(), g.depths.as<double>(), g.nl.as<int>(),
-                                g.vsorted.as<double>(), g.mh_lpr.as<double>(), g.mh_out.as<int>(), st));
-    const BatchArgs a = move_eval_args(B, ldk, d_src_offset, d_src_depth, d_tobs, NSrc, d_sigma,
-                                       next_sched());
-    CK(cudaEventRecord(g.ev_k0[0], st));
-    CK(launch_move_eval(a, cfg, st));
-    CK(cudaEventRecord(g.ev_k1[0], st));
-    // the proposal and its likelihood do not read beta; only the accept test does
-    if (beta_ready_event) CK(cudaStreamWaitEvent(st, (cudaEvent_t)beta_ready_event, 0));
-    CK(rtb::launch_mh_accept(d_k, d_voro, g.vsorted.as<double>(), d_logL, g.mh_ll.as<double>(),
-                             g.mh_lpr.as<double>(), g.mh_out.as<int>(), d_uacc, d_beta, B, ldk, d_accept, st));
-    g.launches += 3;
-    g.last = cfg;
-    if (!stream) {
-        CK(cudaStreamSynchronize(st));
-        float ms = 0.f;
-        CK(cudaEventElapsedTime(&ms, g.ev_k0[0], g.ev_k1[0]));
-        g.kernel_ms = g.total_ms = ms;
-    }
-    if (int rc = scratch_release(st, stream == nullptr)) return rc;
-    return 0;
+    MoveCtx m = move_ctx(d_k, d_voro, d_logL, d_sigma, d_beta, B, ldk, d_src_offset, d_src_depth, d_tobs, NSrc);
+    cudaStream_t st;
+    if (int rc = begin_move(m, stream, false, st)) return rc;
+    CK(enqueue_mh(m, make_prior(prior, enos), d_ivo, d_iwhich, d_cauchy, d_uacc, d_accept,
+                  (cudaEvent_t)beta_ready_event, next_sched(), true, st));
+    return end_move(m, 3, true, stream, st);
 }
 
 // n_moves fixed-dimension moves back to back.  A move is three dependent launches (propose,
 // evaluate, accept) of a few hundred microseconds at most, so a run of moves is launch-bound; the
 // run is captured once into a CUDA graph and replayed while the caller keeps passing the same
-// buffers (the key is every pointer and size).  Each kernel node owns its tile-scheduler slot.
+// buffers and options (the key is everything the capture bakes in).  Each kernel node owns its
+// tile-scheduler slot.
 int rtb200_mh_moves_device(const int *d_k, double *d_voro, double *d_logL, int B, int ldk,
                            int n_moves, const int *d_ivo, const int *d_iwhich,
                            const double *d_cauchy, const double *d_uacc, const double *d_beta,
@@ -1287,70 +1461,27 @@ int rtb200_mh_moves_device_ex(const int *d_k, double *d_voro, double *d_logL, in
     if (int rc = ensure_init()) return rc;
     g.err.clear();
     if (B <= 0 || n_moves <= 0) return 0;
-    if (NSrc <= 0) return fail("rtb200_mh_moves_device needs at least one source");
-    if (ldk < 1 || ldk > 64) return fail("rtb200_mh_moves_device supports 1..64 nodes per state");
+    if (int rc = check_move_args("rtb200_mh_moves_device", NSrc, ldk)) return rc;
     if (!prior) return fail("rtb200_mh_moves_device needs the prior array");
     if (n_moves > kGraphSlots) return fail("rtb200_mh_moves_device: at most 512 moves per call");
-    cudaStream_t st = stream ? (cudaStream_t)stream : g.s_comp;
-    TileCfg cfg;
-    if (int rc = choose_cfg(B, ldk, ldk, NSrc, true, cfg)) return rc;
-    if (int rc = reserve_move_scratch(B, ldk, cfg)) return rc;
-    if (int rc = scratch_acquire(st)) return rc;
-    std::vector<size_t> key = {(size_t)d_k, (size_t)d_voro, (size_t)d_logL, (size_t)B, (size_t)ldk,
-                               (size_t)n_moves, (size_t)d_ivo, (size_t)d_iwhich, (size_t)d_cauchy,
-                               (size_t)d_uacc, (size_t)d_beta, (size_t)d_sigma, (size_t)d_src_offset,
-                               (size_t)d_src_depth, (size_t)d_tobs, (size_t)NSrc, (size_t)d_accept,
-                               (size_t)g.vels.p, (size_t)g.depths.p, (size_t)g.nl.p,
-                               (size_t)g.vsorted.p, (size_t)g.mh_ll.p, (size_t)g.mh_out.p,
-                               (size_t)cfg.M, (size_t)cfg.grid, (size_t)cfg.variant, (size_t)g.opt_static_tiles,
-                               (size_t)g.chain_idxar, (size_t)g.chain_arpar, (size_t)(enos ? 1 : 0),
-                               (size_t)g.mh_lpr.p, (size_t)g.opt_ismpprior};
-    {
-        size_t bits;
-        memcpy(&bits, &g.chain_armx, sizeof bits);
-        key.push_back(bits);
-    }
-    for (int i = 0; i < 7; ++i) {
-        size_t bits;
-        memcpy(&bits, &prior[i], sizeof bits);
-        key.push_back(bits);
-    }
-    if (!g.mv_exec || key != g.mv_key) {
-        if (g.mv_exec) { cudaGraphExecDestroy(g.mv_exec); g.mv_exec = nullptr; }
-        if (!g.s_cap) CK(cudaStreamCreateWithFlags(&g.s_cap, cudaStreamNonBlocking));
+    MoveCtx m = move_ctx(d_k, d_voro, d_logL, d_sigma, d_beta, B, ldk, d_src_offset, d_src_depth, d_tobs, NSrc);
+    cudaStream_t st;
+    if (int rc = begin_move(m, stream, false, st)) return rc;
+    std::vector<size_t> key = move_key(m);
+    key_add(key, n_moves, d_ivo, d_iwhich, d_cauchy, d_uacc, d_accept, enos ? 1 : 0);
+    for (int i = 0; i < 7; ++i) key_add(key, prior[i]);
+    auto capture = [&](cudaStream_t sc) {
         const rtb::MhPrior pr = make_prior(prior, enos);
-        if (rtb::max_ctas_per_sm(cfg) < 1) return fail("batch kernel cannot be resident");   // sets the smem attribute
-        CK(cudaStreamBeginCapture(g.s_cap, cudaStreamCaptureModeThreadLocal));
         cudaError_t e = cudaSuccess;
-        for (int m = 0; m < n_moves && e == cudaSuccess; ++m) {
-            const size_t o = (size_t)m * (size_t)B;
-            e = rtb::launch_propose_voro(d_k, d_voro, B, ldk, d_ivo + o, d_iwhich + o, d_cauchy + o, pr,
-                                         g.vels.as<double>(), g.depths.as<double>(), g.nl.as<int>(),
-                                         g.vsorted.as<double>(), g.mh_lpr.as<double>(), g.mh_out.as<int>(), g.s_cap);
-            if (e != cudaSuccess) break;
-            const BatchArgs a = move_eval_args(B, ldk, d_src_offset, d_src_depth, d_tobs, NSrc, d_sigma,
-                                               g.opt_static_tiles ? nullptr : g.sched.as<int>() + 2 * (kSchedSlots + m));
-            e = launch_move_eval(a, cfg, g.s_cap);
-            if (e != cudaSuccess) break;
-            e = rtb::launch_mh_accept(d_k, d_voro, g.vsorted.as<double>(), d_logL, g.mh_ll.as<double>(),
-                                      g.mh_lpr.as<double>(), g.mh_out.as<int>(), d_uacc + o, d_beta, B, ldk,
-                                      d_accept + o, g.s_cap);
+        for (int i = 0; i < n_moves && e == cudaSuccess; ++i) {
+            const size_t o = (size_t)i * (size_t)B;
+            e = enqueue_mh(m, pr, d_ivo + o, d_iwhich + o, d_cauchy + o, d_uacc + o, d_accept + o, nullptr,
+                           graph_slot(i), false, sc);
         }
-        cudaGraph_t graph = nullptr;
-        cudaError_t e2 = cudaStreamEndCapture(g.s_cap, &graph);
-        if (e != cudaSuccess) { if (graph) cudaGraphDestroy(graph); return fail("capturing the MH moves", e); }
-        if (e2 != cudaSuccess) return fail("cudaStreamEndCapture", e2);
-        e = cudaGraphInstantiate(&g.mv_exec, graph, 0);
-        cudaGraphDestroy(graph);
-        if (e != cudaSuccess) { g.mv_exec = nullptr; return fail("cudaGraphInstantiate", e); }
-        g.mv_key = key;
-    }
-    CK(cudaGraphLaunch(g.mv_exec, st));
-    g.launches += 3LL * n_moves;
-    g.last = cfg;
-    if (!stream) CK(cudaStreamSynchronize(st));
-    if (int rc = scratch_release(st, stream == nullptr)) return rc;
-    return 0;
+        return e;
+    };
+    if (int rc = run_graph(g.mv, key, m.cfg, "capturing the MH moves", capture, 1, st)) return rc;
+    return end_move(m, 3LL * n_moves, false, stream, st);
 }
 
 int rtb200_bd_step_device(int *d_k, double *d_voro, double *d_logL, int B, int ldk,
@@ -1375,41 +1506,15 @@ int rtb200_bd_step_device_ex(int *d_k, double *d_voro, double *d_logL, int B, in
     if (int rc = ensure_init()) return rc;
     g.err.clear();
     if (B <= 0) return 0;
-    if (NSrc <= 0) return fail("rtb200_bd_step_device needs at least one source");
-    if (ldk < 1 || ldk > 64) return fail("rtb200_bd_step_device supports 1..64 nodes per state");
+    if (int rc = check_move_args("rtb200_bd_step_device", NSrc, ldk)) return rc;
     if (!prior) return fail("rtb200_bd_step_device needs the prior array");
     if (kmin < 1 || kmax < kmin || kmax > ldk) return fail("rtb200_bd_step_device needs 1 <= kmin <= kmax <= ldk");
-    cudaStream_t st = stream ? (cudaStream_t)stream : g.s_comp;
-    TileCfg cfg;
-    if (int rc = choose_cfg(B, ldk, ldk, NSrc, true, cfg)) return rc;
-    if (int rc = reserve_move_scratch(B, ldk, cfg)) return rc;
-    if (int rc = scratch_acquire(st)) return rc;
-    const rtb::MhPrior pr = make_prior(prior, enos);
-    rtb::BdPrior bd{};
-    bd.kmin = kmin; bd.kmax = kmax; bd.use_pk = pk ? 1 : 0;
-    for (int i = kmin; pk && i <= kmax; ++i) bd.logpk[i - 1] = std::log(pk[i - 1]);   // LOG(pk(i)), libm
-    CK(rtb::launch_propose_bd(d_k, d_voro, B, ldk, d_uk, d_idel, d_uz, d_uv, pr, bd,
-                              g.vels.as<double>(), g.depths.as<double>(), g.nl.as<int>(),
-                              g.mh_kp.as<int>(), g.vsorted.as<double>(), g.mh_lpr.as<double>(),
-                              g.mh_out.as<int>(), st));
-    const BatchArgs a = move_eval_args(B, ldk, d_src_offset, d_src_depth, d_tobs, NSrc, d_sigma,
-                                       next_sched());
-    CK(cudaEventRecord(g.ev_k0[0], st));
-    CK(launch_move_eval(a, cfg, st));
-    CK(cudaEventRecord(g.ev_k1[0], st));
-    CK(rtb::launch_bd_accept(d_k, d_voro, g.vsorted.as<double>(), g.mh_kp.as<int>(),
-                             g.mh_lpr.as<double>(), d_logL, g.mh_ll.as<double>(),
-                             g.mh_out.as<int>(), d_uacc, d_beta, B, ldk, d_accept, st));
-    g.launches += 3;
-    g.last = cfg;
-    if (!stream) {
-        CK(cudaStreamSynchronize(st));
-        float ms = 0.f;
-        CK(cudaEventElapsedTime(&ms, g.ev_k0[0], g.ev_k1[0]));
-        g.kernel_ms = g.total_ms = ms;
-    }
-    if (int rc = scratch_release(st, stream == nullptr)) return rc;
-    return 0;
+    MoveCtx m = move_ctx(d_k, d_voro, d_logL, d_sigma, d_beta, B, ldk, d_src_offset, d_src_depth, d_tobs, NSrc);
+    cudaStream_t st;
+    if (int rc = begin_move(m, stream, false, st)) return rc;
+    CK(enqueue_bd(m, make_prior(prior, enos), make_bd_prior(pk, kmin, kmax), d_uk, d_idel, d_uz, d_uv, d_uacc,
+                  d_accept, next_sched(), true, st));
+    return end_move(m, 3, true, stream, st);
 }
 
 int rtb200_sd_step_device(const int *d_k, const double *d_voro, double *d_logL, double *d_sigma,
@@ -1421,34 +1526,13 @@ int rtb200_sd_step_device(const int *d_k, const double *d_voro, double *d_logL, 
     if (int rc = ensure_init()) return rc;
     g.err.clear();
     if (B <= 0) return 0;
-    if (NSrc <= 0) return fail("rtb200_sd_step_device needs at least one source");
-    if (ldk < 1 || ldk > 64) return fail("rtb200_sd_step_device supports 1..64 nodes per state");
+    if (int rc = check_move_args("rtb200_sd_step_device", NSrc, ldk)) return rc;
     if (!sd_prior) return fail("rtb200_sd_step_device needs the sd_prior array");
-    cudaStream_t st = stream ? (cudaStream_t)stream : g.s_comp;
-    TileCfg cfg;
-    if (int rc = choose_cfg(B, ldk, ldk, NSrc, true, cfg)) return rc;
-    if (int rc = reserve_move_scratch(B, ldk, cfg)) return rc;
-    if (int rc = scratch_acquire(st)) return rc;
-    CK(rtb::launch_propose_sd(d_k, d_voro, B, ldk, d_sigma, d_ugate, d_gauss, sd_prior[0],
-                              sd_prior[1], sd_prior[2], g.vels.as<double>(), g.depths.as<double>(),
-                              g.nl.as<int>(), g.mh_lpr.as<double>(), g.mh_out.as<int>(), st));
-    const BatchArgs a = move_eval_args(B, ldk, d_src_offset, d_src_depth, d_tobs, NSrc, g.mh_lpr.as<double>(),
-                                       next_sched());
-    CK(cudaEventRecord(g.ev_k0[0], st));
-    CK(launch_move_eval(a, cfg, st));
-    CK(cudaEventRecord(g.ev_k1[0], st));
-    CK(rtb::launch_sd_accept(d_sigma, g.mh_lpr.as<double>(), d_logL, g.mh_ll.as<double>(),
-                             g.mh_out.as<int>(), d_uacc, d_beta, B, d_accept, st));
-    g.launches += 3;
-    g.last = cfg;
-    if (!stream) {
-        CK(cudaStreamSynchronize(st));
-        float ms = 0.f;
-        CK(cudaEventElapsedTime(&ms, g.ev_k0[0], g.ev_k1[0]));
-        g.kernel_ms = g.total_ms = ms;
-    }
-    if (int rc = scratch_release(st, stream == nullptr)) return rc;
-    return 0;
+    MoveCtx m = move_ctx(d_k, d_voro, d_logL, d_sigma, d_beta, B, ldk, d_src_offset, d_src_depth, d_tobs, NSrc);
+    cudaStream_t st;
+    if (int rc = begin_move(m, stream, false, st)) return rc;
+    CK(enqueue_sd(m, sd_prior, d_ugate, d_gauss, d_uacc, d_accept, next_sched(), true, st));
+    return end_move(m, 3, true, stream, st);
 }
 
 int rtb200_set_chain_ar(const int *d_idxar, const double *d_arpar, double armx) {
@@ -1471,41 +1555,14 @@ int rtb200_ar_step_device(const int *d_k, const double *d_voro, double *d_logL,
     if (int rc = ensure_init()) return rc;
     g.err.clear();
     if (B <= 0) return 0;
-    if (NSrc <= 0) return fail("rtb200_ar_step_device needs at least one source");
-    if (ldk < 1 || ldk > 64) return fail("rtb200_ar_step_device supports 1..64 nodes per state");
+    if (int rc = check_move_args("rtb200_ar_step_device", NSrc, ldk)) return rc;
     if (!ar_prior) return fail("rtb200_ar_step_device needs the ar_prior array");
-    cudaStream_t st = stream ? (cudaStream_t)stream : g.s_comp;
-    TileCfg cfg;
-    if (int rc = choose_cfg(B, ldk, ldk, NSrc, true, cfg)) return rc;
-    if (int rc = reserve_move_scratch(B, ldk, cfg)) return rc;
-    if (int rc = scratch_acquire(st)) return rc;
-    CK(g.idxar.reserve((size_t)B * 4));
-    CK(g.arparb.reserve((size_t)B * 8));
-    CK(rtb::launch_propose_ar(d_k, d_voro, B, ldk, d_idxar, d_arpar, d_uchoice, d_uprop, d_gauss,
-                              ar_prior[0], ar_prior[1], ar_prior[2], std::log(0.5), std::log(2.0),
-                              g.vels.as<double>(), g.depths.as<double>(), g.nl.as<int>(),
-                              g.idxar.as<int>(), g.arparb.as<double>(), g.mh_lpr.as<double>(),
-                              g.mh_out.as<int>(), st));
-    BatchArgs a = move_eval_args(B, ldk, d_src_offset, d_src_depth, d_tobs, NSrc, d_sigma, next_sched());
-    a.idxar = g.idxar.as<int>();
-    a.arpar = g.arparb.as<double>();
-    a.armx  = ar_prior[3];
-    CK(cudaEventRecord(g.ev_k0[0], st));
-    CK(launch_move_eval(a, cfg, st));
-    CK(cudaEventRecord(g.ev_k1[0], st));
-    CK(rtb::launch_ar_accept(d_idxar, d_arpar, g.idxar.as<int>(), g.arparb.as<double>(),
-                             g.mh_lpr.as<double>(), d_logL, g.mh_ll.as<double>(), g.mh_out.as<int>(),
-                             d_uacc, d_beta, B, d_accept, st));
-    g.launches += 3;
-    g.last = cfg;
-    if (!stream) {
-        CK(cudaStreamSynchronize(st));
-        float ms = 0.f;
-        CK(cudaEventElapsedTime(&ms, g.ev_k0[0], g.ev_k1[0]));
-        g.kernel_ms = g.total_ms = ms;
-    }
-    if (int rc = scratch_release(st, stream == nullptr)) return rc;
-    return 0;
+    MoveCtx m = move_ctx(d_k, d_voro, d_logL, d_sigma, d_beta, B, ldk, d_src_offset, d_src_depth, d_tobs, NSrc);
+    cudaStream_t st;
+    if (int rc = begin_move(m, stream, true, st)) return rc;
+    CK(enqueue_ar(m, d_idxar, d_arpar, ar_prior, d_uchoice, d_uprop, d_gauss, d_uacc, d_accept, next_sched(),
+                  true, st));
+    return end_move(m, 3, true, stream, st);
 }
 
 size_t rtb200_mcmc_workspace_bytes(int B, int n_moves) {
@@ -1532,17 +1589,14 @@ int rtb200_mcmc_iterations_device(int *d_k, double *d_voro, double *d_logL, doub
     if (B <= 0 || n_iterations <= 0) return 0;
     if ((d_idxar == nullptr) != (d_arpar == nullptr) || (d_idxar && !ar_prior))
         return fail("rtb200_mcmc_iterations_device: the AR move needs idxar, arpar and ar_prior together");
-    if (NSrc <= 0) return fail("rtb200_mcmc_iterations_device needs at least one source");
-    if (ldk < 1 || ldk > 64) return fail("rtb200_mcmc_iterations_device supports 1..64 nodes per state");
+    if (int rc = check_move_args("rtb200_mcmc_iterations_device", NSrc, ldk)) return rc;
     if (!prior || !sd_prior) return fail("rtb200_mcmc_iterations_device needs the prior and sd_prior arrays");
     if (kmin < 1 || kmax < kmin || kmax > ldk) return fail("rtb200_mcmc_iterations_device needs 1 <= kmin <= kmax <= ldk");
     if (n_moves < 0 || n_moves + 3 > kGraphSlots) return fail("rtb200_mcmc_iterations_device: at most 509 moves per iteration");
     if (!d_counter || !d_workspace || !d_pos) return fail("rtb200_mcmc_iterations_device needs counter, workspace and pos");
-    cudaStream_t st = stream ? (cudaStream_t)stream : g.s_comp;
-    TileCfg cfg;
-    if (int rc = choose_cfg(B, ldk, ldk, NSrc, true, cfg)) return rc;
-    if (int rc = reserve_move_scratch(B, ldk, cfg)) return rc;
-    if (int rc = scratch_acquire(st)) return rc;
+    MoveCtx m = move_ctx(d_k, d_voro, d_logL, d_sigma, d_beta, B, ldk, d_src_offset, d_src_depth, d_tobs, NSrc);
+    cudaStream_t st;
+    if (int rc = begin_move(m, stream, d_idxar != nullptr, st)) return rc;
     const rtb::McmcWs w = rtb::mcmc_ws_layout(d_workspace, (size_t)B, (size_t)n_moves);
     // IAR = 1: with the AR move in the iteration, every likelihood of the iteration uses the chains'
     // AR state (as if registered with rtb200_set_chain_ar); the registration is restored on return
@@ -1554,115 +1608,44 @@ int rtb200_mcmc_iterations_device(int *d_k, double *d_voro, double *d_logL, doub
         g.chain_idxar = d_idxar;
         g.chain_arpar = d_arpar;
         g.chain_armx  = ar_prior[3];
-        CK(g.idxar.reserve((size_t)B * 4));
-        CK(g.arparb.reserve((size_t)B * 8));
     }
-    std::vector<size_t> key = {(size_t)d_k, (size_t)d_voro, (size_t)d_logL, (size_t)d_sigma, (size_t)d_beta,
-                               (size_t)d_pos, (size_t)B, (size_t)ldk, (size_t)n_moves, (size_t)kmin, (size_t)kmax,
-                               (size_t)(enos ? 1 : 0), (size_t)d_src_offset, (size_t)d_src_depth, (size_t)d_tobs,
-                               (size_t)NSrc, (size_t)seed, (size_t)d_counter, (size_t)d_workspace, (size_t)d_tally,
-                               (size_t)g.vels.p, (size_t)g.depths.p, (size_t)g.nl.p, (size_t)g.vsorted.p,
-                               (size_t)g.mh_ll.p, (size_t)g.mh_out.p, (size_t)g.mh_kp.p, (size_t)g.mh_lpr.p,
-                               (size_t)cfg.M, (size_t)cfg.grid, (size_t)cfg.variant, (size_t)g.opt_static_tiles,
-                               (size_t)g.chain_idxar, (size_t)g.chain_arpar, (size_t)(pk ? 1 : 0), (size_t)g.opt_ismpprior};
-    auto push_bits = [&](double x) { size_t bits; memcpy(&bits, &x, sizeof bits); key.push_back(bits); };
-    push_bits(g.chain_armx);
-    for (int i = 0; i < 7; ++i) push_bits(prior[i]);
-    for (int i = 0; i < 3; ++i) push_bits(sd_prior[i]);
-    for (int i = kmin; pk && i <= kmax; ++i) push_bits(pk[i - 1]);
-    key.push_back((size_t)d_idxar);
-    key.push_back((size_t)d_arpar);
-    key.push_back((size_t)g.idxar.p);
-    key.push_back((size_t)g.arparb.p);
-    for (int i = 0; d_idxar && i < 4; ++i) push_bits(ar_prior[i]);
-    if (!g.mc_exec || key != g.mc_key) {
-        if (g.mc_exec) { cudaGraphExecDestroy(g.mc_exec); g.mc_exec = nullptr; }
-        if (!g.s_cap) CK(cudaStreamCreateWithFlags(&g.s_cap, cudaStreamNonBlocking));
+    std::vector<size_t> key = move_key(m);
+    key_add(key, d_pos, n_moves, kmin, kmax, enos ? 1 : 0, seed, d_counter, d_workspace, d_tally, pk ? 1 : 0,
+            d_idxar, d_arpar);
+    for (int i = 0; i < 7; ++i) key_add(key, prior[i]);
+    for (int i = 0; i < 3; ++i) key_add(key, sd_prior[i]);
+    for (int i = kmin; pk && i <= kmax; ++i) key_add(key, pk[i - 1]);
+    for (int i = 0; d_idxar && i < 4; ++i) key_add(key, ar_prior[i]);
+    // kernel nodes take the graph slots past the MH-moves graph's
+    auto capture = [&](cudaStream_t sc) {
         const rtb::MhPrior pr = make_prior(prior, enos);
-        rtb::BdPrior bd{};
-        bd.kmin = kmin; bd.kmax = kmax; bd.use_pk = pk ? 1 : 0;
-        for (int i = kmin; pk && i <= kmax; ++i) bd.logpk[i - 1] = std::log(pk[i - 1]);
-        if (rtb::max_ctas_per_sm(cfg) < 1) return fail("batch kernel cannot be resident");
-        int *slots = g.sched.as<int>() + 2 * (kSchedSlots + kGraphSlots);
-        auto slot = [&](int i) { return g.opt_static_tiles ? nullptr : slots + 2 * i; };
-        cudaStream_t sc = g.s_cap;
-        CK(cudaStreamBeginCapture(sc, cudaStreamCaptureModeThreadLocal));
-        cudaError_t e = cudaSuccess;
-        auto ok = [&](cudaError_t x) { if (e == cudaSuccess) e = x; return e == cudaSuccess; };
         // ---- deviates of the birth/death and data-error moves, then the birth/death move
-        ok(rtb::launch_mcmc_draw(d_counter, seed, d_k, B, w, sc));
-        if (e == cudaSuccess && kmin != kmax) {
-            ok(rtb::launch_propose_bd(d_k, d_voro, B, ldk, w.u_k, w.idel, w.u_z, w.u_v, pr, bd,
-                                      g.vels.as<double>(), g.depths.as<double>(), g.nl.as<int>(),
-                                      g.mh_kp.as<int>(), g.vsorted.as<double>(), g.mh_lpr.as<double>(),
-                                      g.mh_out.as<int>(), sc));
-            const BatchArgs a = move_eval_args(B, ldk, d_src_offset, d_src_depth, d_tobs, NSrc, d_sigma, slot(0));
-            if (e == cudaSuccess) ok(launch_move_eval(a, cfg, sc));
-            if (e == cudaSuccess)
-                ok(rtb::launch_bd_accept(d_k, d_voro, g.vsorted.as<double>(), g.mh_kp.as<int>(),
-                                         g.mh_lpr.as<double>(), d_logL, g.mh_ll.as<double>(),
-                                         g.mh_out.as<int>(), w.u_acc_bd, d_beta, B, ldk, w.acc_bd, sc));
-        }
+        cudaError_t e = rtb::launch_mcmc_draw(d_counter, seed, d_k, B, w, sc);
+        if (e == cudaSuccess && kmin != kmax)
+            e = enqueue_bd(m, pr, make_bd_prior(pk, kmin, kmax), w.u_k, w.idel, w.u_z, w.u_v, w.u_acc_bd,
+                           w.acc_bd, graph_slot(kGraphSlots), false, sc);
         // ---- every chain's next n_moves fixed-dimension moves (schedule from the node counts now)
         if (e == cudaSuccess && n_moves > 0)
-            ok(rtb::launch_mcmc_sweep_draw(d_counter, seed, d_k, d_pos, B, n_moves, enos, w, sc));
-        for (int m = 0; m < n_moves && e == cudaSuccess; ++m) {
-            const size_t o = (size_t)m * (size_t)B;
-            ok(rtb::launch_propose_voro(d_k, d_voro, B, ldk, w.ivo + o, w.iwhich + o, w.dev + o, pr,
-                                        g.vels.as<double>(), g.depths.as<double>(), g.nl.as<int>(),
-                                        g.vsorted.as<double>(), g.mh_lpr.as<double>(), g.mh_out.as<int>(), sc));
-            const BatchArgs a = move_eval_args(B, ldk, d_src_offset, d_src_depth, d_tobs, NSrc, d_sigma, slot(1 + m));
-            if (e == cudaSuccess) ok(launch_move_eval(a, cfg, sc));
-            if (e == cudaSuccess)
-                ok(rtb::launch_mh_accept(d_k, d_voro, g.vsorted.as<double>(), d_logL, g.mh_ll.as<double>(),
-                                         g.mh_lpr.as<double>(), g.mh_out.as<int>(), w.u_acc + o, d_beta, B, ldk,
-                                         w.acc_mh + o, sc));
+            e = rtb::launch_mcmc_sweep_draw(d_counter, seed, d_k, d_pos, B, n_moves, enos, w, sc);
+        for (int i = 0; i < n_moves && e == cudaSuccess; ++i) {
+            const size_t o = (size_t)i * (size_t)B;
+            e = enqueue_mh(m, pr, w.ivo + o, w.iwhich + o, w.dev + o, w.u_acc + o, w.acc_mh + o, nullptr,
+                           graph_slot(kGraphSlots + 1 + i), false, sc);
         }
-        // ---- the data-error move
-        if (e == cudaSuccess) {
-            ok(rtb::launch_propose_sd(d_k, d_voro, B, ldk, d_sigma, w.u_gate, w.gauss, sd_prior[0], sd_prior[1],
-                                      sd_prior[2], g.vels.as<double>(), g.depths.as<double>(), g.nl.as<int>(),
-                                      g.mh_lpr.as<double>(), g.mh_out.as<int>(), sc));
-            const BatchArgs a = move_eval_args(B, ldk, d_src_offset, d_src_depth, d_tobs, NSrc,
-                                               g.mh_lpr.as<double>(), slot(1 + n_moves));
-            if (e == cudaSuccess) ok(launch_move_eval(a, cfg, sc));
-            if (e == cudaSuccess)
-                ok(rtb::launch_sd_accept(d_sigma, g.mh_lpr.as<double>(), d_logL, g.mh_ll.as<double>(),
-                                         g.mh_out.as<int>(), w.u_acc_sd, d_beta, B, w.acc_sd, sc));
-        }
-        // ---- the AR(1) move (IAR = 1)
-        if (e == cudaSuccess && d_idxar) {
-            ok(rtb::launch_propose_ar(d_k, d_voro, B, ldk, d_idxar, d_arpar, w.u_choice, w.u_prop_ar, w.gauss_ar,
-                                      ar_prior[0], ar_prior[1], ar_prior[2], std::log(0.5), std::log(2.0),
-                                      g.vels.as<double>(), g.depths.as<double>(), g.nl.as<int>(),
-                                      g.idxar.as<int>(), g.arparb.as<double>(), g.mh_lpr.as<double>(),
-                                      g.mh_out.as<int>(), sc));
-            BatchArgs a = move_eval_args(B, ldk, d_src_offset, d_src_depth, d_tobs, NSrc, d_sigma, slot(2 + n_moves));
-            a.idxar = g.idxar.as<int>();
-            a.arpar = g.arparb.as<double>();
-            a.armx  = ar_prior[3];
-            if (e == cudaSuccess) ok(launch_move_eval(a, cfg, sc));
-            if (e == cudaSuccess)
-                ok(rtb::launch_ar_accept(d_idxar, d_arpar, g.idxar.as<int>(), g.arparb.as<double>(),
-                                         g.mh_lpr.as<double>(), d_logL, g.mh_ll.as<double>(), g.mh_out.as<int>(),
-                                         w.u_acc_ar, d_beta, B, w.acc_ar, sc));
-        }
-        if (e == cudaSuccess) ok(rtb::launch_mcmc_finish(d_counter, d_k, d_pos, B, n_moves, w, d_tally, sc));
-        cudaGraph_t graph = nullptr;
-        cudaError_t e2 = cudaStreamEndCapture(sc, &graph);
-        if (e != cudaSuccess) { if (graph) cudaGraphDestroy(graph); return fail("capturing the MCMC iteration", e); }
-        if (e2 != cudaSuccess) return fail("cudaStreamEndCapture", e2);
-        e = cudaGraphInstantiate(&g.mc_exec, graph, 0);
-        cudaGraphDestroy(graph);
-        if (e != cudaSuccess) { g.mc_exec = nullptr; return fail("cudaGraphInstantiate", e); }
-        g.mc_key = key;
-    }
-    for (int it = 0; it < n_iterations; ++it) CK(cudaGraphLaunch(g.mc_exec, st));
-    g.launches += (long long)n_iterations * (3LL * n_moves + (kmin != kmax ? 3 : 0) + 3 + (d_idxar ? 3 : 0) + 2 + (n_moves > 0 ? 1 : 0));
-    g.last = cfg;
-    if (int rc = scratch_release(st, stream == nullptr)) return rc;
-    if (!stream) CK(cudaStreamSynchronize(st));
-    return 0;
+        // ---- the data-error move, then the AR(1) move (IAR = 1)
+        if (e == cudaSuccess)
+            e = enqueue_sd(m, sd_prior, w.u_gate, w.gauss, w.u_acc_sd, w.acc_sd, graph_slot(kGraphSlots + 1 + n_moves),
+                           false, sc);
+        if (e == cudaSuccess && d_idxar)
+            e = enqueue_ar(m, d_idxar, d_arpar, ar_prior, w.u_choice, w.u_prop_ar, w.gauss_ar, w.u_acc_ar, w.acc_ar,
+                           graph_slot(kGraphSlots + 2 + n_moves), false, sc);
+        if (e == cudaSuccess) e = rtb::launch_mcmc_finish(d_counter, d_k, d_pos, B, n_moves, w, d_tally, sc);
+        return e;
+    };
+    if (int rc = run_graph(g.mc, key, m.cfg, "capturing the MCMC iteration", capture, n_iterations, st)) return rc;
+    const long long per_iteration =
+        3LL * n_moves + (kmin != kmax ? 3 : 0) + 3 + (d_idxar ? 3 : 0) + 2 + (n_moves > 0 ? 1 : 0);
+    return end_move(m, (long long)n_iterations * per_iteration, false, stream, st);
 }
 
 int rtb200_swap_pack_device(const double *d_logL, const double *d_beta, int n, double *d_out,
@@ -1734,12 +1717,8 @@ void rtb200_shutdown(void) {
     g.scratch_pending = false;
     cudaStreamDestroy(g.s_comp);
     cudaStreamDestroy(g.s_comp2);
-    if (g.mv_exec) cudaGraphExecDestroy(g.mv_exec);
-    g.mv_exec = nullptr;
-    g.mv_key.clear();
-    if (g.mc_exec) cudaGraphExecDestroy(g.mc_exec);
-    g.mc_exec = nullptr;
-    g.mc_key.clear();
+    g.mv.reset();
+    g.mc.reset();
     g.chain_idxar = nullptr;
     g.chain_arpar = nullptr;
     if (g.s_cap) cudaStreamDestroy(g.s_cap);

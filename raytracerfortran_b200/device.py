@@ -49,20 +49,20 @@ def dff_batch_device(vels, depths, nlayers, src_offset, src_depth, tobs=None, si
         p_out = torch.empty((B, nsrc), dtype=f64, device=dev)
     if tobs is not None and logL is None:
         logL = torch.empty((B,), dtype=f64, device=dev)
-    st = stream if stream is not None else torch.cuda.current_stream(dev)
     rc = _lib.load().rtb200_dff_batch_device(
         _ptr(vels, f64), _ptr(depths, f64) if ldz else None, _ptr(nlayers, torch.int32), B, ldv, ldz,
         _ptr(src_offset, f64), _ptr(src_depth, f64), nsrc, _ptr(timeP, f64), _ptr(tobs, f64),
-        _ptr(sigma, f64), _ptr(logL, f64), _ptr(p_out, f64), 1 if kmode else 0,
-        st.cuda_stream if st.cuda_stream != 0 else _legacy_stream_handle())
+        _ptr(sigma, f64), _ptr(logL, f64), _ptr(p_out, f64), 1 if kmode else 0, _stream_handle(stream, dev))
     _lib.check(rc)
     return {"timeP": timeP, "p": p_out, "logL": logL}
 
 
-def _legacy_stream_handle():
+def _stream_handle(stream, device):
+    """The C ABI's handle of `stream` (default: torch's current stream on `device`)."""
+    st = stream if stream is not None else torch.cuda.current_stream(device)
     # torch's default stream is the legacy stream (handle 0).  The C ABI reads NULL as "use the
     # library's own stream and synchronise", so name the legacy stream explicitly instead.
-    return 1  # cudaStreamLegacy
+    return st.cuda_stream if st.cuda_stream != 0 else 1  # cudaStreamLegacy
 
 
 def _check_grad_shapes(vels, depths, nlayers, src_offset, src_depth, per_ray):
@@ -111,11 +111,10 @@ def dff_grad_device(vels, depths, nlayers, src_offset, src_depth, timeP, p, w, g
         dtdr = torch.empty((B, S), dtype=f64, device=dev)
     if want_src and dtdd is None:
         dtdd = torch.empty((B, S), dtype=f64, device=dev)
-    st = stream if stream is not None else torch.cuda.current_stream(dev)
     rc = _lib.load().rtb200_dff_grad_device(
         _ptr(vels, f64), _ptr(depths, f64) if ldz else None, _ptr(nlayers, torch.int32), B, ldv, ldz,
         _ptr(src_offset, f64), _ptr(src_depth, f64), S, _ptr(timeP, f64), _ptr(p, f64), _ptr(w, f64),
         _ptr(gvels, f64), _ptr(gdepths, f64) if ldz else None, _ptr(dtdr, f64), _ptr(dtdd, f64),
-        1 if kmode else 0, st.cuda_stream if st.cuda_stream != 0 else _legacy_stream_handle())
+        1 if kmode else 0, _stream_handle(stream, dev))
     _lib.check(rc)
     return {"gvels": gvels, "gdepths": gdepths, "dtdr": dtdr, "dtdd": dtdd}
