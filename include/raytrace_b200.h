@@ -124,6 +124,16 @@ int dff_batch_grad(const double *vels, const double *depths, const int *nlayers,
                    const double *w, double *timeP, double *p_out,
                    double *gvels, double *gdepths, double *dtdr, double *dtdd);
 
+/* dff_batch and the Jacobian of its travel times in one call (host pointers, scalars by
+ * reference): the forward, then rtb200_dff_jac_device.  jvels [B][NSrc][ldv] and
+ * jdepths [B][NSrc][ldz] receive dT/dV and dT/dz per ray; timeP, p_out, dtdr and dtdd
+ * [B][NSrc] may each be NULL.  No kmode.  Returns 0, or a non-zero status (see
+ * rtb200_last_error()). */
+int dff_batch_jac(const double *vels, const double *depths, const int *nlayers, const int *B,
+                  const int *ldv, const int *ldz, const double *src_offset,
+                  const double *src_depth, const int *NSrc, double *timeP, double *p_out,
+                  double *jvels, double *jdepths, double *dtdr, double *dtdd);
+
 /* LOGLHOOD / LOGLHOOD_RT (loglhood.f90:3-32,35-211) over B chain states, with the model
  * mapping of :127-146: state b has k[b] Voronoi nodes, vp[b][0..k-1] = voro(1:k,2),
  * ziface[b][0..k-2] = ziface(1:k-1); k == 1 becomes two equal velocities over one fake
@@ -192,6 +202,24 @@ int rtb200_dff_grad_device(const double *d_vels, const double *d_depths, const i
                            const double *d_timeP, const double *d_p, const double *d_w,
                            double *d_gvels, double *d_gdepths, double *d_dtdr, double *d_dtdd,
                            int kmode, void *stream);
+
+/* Jacobian of the travel times with respect to the layered model, per ray (DESIGN.md section 12):
+ * the terms rtb200_dff_grad_device sums over the sources, written unsummed.  Inputs as for that
+ * entry, without w.  Out:
+ *   jvels      [B][NSrc][ldv]  dT_bs/dV_i: n >= 2 layers and i < n: -H_i / (V_i^2 cos_i);
+ *                              a top-layer ray (n = 1): -T/V_0 at i = 0
+ *   jdepths    [B][NSrc][ldz]  dT_bs/dz_j = eta_j - eta_{j+1} for j <= n - 2 (kmode: ziface)
+ *   dtdr, dtdd [B][NSrc]       or NULL: as rtb200_dff_grad_device writes them
+ * Every other entry is 0, and so is the row of a ray with timeP = -999.  At k = 1 (kmode)
+ * jvels[b][s][0] is the sum of both layers' terms and jdepths is 0.  Each term is rounded as in
+ * rtb200_dff_grad_device, so that entry with a one-hot w returns the ray's row bit for bit.
+ * jdepths may be NULL when ldz = 0.  Stream semantics of rtb200_dff_batch_device. */
+int rtb200_dff_jac_device(const double *d_vels, const double *d_depths, const int *d_nlayers,
+                          int B, int ldv, int ldz,
+                          const double *d_src_offset, const double *d_src_depth, int NSrc,
+                          const double *d_timeP, const double *d_p, double *d_jvels,
+                          double *d_jdepths, double *d_dtdr, double *d_dtdd, int kmode,
+                          void *stream);
 
 /* One fixed-dimension Metropolis-Hastings move of B independent chains, entirely on the device:
  * PROPOSAL (prjmh_temper_rf.f90:1386-1447, ENOS = 0: Cauchy step on voro(ivo,iwhich), |.| for a

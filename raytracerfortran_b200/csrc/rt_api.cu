@@ -1160,6 +1160,134 @@ int dff_batch_grad(const double *vels, const double *depths, const int *nlayers,
     return 0;
 }
 
+namespace {
+
+// The argument checks both Jacobian entries share; timeP and p are checked by the device entry,
+// whose inputs they are.
+int check_jac_args(int ldv, int ldz, const void *vels, const void *nlayers, const void *off,
+                   const void *dep, const void *jvels, const void *jdepths) {
+    if (ldv < 1) return fail("ldv must be >= 1");
+    if (ldv > 255) return fail("more than 254 interfaces per model are not supported");
+    if (!vels || !nlayers || !jvels) return fail("the Jacobian needs vels, nlayers and jvels");
+    if (ldz > 0 && !jdepths) return fail("the Jacobian needs jdepths when ldz > 0");
+    if (!off || !dep) return fail("the Jacobian needs src_offset and src_depth");
+    return 0;
+}
+
+rtb::JacArgs jac_args(const double *vels, const double *depths, const int *nlayers, int B, int ldv,
+                      int ldz, const double *off, const double *dep, int nsrc, const double *timeP,
+                      const double *p, double *jvels, double *jdepths, double *dtdr, double *dtdd,
+                      int kmode) {
+    rtb::JacArgs a{};
+    a.vels = vels; a.depths = depths; a.nlayers = nlayers;
+    a.B = B; a.ldv = ldv; a.ldz = ldz; a.kmode = kmode;
+    a.src_offset = off; a.src_depth = dep; a.nsrc = nsrc;
+    a.timeP = timeP; a.p = p;
+    a.jvels = jvels; a.jdepths = jdepths; a.dtdr = dtdr; a.dtdd = dtdd;
+    return a;
+}
+
+}  // namespace
+
+int rtb200_dff_jac_device(const double *d_vels, const double *d_depths, const int *d_nlayers,
+                          int B, int ldv, int ldz, const double *d_src_offset,
+                          const double *d_src_depth, int NSrc, const double *d_timeP,
+                          const double *d_p, double *d_jvels, double *d_jdepths, double *d_dtdr,
+                          double *d_dtdd, int kmode, void *stream) {
+    ApiLock api_lock_;
+    if (int rc = ensure_init()) return rc;
+    g.err.clear();
+    if (B <= 0 || NSrc <= 0) return 0;
+    ldz = std::max(ldz, 0);
+    if (int rc = check_jac_args(ldv, ldz, d_vels, d_nlayers, d_src_offset, d_src_depth, d_jvels,
+                                d_jdepths))
+        return rc;
+    if (!d_timeP || !d_p) return fail("the Jacobian needs the forward's timeP and p");
+    cudaStream_t st = stream ? (cudaStream_t)stream : g.s_comp;
+    const rtb::JacArgs a = jac_args(d_vels, d_depths, d_nlayers, B, ldv, ldz, d_src_offset,
+                                    d_src_depth, NSrc, d_timeP, d_p, d_jvels, d_jdepths, d_dtdr,
+                                    d_dtdd, kmode);
+    CK(cudaEventRecord(g.ev_k0[0], st));
+    CK(rtb::launch_jac(a, st));
+    CK(cudaEventRecord(g.ev_k1[0], st));
+    g.launches++;
+    if (!stream) {
+        CK(cudaStreamSynchronize(st));
+        float ms = 0.f;
+        CK(cudaEventElapsedTime(&ms, g.ev_k0[0], g.ev_k1[0]));
+        g.kernel_ms = g.total_ms = ms;
+    }
+    return 0;
+}
+
+int dff_batch_jac(const double *vels, const double *depths, const int *nlayers, const int *B,
+                  const int *ldv, const int *ldz, const double *src_offset,
+                  const double *src_depth, const int *NSrc, double *timeP, double *p_out,
+                  double *jvels, double *jdepths, double *dtdr, double *dtdd) {
+    ApiLock api_lock_;
+    if (int rc = ensure_init()) return rc;
+    g.err.clear();
+    g.kernel_ms = g.total_ms = 0.0;
+    const int nb = *B, lv = *ldv, lz = std::max(*ldz, 0), ns = *NSrc;
+    if (nb <= 0 || ns <= 0) return 0;
+    if (int rc = check_jac_args(lv, lz, vels, nlayers, src_offset, src_depth, jvels, jdepths))
+        return rc;
+    const size_t Bz = (size_t)nb, S = (size_t)ns;
+    TileCfg cfg{};
+    if (int rc = choose_cfg(nb, lv, lz, ns, true, cfg)) return rc;
+    // copy in, forward, Jacobian, copy out; our buffers are padded to whole tiles as in run_host
+    const size_t M = (size_t)cfg.M, Bpad = (Bz + M - 1) / M * M + M;
+    CK(g.vels.reserve(Bpad * lv * 8));
+    CK(g.depths.reserve(Bpad * std::max(lz, 1) * 8));
+    CK(g.nl.reserve(Bpad * 4));
+    CK(g.off.reserve(S * 8));
+    CK(g.dep.reserve(S * 8));
+    CK(g.timeP.reserve(Bz * S * 8));
+    CK(g.pout.reserve(Bz * S * 8));
+    CK(g.ggv.reserve(Bz * S * lv * 8));
+    if (lz > 0) CK(g.ggz.reserve(Bz * S * lz * 8));
+    if (dtdr) CK(g.gdr.reserve(Bz * S * 8));
+    if (dtdd) CK(g.gdd.reserve(Bz * S * 8));
+    cudaStream_t st = g.s_comp;
+    if (int rc = scratch_acquire(st)) return rc;
+    CK(cudaMemcpyAsync(g.vels.p, vels, Bz * lv * 8, cudaMemcpyHostToDevice, st));
+    if (lz > 0) CK(cudaMemcpyAsync(g.depths.p, depths, Bz * lz * 8, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(g.nl.p, nlayers, Bz * 4, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(g.off.p, src_offset, S * 8, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(g.dep.p, src_depth, S * 8, cudaMemcpyHostToDevice, st));
+    CK(cudaEventRecord(g.ev_k0[0], st));
+    BatchArgs a{};
+    a.vels = g.vels.as<double>(); a.depths = g.depths.as<double>(); a.nlayers = g.nl.as<int>();
+    a.B = nb; a.ldv = lv; a.ldz = lz; a.kmode = 0;
+    a.src_offset = g.off.as<double>(); a.src_depth = g.dep.as<double>(); a.nsrc = ns;
+    a.timeP = g.timeP.as<double>(); a.p_out = g.pout.as<double>();
+    a.padded = 1;
+    a.sched = next_sched();
+    CK(rtb::launch_batch(a, cfg, st));
+    g.launches++;
+    g.last = cfg;
+    const rtb::JacArgs ja = jac_args(g.vels.as<double>(), g.depths.as<double>(), g.nl.as<int>(), nb, lv,
+                                     lz, g.off.as<double>(), g.dep.as<double>(), ns, g.timeP.as<double>(),
+                                     g.pout.as<double>(), g.ggv.as<double>(),
+                                     lz > 0 ? g.ggz.as<double>() : nullptr,
+                                     dtdr ? g.gdr.as<double>() : nullptr,
+                                     dtdd ? g.gdd.as<double>() : nullptr, 0);
+    CK(rtb::launch_jac(ja, st));
+    CK(cudaEventRecord(g.ev_k1[0], st));
+    g.launches++;
+    CK(cudaMemcpyAsync(jvels, g.ggv.p, Bz * S * lv * 8, cudaMemcpyDeviceToHost, st));
+    if (lz > 0) CK(cudaMemcpyAsync(jdepths, g.ggz.p, Bz * S * lz * 8, cudaMemcpyDeviceToHost, st));
+    if (timeP) CK(cudaMemcpyAsync(timeP, g.timeP.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
+    if (p_out) CK(cudaMemcpyAsync(p_out, g.pout.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
+    if (dtdr) CK(cudaMemcpyAsync(dtdr, g.gdr.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
+    if (dtdd) CK(cudaMemcpyAsync(dtdd, g.gdd.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (int rc = scratch_release(st, true)) return rc;
+    float ms = 0.f;
+    if (cudaEventElapsedTime(&ms, g.ev_k0[0], g.ev_k1[0]) == cudaSuccess) g.kernel_ms = g.total_ms = ms;
+    return 0;
+}
+
 extern "C++" {   // the helpers below include templates
 namespace {
 

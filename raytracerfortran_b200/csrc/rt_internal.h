@@ -62,6 +62,25 @@ struct GradArgs {
     double       *dtdd;        // [B][nsrc] or null: dT/d(depth)
 };
 
+// One launch of the Jacobian kernel (the per-ray terms the gradient kernel sums, DESIGN.md
+// section 12).  Every pointer is a device pointer; inputs as in GradArgs.
+struct JacArgs {
+    const double *vels;        // [B][ldv]
+    const double *depths;      // [B][ldz]
+    const int    *nlayers;     // [B]; kmode: node counts k
+    int           B, ldv, ldz;
+    int           kmode;
+    const double *src_offset;  // [nsrc]
+    const double *src_depth;   // [nsrc]
+    int           nsrc;
+    const double *timeP;       // [B][nsrc] the batch kernel's travel times
+    const double *p;           // [B][nsrc] and ray parameters
+    double       *jvels;       // [B][nsrc][ldv]  dT_bs/dV_i
+    double       *jdepths;     // [B][nsrc][ldz]  dT_bs/dz_j (null when ldz = 0)
+    double       *dtdr;        // [B][nsrc] or null: dT/d(offset)
+    double       *dtdd;        // [B][nsrc] or null: dT/d(depth)
+};
+
 // Tile geometry chosen by the host for one launch.
 struct TileCfg {
     int M;        // models per tile (even unless forced by the tile_models option)
@@ -131,6 +150,7 @@ cudaError_t launch_mcmc_finish(unsigned long long *counter, const int *k, int *p
 size_t      tile_smem_bytes(const TileCfg &c, int ldv, int ldz);
 cudaError_t launch_batch(const BatchArgs &a, const TileCfg &c, cudaStream_t st);
 cudaError_t launch_grad(const GradArgs &a, cudaStream_t st);
+cudaError_t launch_jac(const JacArgs &a, cudaStream_t st);
 cudaError_t launch_prep_voro(const int *k, const double *voro, int B, int ldk, double *vels,
                              double *depths, double *sorted, cudaStream_t st);
 cudaError_t launch_propose_voro(const int *k, const double *voro, int B, int ldk, const int *ivo,

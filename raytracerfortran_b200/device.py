@@ -1,8 +1,8 @@
 """The ray-tracing path on tensors that already live in HBM.
 
 torch is used for device memory and streams only; the work is done by the sm_100a kernels in
-libraytrace_b200.so through rtb200_dff_batch_device and, for gradients, rtb200_dff_grad_device
-(include/raytrace_b200.h).
+libraytrace_b200.so through rtb200_dff_batch_device and, for derivatives, rtb200_dff_grad_device
+and rtb200_dff_jac_device (include/raytrace_b200.h).
 """
 import torch
 
@@ -118,3 +118,39 @@ def dff_grad_device(vels, depths, nlayers, src_offset, src_depth, timeP, p, w, g
         1 if kmode else 0, _stream_handle(stream, dev))
     _lib.check(rc)
     return {"gvels": gvels, "gdepths": gdepths, "dtdr": dtdr, "dtdd": dtdd}
+
+
+def dff_jac_device(vels, depths, nlayers, src_offset, src_depth, timeP, p, jvels=None, jdepths=None,
+                   want_src=False, dtdr=None, dtdd=None, kmode=False, stream=None):
+    """Jacobian of the travel times dff_batch_device returned (timeP, p [B, NSrc]), per ray, on the
+    GPU (rtb200_dff_jac_device; DESIGN.md section 12).
+
+    Returns {"jvels" [B, NSrc, ldv], "jdepths" [B, NSrc, ldz], "dtdr", "dtdd" [B, NSrc] or None}:
+    jvels[b, s, i] = dT[b, s]/dV_i, jdepths[b, s, j] = dT[b, s]/dz_j (kmode: ziface), dtdr / dtdd
+    as dff_grad_device returns them (want_src).  Asynchronous on `stream` (default: torch's
+    current stream)."""
+    B, ldv, ldz, S = _check_grad_shapes(vels, depths, nlayers, src_offset, src_depth,
+                                        {"timeP": timeP, "p": p, "dtdr": dtdr, "dtdd": dtdd})
+    for name, t, shape in (("jvels", jvels, (B, S, ldv)), ("jdepths", jdepths, (B, S, ldz))):
+        if t is not None and tuple(t.shape) != shape:
+            raise ValueError(f"{name} must be {list(shape)}, got {list(t.shape)}")
+    if not vels.is_cuda:
+        raise ValueError("dff_jac_device needs CUDA tensors (there is no CPU path)")
+    dev = vels.device
+    _ensure_device(dev.index if dev.index is not None else torch.cuda.current_device())
+    f64 = torch.float64
+    if jvels is None:
+        jvels = torch.empty((B, S, ldv), dtype=f64, device=dev)
+    if jdepths is None:
+        jdepths = torch.empty((B, S, ldz), dtype=f64, device=dev)
+    if want_src and dtdr is None:
+        dtdr = torch.empty((B, S), dtype=f64, device=dev)
+    if want_src and dtdd is None:
+        dtdd = torch.empty((B, S), dtype=f64, device=dev)
+    rc = _lib.load().rtb200_dff_jac_device(
+        _ptr(vels, f64), _ptr(depths, f64) if ldz else None, _ptr(nlayers, torch.int32), B, ldv, ldz,
+        _ptr(src_offset, f64), _ptr(src_depth, f64), S, _ptr(timeP, f64), _ptr(p, f64),
+        _ptr(jvels, f64), _ptr(jdepths, f64) if ldz else None, _ptr(dtdr, f64), _ptr(dtdd, f64),
+        1 if kmode else 0, _stream_handle(stream, dev))
+    _lib.check(rc)
+    return {"jvels": jvels, "jdepths": jdepths, "dtdr": dtdr, "dtdd": dtdd}

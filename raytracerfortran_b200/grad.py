@@ -9,6 +9,11 @@ derivatives are those of the exact travel-time function there, not of the solver
 iteration.  Gradients flow to vels, depths (kmode: vp nodes and ziface), src_offset, src_depth,
 and for loglhood to tobs and sigma; nlayers is not differentiable.  Every tensor is a CUDA
 tensor, float64 (nlayers int32).  Both functions are once differentiable.
+
+    J = jacobian(vels, depths, nlayers, src_offset, src_depth, kmode=False)  # dict, no graph
+
+returns the travel times with their per-ray derivatives (rtb200_dff_jac_device), the rows
+Gauss-Newton and linearised-uncertainty computations need.
 """
 import torch
 from torch.autograd.function import once_differentiable
@@ -106,6 +111,21 @@ def travel_times(vels, depths, nlayers, src_offset, src_depth, kmode=False):
     _check(vels, depths, nlayers, src_offset, src_depth)
     return _TravelTimes.apply(vels.contiguous(), depths.contiguous(), nlayers.contiguous(),
                               src_offset.contiguous(), src_depth.contiguous(), bool(kmode))
+
+
+def jacobian(vels, depths, nlayers, src_offset, src_depth, kmode=False, want_src=True):
+    """Travel times and their Jacobian per ray, without an autograd graph (DESIGN.md section 12).
+
+    Returns {"timeP", "p" [B, NSrc], "jvels" [B, NSrc, ldv], "jdepths" [B, NSrc, ldz],
+    "dtdr", "dtdd" [B, NSrc] (None unless want_src)}: jvels[b, s, i] = dT[b, s]/dV_i and
+    jdepths[b, s, j] = dT[b, s]/dz_j, the rows whose sums over s travel_times' backward forms.
+    timeP is dff_batch_device's, bit for bit."""
+    _check(vels, depths, nlayers, src_offset, src_depth)
+    with torch.no_grad():
+        args = tuple(t.detach().contiguous() for t in (vels, depths, nlayers, src_offset, src_depth))
+        out = device.dff_batch_device(*args, want_times=True, want_p=True, kmode=bool(kmode))
+        r = device.dff_jac_device(*args, out["timeP"], out["p"], want_src=want_src, kmode=bool(kmode))
+    return {"timeP": out["timeP"], "p": out["p"], **r}
 
 
 def loglhood(vels, depths, nlayers, src_offset, src_depth, tobs, sigma, kmode=False):

@@ -143,6 +143,38 @@ def dff_batch_grad(vels, depths, nlayers, src_offset, src_depth, w, want_times=F
     return {"gvels": gv, "gdepths": gz, "timeP": t, "p": p, "dtdr": dr, "dtdd": dd}
 
 
+def dff_batch_jac(vels, depths, nlayers, src_offset, src_depth, want_times=False, want_p=False,
+                  want_src=False):
+    """dff_batch and the Jacobian of its travel times in one call (DESIGN.md section 12).
+
+    Returns a dict with "jvels" [B, NSrc, ldv] = dT/dV and "jdepths" [B, NSrc, ldz] = dT/dz per
+    ray, and, on request, "timeP" / "p" [B, NSrc] of the forward and "dtdr" / "dtdd" [B, NSrc],
+    the per-ray derivatives with respect to the source offset and depth (None otherwise)."""
+    v = _d(vels)
+    z = _d(depths)
+    if v.ndim != 2 or z.ndim != 2 or v.shape[0] != z.shape[0]:
+        raise ValueError("vels and depths must be [B, ldv] and [B, ldz]")
+    nl = np.ascontiguousarray(nlayers, dtype=np.int32)
+    so, sd = _d(src_offset), _d(src_depth)
+    B, ldv, ldz, nsrc = v.shape[0], v.shape[1], z.shape[1], so.size
+    if nl.shape != (B,) or so.ndim != 1 or sd.shape != so.shape:
+        raise ValueError("nlayers must be [B], src_offset and src_depth [NSrc]")
+    if not 1 <= ldv <= 255:
+        raise ValueError("ldv must be 1..255 (at most 254 interfaces)")
+    if B and (nl.min() < 0 or int(nl.max()) + 1 > ldv or int(nl.max()) > ldz):
+        raise ValueError("nlayers exceeds the row length of vels / depths")
+    jv, jz = np.empty((B, nsrc, ldv)), np.empty((B, nsrc, ldz))
+    t = np.empty((B, nsrc)) if want_times else None
+    p = np.empty((B, nsrc)) if want_p else None
+    dr = np.empty((B, nsrc)) if want_src else None
+    dd = np.empty((B, nsrc)) if want_src else None
+    rc = _lib.load().dff_batch_jac(_p(v), _p(z), nl.ctypes.data_as(_IP), _ci(B), _ci(ldv), _ci(ldz),
+                                   _p(so), _p(sd), _ci(nsrc), _p(t), _p(p), _p(jv), _p(jz), _p(dr),
+                                   _p(dd))
+    _lib.check(rc)
+    return {"jvels": jv, "jdepths": jz, "timeP": t, "p": p, "dtdr": dr, "dtdd": dd}
+
+
 def loglhood_batch(k, voro_vp, ziface, src_offset, src_depth, DobsRT, sdparRT, want_pred=False):
     """LOGLHOOD / LOGLHOOD_RT (loglhood.f90:3-32,35-211) over B chain states.
 
