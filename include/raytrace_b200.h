@@ -420,7 +420,7 @@ int         rtb200_device_count(void);        /* 0 without a driver / device    
  *          "latency_path" (1 default: a one-model call without likelihood -- dff_, TraceRays --
  *          runs the one-warp-per-ray kernel on mapped pinned memory; 0: the batch kernel);
  *          "stable_lognorm" (0 default: LOG(1/(2 PI2)**(N/2)) as loglhood.f90:194 writes it, which
- *          is -Inf for N >= 772 sources; 1: the same constant as -(N/2) LOG(2 PI2), finite for any
+ *          is -Inf for N >= 773 sources; 1: the same constant as -(N/2) LOG(2 PI2), finite for any
  *          N -- a deviation from the reference, for likelihoods over more than 771 data);
  *          "ismpprior" (ISMPPRIOR of the parameter file: 1 = the chain move entries sample the
  *          prior -- every proposal's likelihood is LOGLHOOD2's constant 1, loglhood.f90:704-716,

@@ -10,7 +10,7 @@ data path; the timed region is bracketed by barriers and the time is the max ove
 
 Checks on every rank: a sample of models re-evaluated alone gives the same bits (batch invariance)
 and matches the CPU oracle bit for bit in travel time.  --stable-norm switches on the opt-in
-overflow-free normaliser -(N/2) log(2 pi) (the reference's (2 pi)^(N/2) overflows for N >= 772 and
+overflow-free normaliser -(N/2) log(2 pi) (the reference's (2 pi)^(N/2) overflows for N >= 773 and
 every logL is -inf, loglhood.f90:194; default: reproduce that)."""
 import json
 import os

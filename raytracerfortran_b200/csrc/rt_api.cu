@@ -102,7 +102,7 @@ struct Ctx {
     void  *lat = nullptr;
     size_t lat_cap = 0;
     int opt_latency = 1;           // 1: one-model calls take the latency kernel; 0: the batch kernel
-    int opt_stable_lognorm = 0;    // 1: log-likelihood constant as -(N/2) log(2 pi) (finite for N >= 772)
+    int opt_stable_lognorm = 0;    // 1: log-likelihood constant as -(N/2) log(2 pi) (finite for N >= 773)
     int opt_ismpprior = 0;         // 1: the chain moves sample the prior (LOGLHOOD2: logL = 1)
     // options (<= 0: automatic)
     int opt_variant = -1, opt_threads = 0, opt_tile_models = 0, opt_tile_sources = 0,
@@ -289,7 +289,7 @@ int choose_cfg(int B, int ldv, int ldz, int nsrc, bool aligned, TileCfg &c) {
 
 double log_norm_const(int nsrc) {
     // LOG(1._RP/(2._RP*PI2)**(REAL(NDAT_RT,RP)/2._RP))     loglhood.f90:194
-    // For NDAT_RT >= 772 the power overflows, 1/Inf = 0 and the reference's logL is -Inf for every
+    // For NDAT_RT >= 773 the power overflows, 1/Inf = 0 and the reference's logL is -Inf for every
     // model; that is reproduced by default.  Option "stable_lognorm" (a documented deviation, off
     // by default) evaluates the same constant as -(N/2) LOG(2 PI2), which stays finite.
     const double n = (double)nsrc;

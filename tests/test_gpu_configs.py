@@ -84,7 +84,7 @@ def test_config5_stress_slice():
     only_ll = rt.dff_batch(v, z, nl, so, sd, tobs=tobs, sigma=sigma, want_times=False)
     assert np.array_equal(only_ll["logL"], got["logL"])
     assert np.all(np.isneginf(got["logL"]))
-    # opt-in deviation: the same constant as -(N/2) log(2 pi) keeps logL finite for N >= 772
+    # opt-in deviation: the same constant as -(N/2) log(2 pi) keeps logL finite for N >= 773
     rt.set_option("stable_lognorm", 1)
     try:
         st = rt.dff_batch(v[pick], z[pick], nl[pick], so, sd, tobs=tobs, sigma=sigma[pick], want_times=True)

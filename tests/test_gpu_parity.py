@@ -166,7 +166,7 @@ def test_transdimensional_loglhood_batch():
 
 
 def test_loglhood_overflowing_normaliser_is_minus_inf_like_the_reference():
-    """(2 pi)^(N/2) overflows for N >= 772, so LOG(1/inf) = -inf (loglhood.f90:194)."""
+    """(2 pi)^(N/2) overflows for N >= 773, so LOG(1/inf) = -inf (loglhood.f90:194)."""
     B, nsrc = 6, 800
     v, z, nl = workloads.make_models(B, 6, 9)
     so, sd = workloads.make_sources(nsrc, 9)
