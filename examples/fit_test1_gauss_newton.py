@@ -1,10 +1,11 @@
 #!/usr/bin/env python
-"""Fit the test_1 model from many starts with Levenberg-Marquardt on the per-ray Jacobian
-(raytracerfortran_b200.grad.jacobian), in torch on the GPU.
+"""Fit the test_1 model from many starts with Levenberg-Marquardt on the per-model normal equations
+(raytracerfortran_b200.grad.normal_equations), in torch on the GPU.
 
 1024 starts are perturbed as in fit_test1_gradient.py (velocities +-10 %, interfaces +-50 m, the
-number of layers fixed).  The unknowns are slowness (s/km) and interface depth (km), as there; the
-chain rule turns the library's dT/dV and dT/dz into the columns of J for them.  Every start has its
+number of layers fixed).  The unknowns are slowness (s/km) and interface depth (km), as there; for
+them the library's J^T J and J^T r in V and z become S J^T J S and S J^T r with the diagonal chain
+rule S = diag(-V^2 / 1000, 1000).  The Jacobian itself is never stored.  Every start has its
 own damping lambda: its step solves (J^T J + lambda D) dx = J^T r with D = diag(J^T J), and it
 keeps the step only if its own logL rises (then lambda shrinks, otherwise it grows).  All steps of
 an iteration are one torch.linalg.solve on [B, P, P].  Prints the best logL against the true
@@ -57,12 +58,12 @@ def main():
     P = x.shape[1]
     model = lambda x: (1000.0 / x[:, :nv], (x[:, nv:] * 1000.0).contiguous())
 
-    def jac_and_residual(x):
+    def normal_equations(x):
         v, z = model(x)
-        J = grad.jacobian(v, z, nl[:v.shape[0]], so, sd, want_src=False)
+        N = grad.normal_equations(v, z, nl[:v.shape[0]], so, sd, tobs=tobs)
         # dT/ds = dT/dV dV/ds = -dT/dV V^2 / 1000,  dT/dz_km = 1000 dT/dz
-        Jx = torch.cat([J["jvels"] * (-(v * v) / 1000.0)[:, None, :], J["jdepths"] * 1000.0], 2)
-        return Jx, tobs[None, :] - J["timeP"]
+        S = torch.cat([-(v * v) / 1000.0, torch.full_like(z, 1000.0)], 1)
+        return S[:, :, None] * N["JtJ"] * S[:, None, :], S * N["Jtr"]
 
     L = logl(*model(x))
     l_start = L.clone()
@@ -70,9 +71,7 @@ def main():
     eye = torch.eye(P, dtype=f64, device=dev)
     it, quiet = 0, 0
     for it in range(1, args.iters + 1):
-        J, r = jac_and_residual(x)
-        A = J.transpose(1, 2) @ J
-        g = (J.transpose(1, 2) @ r[:, :, None])[:, :, 0]
+        A, g = normal_equations(x)
         D = torch.diagonal(A, dim1=1, dim2=2)
         D = torch.maximum(D, 1e-12 * D.amax(1, keepdim=True))
         dx = torch.linalg.solve(A + lam[:, None, None] * D[:, :, None] * eye, g[:, :, None])[:, :, 0]
@@ -93,8 +92,8 @@ def main():
           f"median start {l_start.median().item():.3f}")
     print(f"starts ending within 1 of the true model's logL: {within} of {B}")
     vb, zb = model(x[best:best + 1])
-    J, _ = jac_and_residual(x[best:best + 1])
-    cov = torch.linalg.inv(J[0].T @ J[0] / (sigma[0] * sigma[0]))
+    A, _ = normal_equations(x[best:best + 1])
+    cov = torch.linalg.inv(A[0] / (sigma[0] * sigma[0]))
     sd_x = torch.sqrt(torch.diagonal(cov))
     sd_v = sd_x[:nv] * (vb[0] * vb[0]) / 1000.0             # |dV/ds| = V^2 / 1000
     sd_z = sd_x[nv:] * 1000.0

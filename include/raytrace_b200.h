@@ -134,6 +134,15 @@ int dff_batch_jac(const double *vels, const double *depths, const int *nlayers, 
                   const double *src_depth, const int *NSrc, double *timeP, double *p_out,
                   double *jvels, double *jdepths, double *dtdr, double *dtdd);
 
+/* dff_batch and the Gauss-Newton normal equations of its travel times in one call (host pointers,
+ * scalars by reference): the forward, then rtb200_dff_normal_device.  JtJ [B][P][P], P = ldv + ldz;
+ * tobs [NSrc] and Jtr [B][P] are both given or both NULL; timeP and p_out [B][NSrc] may each be
+ * NULL.  No kmode.  Returns 0, or a non-zero status (see rtb200_last_error()). */
+int dff_batch_normal(const double *vels, const double *depths, const int *nlayers, const int *B,
+                     const int *ldv, const int *ldz, const double *src_offset,
+                     const double *src_depth, const int *NSrc, const double *tobs, double *timeP,
+                     double *p_out, double *JtJ, double *Jtr);
+
 /* LOGLHOOD / LOGLHOOD_RT (loglhood.f90:3-32,35-211) over B chain states, with the model
  * mapping of :127-146: state b has k[b] Voronoi nodes, vp[b][0..k-1] = voro(1:k,2),
  * ziface[b][0..k-2] = ziface(1:k-1); k == 1 becomes two equal velocities over one fake
@@ -220,6 +229,27 @@ int rtb200_dff_jac_device(const double *d_vels, const double *d_depths, const in
                           const double *d_timeP, const double *d_p, double *d_jvels,
                           double *d_jdepths, double *d_dtdr, double *d_dtdd, int kmode,
                           void *stream);
+
+/* Gauss-Newton normal equations of the travel times, per model (DESIGN.md section 13), without
+ * storing the Jacobian.  Inputs as for rtb200_dff_jac_device, plus the observations d_tobs [NSrc].
+ * With J_s = [jvels[b][s][:] | jdepths[b][s][:]] the row rtb200_dff_jac_device writes for ray
+ * (b, s), P = ldv + ldz and r_s = tobs_s - timeP[b][s]:
+ *   JtJ  [B][P][P]  sum_s J_si J_sj
+ *   Jtr  [B][P]     sum_s J_si r_s
+ * Each sum runs over s in increasing order from +0.0, one rounded multiply and one rounded add a
+ * term (no FMA), and takes only the terms whose columns the ray reaches: velocity column i < n
+ * (kmode k = 1: column 0 when n >= 1), depth column j <= n - 2 (none at k = 1), nothing for a ray
+ * with timeP = -999.  So the result depends on no launch geometry, JtJ is exactly symmetric, and
+ * a column no ray of a model reaches is a zero row and column: JtJ is then singular, and a
+ * damped solve (Levenberg-Marquardt) is the caller's remedy.  No weights: with one sigma per
+ * model the caller scales the result by 1 / sigma^2.  d_tobs and d_Jtr are NULL together.
+ * NSrc = 0 gives zeros; the source arrays, timeP, p and d_tobs may then be NULL.  Stream
+ * semantics of rtb200_dff_batch_device. */
+int rtb200_dff_normal_device(const double *d_vels, const double *d_depths, const int *d_nlayers,
+                             int B, int ldv, int ldz, const double *d_src_offset,
+                             const double *d_src_depth, int NSrc, const double *d_timeP,
+                             const double *d_p, const double *d_tobs, double *d_JtJ,
+                             double *d_Jtr, int kmode, void *stream);
 
 /* One fixed-dimension Metropolis-Hastings move of B independent chains, entirely on the device:
  * PROPOSAL (prjmh_temper_rf.f90:1386-1447, ENOS = 0: Cauchy step on voro(ivo,iwhich), |.| for a

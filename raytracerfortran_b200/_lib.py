@@ -12,8 +12,8 @@ LIB_PATH = os.environ.get("RTB200_LIB") or os.path.join(_HERE, "libraytrace_b200
 
 # every symbol include/raytrace_b200.h declares
 EXPORTS = (
-    "dff_", "dff7_", "tracerays_", "__raymod_MOD_tracerays", "raymod_mp_tracerays_", "raymod_tracerays_", "dff_batch", "dff_batch_grad", "dff_batch_jac", "dff_batch_status", "dff_batch_status_", "loglhood_batch", "loglhood_batch_ar", "loglhood_batch_voro",
-    "rtb200_dff_batch_device", "rtb200_dff_grad_device", "rtb200_dff_jac_device", "rtb200_mh_step_device", "rtb200_mh_step_device_ev", "rtb200_mh_moves_device", "rtb200_mh_moves_device_ex", "rtb200_bd_step_device_ex", "rtb200_bd_step_device", "rtb200_sd_step_device", "rtb200_ar_step_device", "rtb200_set_chain_ar",
+    "dff_", "dff7_", "tracerays_", "__raymod_MOD_tracerays", "raymod_mp_tracerays_", "raymod_tracerays_", "dff_batch", "dff_batch_grad", "dff_batch_jac", "dff_batch_normal", "dff_batch_status", "dff_batch_status_", "loglhood_batch", "loglhood_batch_ar", "loglhood_batch_voro",
+    "rtb200_dff_batch_device", "rtb200_dff_grad_device", "rtb200_dff_jac_device", "rtb200_dff_normal_device", "rtb200_mh_step_device", "rtb200_mh_step_device_ev", "rtb200_mh_moves_device", "rtb200_mh_moves_device_ex", "rtb200_bd_step_device_ex", "rtb200_bd_step_device", "rtb200_sd_step_device", "rtb200_ar_step_device", "rtb200_set_chain_ar",
     "rtb200_swap_pack_device", "rtb200_swap_round_device", "rtb200_mcmc_workspace_bytes", "rtb200_mcmc_iterations_device",
     "rtb200_init", "rtb200_shutdown", "rtb200_last_error", "rtb200_device_count",
     "rtb200_set_option", "rtb200_get_stat", "rtb200_fp64_peak_tflops", "rtb200_shard_range",
@@ -68,6 +68,10 @@ def load():
     lib.rtb200_dff_jac_device.argtypes = [vp, vp, vp, i, i, i, vp, vp, i, vp, vp, vp, vp, vp, vp, i, vp]
     lib.dff_batch_jac.restype = i
     lib.dff_batch_jac.argtypes = [dp, dp, ip, ip, ip, ip, dp, dp, ip, dp, dp, dp, dp, dp, dp]
+    lib.rtb200_dff_normal_device.restype = i
+    lib.rtb200_dff_normal_device.argtypes = [vp, vp, vp, i, i, i, vp, vp, i, vp, vp, vp, vp, vp, i, vp]
+    lib.dff_batch_normal.restype = i
+    lib.dff_batch_normal.argtypes = [dp, dp, ip, ip, ip, ip, dp, dp, ip, dp, dp, dp, dp, dp]
     lib.rtb200_mh_step_device.restype = i
     lib.rtb200_mh_step_device.argtypes = [vp, vp, vp, i, i, vp, vp, vp, vp, vp, vp, dp, vp, vp, vp, i, vp, vp]
     lib.rtb200_mh_step_device_ev.restype = i

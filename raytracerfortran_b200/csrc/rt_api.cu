@@ -1288,6 +1288,147 @@ int dff_batch_jac(const double *vels, const double *depths, const int *nlayers, 
     return 0;
 }
 
+namespace {
+
+// The argument checks both normal-equations entries share; timeP and p are checked by the device
+// entry, whose inputs they are.
+int check_normal_args(int ldv, int ldz, int nsrc, const void *vels, const void *nlayers,
+                      const void *off, const void *dep, const void *JtJ, const void *tobs,
+                      const void *Jtr) {
+    if (ldv < 1) return fail("ldv must be >= 1");
+    if (ldv > 255) return fail("more than 254 interfaces per model are not supported");
+    if (!vels || !nlayers || !JtJ) return fail("the normal equations need vels, nlayers and JtJ");
+    // empty source arrays may arrive as NULL: with no source there is nothing to read
+    if ((tobs && !Jtr) || (!tobs && Jtr && nsrc > 0)) return fail("tobs and Jtr must be given together");
+    if (nsrc > 0 && (!off || !dep)) return fail("the normal equations need src_offset and src_depth");
+    return 0;
+}
+
+rtb::NormalArgs normal_args(const double *vels, const double *depths, const int *nlayers, int B,
+                            int ldv, int ldz, const double *off, const double *dep, int nsrc,
+                            const double *timeP, const double *p, const double *tobs, double *JtJ,
+                            double *Jtr, int kmode) {
+    rtb::NormalArgs a{};
+    a.vels = vels; a.depths = depths; a.nlayers = nlayers;
+    a.B = B; a.ldv = ldv; a.ldz = ldz; a.kmode = kmode;
+    a.src_offset = off; a.src_depth = dep; a.nsrc = nsrc;
+    a.timeP = timeP; a.p = p; a.tobs = tobs;
+    a.JtJ = JtJ; a.Jtr = Jtr;
+    return a;
+}
+
+}  // namespace
+
+int rtb200_dff_normal_device(const double *d_vels, const double *d_depths, const int *d_nlayers,
+                             int B, int ldv, int ldz, const double *d_src_offset,
+                             const double *d_src_depth, int NSrc, const double *d_timeP,
+                             const double *d_p, const double *d_tobs, double *d_JtJ,
+                             double *d_Jtr, int kmode, void *stream) {
+    ApiLock api_lock_;
+    if (int rc = ensure_init()) return rc;
+    g.err.clear();
+    if (B <= 0) return 0;
+    ldz = std::max(ldz, 0);
+    if (int rc = check_normal_args(ldv, ldz, NSrc, d_vels, d_nlayers, d_src_offset, d_src_depth,
+                                   d_JtJ, d_tobs, d_Jtr))
+        return rc;
+    if (NSrc > 0 && (!d_timeP || !d_p)) return fail("the normal equations need the forward's timeP and p");
+    cudaStream_t st = stream ? (cudaStream_t)stream : g.s_comp;
+    const size_t P = (size_t)(ldv + ldz);
+    CK(cudaEventRecord(g.ev_k0[0], st));
+    if (NSrc <= 0) {            // sums over no source
+        CK(cudaMemsetAsync(d_JtJ, 0, (size_t)B * P * P * 8, st));
+        if (d_Jtr) CK(cudaMemsetAsync(d_Jtr, 0, (size_t)B * P * 8, st));
+    } else {
+        const rtb::NormalArgs a = normal_args(d_vels, d_depths, d_nlayers, B, ldv, ldz, d_src_offset,
+                                              d_src_depth, NSrc, d_timeP, d_p, d_tobs, d_JtJ, d_Jtr,
+                                              kmode);
+        CK(rtb::launch_normal(a, st));
+        g.launches++;
+    }
+    CK(cudaEventRecord(g.ev_k1[0], st));
+    if (!stream) {
+        CK(cudaStreamSynchronize(st));
+        float ms = 0.f;
+        CK(cudaEventElapsedTime(&ms, g.ev_k0[0], g.ev_k1[0]));
+        g.kernel_ms = g.total_ms = ms;
+    }
+    return 0;
+}
+
+int dff_batch_normal(const double *vels, const double *depths, const int *nlayers, const int *B,
+                     const int *ldv, const int *ldz, const double *src_offset,
+                     const double *src_depth, const int *NSrc, const double *tobs, double *timeP,
+                     double *p_out, double *JtJ, double *Jtr) {
+    ApiLock api_lock_;
+    if (int rc = ensure_init()) return rc;
+    g.err.clear();
+    g.kernel_ms = g.total_ms = 0.0;
+    const int nb = *B, lv = *ldv, lz = std::max(*ldz, 0), ns = *NSrc;
+    if (nb <= 0) return 0;
+    if (int rc = check_normal_args(lv, lz, ns, vels, nlayers, src_offset, src_depth, JtJ, tobs, Jtr))
+        return rc;
+    const size_t Bz = (size_t)nb, P = (size_t)(lv + lz);
+    if (ns <= 0) {              // sums over no source
+        std::memset(JtJ, 0, Bz * P * P * 8);
+        if (Jtr) std::memset(Jtr, 0, Bz * P * 8);
+        return 0;
+    }
+    const size_t S = (size_t)ns;
+    TileCfg cfg{};
+    if (int rc = choose_cfg(nb, lv, lz, ns, true, cfg)) return rc;
+    // copy in, forward, normal equations, copy out; our buffers are padded to whole tiles as in run_host
+    const size_t M = (size_t)cfg.M, Bpad = (Bz + M - 1) / M * M + M;
+    CK(g.vels.reserve(Bpad * lv * 8));
+    CK(g.depths.reserve(Bpad * std::max(lz, 1) * 8));
+    CK(g.nl.reserve(Bpad * 4));
+    CK(g.off.reserve(S * 8));
+    CK(g.dep.reserve(S * 8));
+    CK(g.timeP.reserve(Bz * S * 8));
+    CK(g.pout.reserve(Bz * S * 8));
+    CK(g.ggv.reserve(Bz * P * P * 8));
+    if (tobs) {
+        CK(g.gdr.reserve(S * 8));
+        CK(g.ggz.reserve(Bz * P * 8));
+    }
+    cudaStream_t st = g.s_comp;
+    if (int rc = scratch_acquire(st)) return rc;
+    CK(cudaMemcpyAsync(g.vels.p, vels, Bz * lv * 8, cudaMemcpyHostToDevice, st));
+    if (lz > 0) CK(cudaMemcpyAsync(g.depths.p, depths, Bz * lz * 8, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(g.nl.p, nlayers, Bz * 4, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(g.off.p, src_offset, S * 8, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(g.dep.p, src_depth, S * 8, cudaMemcpyHostToDevice, st));
+    if (tobs) CK(cudaMemcpyAsync(g.gdr.p, tobs, S * 8, cudaMemcpyHostToDevice, st));
+    CK(cudaEventRecord(g.ev_k0[0], st));
+    BatchArgs a{};
+    a.vels = g.vels.as<double>(); a.depths = g.depths.as<double>(); a.nlayers = g.nl.as<int>();
+    a.B = nb; a.ldv = lv; a.ldz = lz; a.kmode = 0;
+    a.src_offset = g.off.as<double>(); a.src_depth = g.dep.as<double>(); a.nsrc = ns;
+    a.timeP = g.timeP.as<double>(); a.p_out = g.pout.as<double>();
+    a.padded = 1;
+    a.sched = next_sched();
+    CK(rtb::launch_batch(a, cfg, st));
+    g.launches++;
+    g.last = cfg;
+    const rtb::NormalArgs na = normal_args(g.vels.as<double>(), g.depths.as<double>(), g.nl.as<int>(), nb,
+                                           lv, lz, g.off.as<double>(), g.dep.as<double>(), ns,
+                                           g.timeP.as<double>(), g.pout.as<double>(),
+                                           tobs ? g.gdr.as<double>() : nullptr, g.ggv.as<double>(),
+                                           tobs ? g.ggz.as<double>() : nullptr, 0);
+    CK(rtb::launch_normal(na, st));
+    CK(cudaEventRecord(g.ev_k1[0], st));
+    g.launches++;
+    CK(cudaMemcpyAsync(JtJ, g.ggv.p, Bz * P * P * 8, cudaMemcpyDeviceToHost, st));
+    if (tobs) CK(cudaMemcpyAsync(Jtr, g.ggz.p, Bz * P * 8, cudaMemcpyDeviceToHost, st));
+    if (timeP) CK(cudaMemcpyAsync(timeP, g.timeP.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
+    if (p_out) CK(cudaMemcpyAsync(p_out, g.pout.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (int rc = scratch_release(st, true)) return rc;
+    float ms = 0.f;
+    if (cudaEventElapsedTime(&ms, g.ev_k0[0], g.ev_k1[0]) == cudaSuccess) g.kernel_ms = g.total_ms = ms;
+    return 0;
+}
+
 extern "C++" {   // the helpers below include templates
 namespace {
 

@@ -81,6 +81,24 @@ struct JacArgs {
     double       *dtdd;        // [B][nsrc] or null: dT/d(depth)
 };
 
+// One launch of the normal-equations kernel (DESIGN.md section 13).  Every pointer is a device
+// pointer; inputs as in JacArgs.  P = ldv + ldz parameter columns, [vels | depths].
+struct NormalArgs {
+    const double *vels;        // [B][ldv]
+    const double *depths;      // [B][ldz]
+    const int    *nlayers;     // [B]; kmode: node counts k
+    int           B, ldv, ldz;
+    int           kmode;
+    const double *src_offset;  // [nsrc]
+    const double *src_depth;   // [nsrc]
+    int           nsrc;
+    const double *timeP;       // [B][nsrc] the batch kernel's travel times
+    const double *p;           // [B][nsrc] and ray parameters
+    const double *tobs;        // [nsrc] or null (then Jtr is null)
+    double       *JtJ;         // [B][P][P]
+    double       *Jtr;         // [B][P] or null
+};
+
 // Tile geometry chosen by the host for one launch.
 struct TileCfg {
     int M;        // models per tile (even unless forced by the tile_models option)
@@ -151,6 +169,7 @@ size_t      tile_smem_bytes(const TileCfg &c, int ldv, int ldz);
 cudaError_t launch_batch(const BatchArgs &a, const TileCfg &c, cudaStream_t st);
 cudaError_t launch_grad(const GradArgs &a, cudaStream_t st);
 cudaError_t launch_jac(const JacArgs &a, cudaStream_t st);
+cudaError_t launch_normal(const NormalArgs &a, cudaStream_t st);
 cudaError_t launch_prep_voro(const int *k, const double *voro, int B, int ldk, double *vels,
                              double *depths, double *sorted, cudaStream_t st);
 cudaError_t launch_propose_voro(const int *k, const double *voro, int B, int ldk, const int *ivo,

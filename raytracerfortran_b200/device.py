@@ -1,8 +1,8 @@
 """The ray-tracing path on tensors that already live in HBM.
 
 torch is used for device memory and streams only; the work is done by the sm_100a kernels in
-libraytrace_b200.so through rtb200_dff_batch_device and, for derivatives, rtb200_dff_grad_device
-and rtb200_dff_jac_device (include/raytrace_b200.h).
+libraytrace_b200.so through rtb200_dff_batch_device and, for derivatives, rtb200_dff_grad_device,
+rtb200_dff_jac_device and rtb200_dff_normal_device (include/raytrace_b200.h).
 """
 import torch
 
@@ -154,3 +154,39 @@ def dff_jac_device(vels, depths, nlayers, src_offset, src_depth, timeP, p, jvels
         1 if kmode else 0, _stream_handle(stream, dev))
     _lib.check(rc)
     return {"jvels": jvels, "jdepths": jdepths, "dtdr": dtdr, "dtdd": dtdd}
+
+
+def dff_normal_device(vels, depths, nlayers, src_offset, src_depth, timeP, p, tobs=None, JtJ=None, Jtr=None,
+                      kmode=False, stream=None):
+    """Gauss-Newton normal equations of the travel times dff_batch_device returned (timeP, p
+    [B, NSrc]), per model, on the GPU without storing the Jacobian (rtb200_dff_normal_device;
+    DESIGN.md section 13).
+
+    Returns {"JtJ" [B, P, P], "Jtr" [B, P] or None}, P = ldv + ldz: with J the rows dff_jac_device
+    writes, [jvels | jdepths], JtJ = J^T J and, given tobs [NSrc], Jtr = J^T (tobs - timeP), each
+    sum in source order.  Asynchronous on `stream` (default: torch's current stream)."""
+    B, ldv, ldz, S = _check_grad_shapes(vels, depths, nlayers, src_offset, src_depth,
+                                        {"timeP": timeP, "p": p})
+    P = ldv + ldz
+    if tobs is not None and tuple(tobs.shape) != (S,):
+        raise ValueError(f"tobs must be [NSrc] = [{S}], got {list(tobs.shape)}")
+    if Jtr is not None and tobs is None:
+        raise ValueError("Jtr needs tobs")
+    for name, t, shape in (("JtJ", JtJ, (B, P, P)), ("Jtr", Jtr, (B, P))):
+        if t is not None and tuple(t.shape) != shape:
+            raise ValueError(f"{name} must be {list(shape)}, got {list(t.shape)}")
+    if not vels.is_cuda:
+        raise ValueError("dff_normal_device needs CUDA tensors (there is no CPU path)")
+    dev = vels.device
+    _ensure_device(dev.index if dev.index is not None else torch.cuda.current_device())
+    f64 = torch.float64
+    if JtJ is None:
+        JtJ = torch.empty((B, P, P), dtype=f64, device=dev)
+    if tobs is not None and Jtr is None:
+        Jtr = torch.empty((B, P), dtype=f64, device=dev)
+    rc = _lib.load().rtb200_dff_normal_device(
+        _ptr(vels, f64), _ptr(depths, f64) if ldz else None, _ptr(nlayers, torch.int32), B, ldv, ldz,
+        _ptr(src_offset, f64), _ptr(src_depth, f64), S, _ptr(timeP, f64), _ptr(p, f64), _ptr(tobs, f64),
+        _ptr(JtJ, f64), _ptr(Jtr, f64), 1 if kmode else 0, _stream_handle(stream, dev))
+    _lib.check(rc)
+    return {"JtJ": JtJ, "Jtr": Jtr}

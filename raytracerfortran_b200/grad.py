@@ -14,6 +14,11 @@ tensor, float64 (nlayers int32).  Both functions are once differentiable.
 
 returns the travel times with their per-ray derivatives (rtb200_dff_jac_device), the rows
 Gauss-Newton and linearised-uncertainty computations need.
+
+    N = normal_equations(vels, depths, nlayers, src_offset, src_depth, tobs=None, kmode=False)
+
+returns the travel times with the per-model normal equations J^T J and J^T (tobs - T) of those
+rows (rtb200_dff_normal_device), accumulated on the device without writing J.
 """
 import torch
 from torch.autograd.function import once_differentiable
@@ -125,6 +130,26 @@ def jacobian(vels, depths, nlayers, src_offset, src_depth, kmode=False, want_src
         args = tuple(t.detach().contiguous() for t in (vels, depths, nlayers, src_offset, src_depth))
         out = device.dff_batch_device(*args, want_times=True, want_p=True, kmode=bool(kmode))
         r = device.dff_jac_device(*args, out["timeP"], out["p"], want_src=want_src, kmode=bool(kmode))
+    return {"timeP": out["timeP"], "p": out["p"], **r}
+
+
+def normal_equations(vels, depths, nlayers, src_offset, src_depth, tobs=None, kmode=False):
+    """Travel times and the Gauss-Newton normal equations of their Jacobian, per model, without an
+    autograd graph (DESIGN.md section 13).
+
+    Returns {"timeP", "p" [B, NSrc], "JtJ" [B, P, P], "Jtr" [B, P] or None}, P = ldv + ldz: with
+    J_s = [jvels[b, s] | jdepths[b, s]] the rows jacobian() returns, JtJ[b] = sum_s J_s^T J_s and,
+    given tobs [NSrc], Jtr[b] = sum_s J_s^T (tobs_s - timeP[b, s]).  The Jacobian is never stored.
+    timeP is dff_batch_device's, bit for bit."""
+    _, S = _check(vels, depths, nlayers, src_offset, src_depth)
+    if tobs is not None and (tobs.dtype != torch.float64 or tuple(tobs.shape) != (S,)):
+        raise ValueError(f"tobs must be a float64 [NSrc] = [{S}] tensor")
+    with torch.no_grad():
+        args = tuple(t.detach().contiguous() for t in (vels, depths, nlayers, src_offset, src_depth))
+        out = device.dff_batch_device(*args, want_times=True, want_p=True, kmode=bool(kmode))
+        r = device.dff_normal_device(*args, out["timeP"], out["p"],
+                                     tobs=None if tobs is None else tobs.detach().contiguous(),
+                                     kmode=bool(kmode))
     return {"timeP": out["timeP"], "p": out["p"], **r}
 
 

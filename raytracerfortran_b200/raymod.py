@@ -175,6 +175,41 @@ def dff_batch_jac(vels, depths, nlayers, src_offset, src_depth, want_times=False
     return {"jvels": jv, "jdepths": jz, "timeP": t, "p": p, "dtdr": dr, "dtdd": dd}
 
 
+def dff_batch_normal(vels, depths, nlayers, src_offset, src_depth, tobs=None, want_times=False,
+                     want_p=False):
+    """dff_batch and the Gauss-Newton normal equations of its travel times in one call (DESIGN.md
+    section 13).
+
+    Returns a dict with "JtJ" [B, P, P] = J^T J, P = ldv + ldz, over the rows dff_batch_jac
+    returns ([jvels | jdepths]), "Jtr" [B, P] = J^T (tobs - timeP) when tobs [NSrc] is given, and,
+    on request, "timeP" / "p" [B, NSrc] of the forward (None otherwise)."""
+    v = _d(vels)
+    z = _d(depths)
+    if v.ndim != 2 or z.ndim != 2 or v.shape[0] != z.shape[0]:
+        raise ValueError("vels and depths must be [B, ldv] and [B, ldz]")
+    nl = np.ascontiguousarray(nlayers, dtype=np.int32)
+    so, sd = _d(src_offset), _d(src_depth)
+    B, ldv, ldz, nsrc = v.shape[0], v.shape[1], z.shape[1], so.size
+    if nl.shape != (B,) or so.ndim != 1 or sd.shape != so.shape:
+        raise ValueError("nlayers must be [B], src_offset and src_depth [NSrc]")
+    to = None if tobs is None else _d(tobs)
+    if to is not None and to.shape != so.shape:
+        raise ValueError("tobs must be [NSrc]")
+    if not 1 <= ldv <= 255:
+        raise ValueError("ldv must be 1..255 (at most 254 interfaces)")
+    if B and (nl.min() < 0 or int(nl.max()) + 1 > ldv or int(nl.max()) > ldz):
+        raise ValueError("nlayers exceeds the row length of vels / depths")
+    P = ldv + ldz
+    jtj = np.empty((B, P, P))
+    jtr = np.empty((B, P)) if to is not None else None
+    t = np.empty((B, nsrc)) if want_times else None
+    p = np.empty((B, nsrc)) if want_p else None
+    rc = _lib.load().dff_batch_normal(_p(v), _p(z), nl.ctypes.data_as(_IP), _ci(B), _ci(ldv), _ci(ldz),
+                                      _p(so), _p(sd), _ci(nsrc), _p(to), _p(t), _p(p), _p(jtj), _p(jtr))
+    _lib.check(rc)
+    return {"JtJ": jtj, "Jtr": jtr, "timeP": t, "p": p}
+
+
 def loglhood_batch(k, voro_vp, ziface, src_offset, src_depth, DobsRT, sdparRT, want_pred=False):
     """LOGLHOOD / LOGLHOOD_RT (loglhood.f90:3-32,35-211) over B chain states.
 
