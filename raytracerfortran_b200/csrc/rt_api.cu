@@ -73,8 +73,11 @@ struct Ctx {
     cudaEvent_t  ev_h2d[kMaxChunks], ev_d2h[kMaxChunks], ev_k0[kMaxChunks], ev_k1[kMaxChunks];
     cudaEvent_t  ev_t0 = nullptr, ev_t1 = nullptr;
     DevBuf vels, depths, nl, off, dep, tobs, sigma, timeP, pout, logL, arena, voro, vsorted,
-        idxar, arparb, sched, mh_ll, mh_out, mh_kp, mh_lpr, gw, ggv, ggz, gdr, gdd;
-    // The scratch buffers below (vels ... gdd) are shared by every entry.  Entries that return
+        idxar, arparb, sched, mh_ll, mh_out, mh_kp, mh_lpr,
+        // the derivative entries': the gradient's weights; the derivatives with respect to the
+        // model (the gradient's sums, the Jacobian's rows) and to the sources; the normal equations
+        w, dvels, ddepths, dtdr, dtdd, JtJ, Jtr;
+    // The scratch buffers above (vels ... Jtr) are shared by every entry.  Entries that return
     // without synchronising (a caller stream was given) leave an event behind; any later entry that
     // uses the scratch from another stream first makes that stream wait for it.
     cudaEvent_t  ev_scratch = nullptr;
@@ -1023,33 +1026,148 @@ int rtb200_dff_batch_device(const double *d_vels, const double *d_depths, const 
     return 0;
 }
 
+extern "C++" {   // device_launch is a template
 namespace {
+
+// The row-length rule of dff_batch, which every derivative entry checks first.
+int check_ldv(int ldv) {
+    if (ldv < 1) return fail("ldv must be >= 1");
+    if (ldv > 255) return fail("more than 254 interfaces per model are not supported");
+    return 0;
+}
+
+// A device entry's inputs from the forward; `who_needs` names the derivative in the message
+// ("the gradient needs").
+int check_forward(const char *who_needs, int nsrc, const void *timeP, const void *p) {
+    if (nsrc > 0 && (!timeP || !p)) return fail(std::string(who_needs) + " the forward's timeP and p");
+    return 0;
+}
+
+// The inputs every derivative kernel reads, from the arguments of the entries (whose order puts
+// kmode last).
+rtb::DerivArgs deriv_args(const double *vels, const double *depths, const int *nlayers, int B, int ldv,
+                          int ldz, const double *off, const double *dep, int nsrc, const double *timeP,
+                          const double *p, int kmode) {
+    return {vels, depths, nlayers, B, ldv, ldz, kmode, off, dep, nsrc, timeP, p};
+}
+
+// The host derivative entries' copy-in and forward on g.s_comp, after each has reserved its own
+// buffers: models and sources into the scratch (padded to whole tiles as in run_host), `in`
+// (in_bytes: the entry's one further input, or null) to `in_dev`, ev_k0, then the batch kernel
+// for timeP and p.  With no source there is nothing to copy of them and no forward.  `d` is set to
+// the inputs of the derivative kernel over the scratch.
+int host_forward(const double *vels, const double *depths, const int *nlayers, int nb, int lv, int lz,
+                 const double *off, const double *dep, int ns, void *in_dev, const double *in,
+                 size_t in_bytes, rtb::DerivArgs &d) {
+    const size_t Bz = (size_t)nb, S = (size_t)ns;
+    TileCfg cfg{};
+    if (ns > 0)
+        if (int rc = choose_cfg(nb, lv, lz, ns, true, cfg)) return rc;
+    const size_t M = ns > 0 ? (size_t)cfg.M : 1, Bpad = (Bz + M - 1) / M * M + M;
+    CK(g.vels.reserve(Bpad * lv * 8));
+    CK(g.depths.reserve(Bpad * std::max(lz, 1) * 8));
+    CK(g.nl.reserve(Bpad * 4));
+    CK(g.off.reserve(std::max<size_t>(S, 1) * 8));
+    CK(g.dep.reserve(std::max<size_t>(S, 1) * 8));
+    CK(g.timeP.reserve(std::max<size_t>(Bz * S, 1) * 8));
+    CK(g.pout.reserve(std::max<size_t>(Bz * S, 1) * 8));
+    cudaStream_t st = g.s_comp;
+    if (int rc = scratch_acquire(st)) return rc;
+    CK(cudaMemcpyAsync(g.vels.p, vels, Bz * lv * 8, cudaMemcpyHostToDevice, st));
+    if (lz > 0) CK(cudaMemcpyAsync(g.depths.p, depths, Bz * lz * 8, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(g.nl.p, nlayers, Bz * 4, cudaMemcpyHostToDevice, st));
+    if (ns > 0) {
+        CK(cudaMemcpyAsync(g.off.p, off, S * 8, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(g.dep.p, dep, S * 8, cudaMemcpyHostToDevice, st));
+        if (in) CK(cudaMemcpyAsync(in_dev, in, in_bytes, cudaMemcpyHostToDevice, st));
+    }
+    CK(cudaEventRecord(g.ev_k0[0], st));
+    d = deriv_args(g.vels.as<double>(), g.depths.as<double>(), g.nl.as<int>(), nb, lv, lz, g.off.as<double>(),
+                   g.dep.as<double>(), ns, g.timeP.as<double>(), g.pout.as<double>(), 0);
+    if (ns > 0) {
+        BatchArgs a{};
+        a.vels = g.vels.as<double>(); a.depths = g.depths.as<double>(); a.nlayers = g.nl.as<int>();
+        a.B = nb; a.ldv = lv; a.ldz = lz; a.kmode = 0;
+        a.src_offset = g.off.as<double>(); a.src_depth = g.dep.as<double>(); a.nsrc = ns;
+        a.timeP = g.timeP.as<double>(); a.p_out = g.pout.as<double>();
+        a.padded = 1;
+        a.sched = next_sched();
+        CK(rtb::launch_batch(a, cfg, st));
+        g.launches++;
+        g.last = cfg;
+    }
+    return 0;
+}
+
+// The host derivative entries' tail, after each has recorded ev_k1 and queued its own outputs: the
+// forward's timeP and p out where asked for, the wait, and the kernel time.
+int host_finish(const rtb::DerivArgs &d, double *timeP, double *p_out) {
+    cudaStream_t st = g.s_comp;
+    const size_t bytes = (size_t)d.B * (size_t)d.nsrc * 8;
+    if (d.nsrc > 0) {
+        if (timeP) CK(cudaMemcpyAsync(timeP, g.timeP.p, bytes, cudaMemcpyDeviceToHost, st));
+        if (p_out) CK(cudaMemcpyAsync(p_out, g.pout.p, bytes, cudaMemcpyDeviceToHost, st));
+    }
+    CK(cudaStreamSynchronize(st));
+    if (int rc = scratch_release(st, true)) return rc;
+    float ms = 0.f;
+    if (cudaEventElapsedTime(&ms, g.ev_k0[0], g.ev_k1[0]) == cudaSuccess) g.kernel_ms = g.total_ms = ms;
+    return 0;
+}
+
+// A device entry's work, enqueue(st), between the kernel-time events on the caller's stream (or
+// the library's); without a caller stream it is waited for and timed.
+template <class Enqueue>
+int device_launch(void *stream, Enqueue enqueue) {
+    cudaStream_t st = stream ? (cudaStream_t)stream : g.s_comp;
+    CK(cudaEventRecord(g.ev_k0[0], st));
+    if (int rc = enqueue(st)) return rc;
+    CK(cudaEventRecord(g.ev_k1[0], st));
+    if (!stream) {
+        CK(cudaStreamSynchronize(st));
+        float ms = 0.f;
+        CK(cudaEventElapsedTime(&ms, g.ev_k0[0], g.ev_k1[0]));
+        g.kernel_ms = g.total_ms = ms;
+    }
+    return 0;
+}
 
 // The argument checks both gradient entries share (the shape rules of dff_batch).
 int check_grad_args(int ldv, int ldz, const void *vels, const void *nlayers, const void *off,
                     const void *dep, int nsrc, const void *w, const void *gvels, const void *gdepths) {
-    if (ldv < 1) return fail("ldv must be >= 1");
-    if (ldv > 255) return fail("more than 254 interfaces per model are not supported");
+    if (int rc = check_ldv(ldv)) return rc;
     if (!vels || !nlayers || !gvels || (ldz > 0 && !gdepths))
         return fail("the gradient needs vels, nlayers, gvels and (ldz > 0) gdepths");
     if (nsrc > 0 && (!off || !dep || !w)) return fail("the gradient needs src_offset, src_depth and w");
     return 0;
 }
 
-rtb::GradArgs grad_args(const double *vels, const double *depths, const int *nlayers, int B, int ldv,
-                        int ldz, const double *off, const double *dep, int nsrc, const double *timeP,
-                        const double *p, const double *w, double *gvels, double *gdepths,
-                        double *dtdr, double *dtdd, int kmode) {
-    rtb::GradArgs a{};
-    a.vels = vels; a.depths = depths; a.nlayers = nlayers;
-    a.B = B; a.ldv = ldv; a.ldz = ldz; a.kmode = kmode;
-    a.src_offset = off; a.src_depth = dep; a.nsrc = nsrc;
-    a.timeP = timeP; a.p = p; a.w = w;
-    a.gvels = gvels; a.gdepths = gdepths; a.dtdr = dtdr; a.dtdd = dtdd;
-    return a;
+// The argument checks both Jacobian entries share; timeP and p are checked by the device entry,
+// whose inputs they are.
+int check_jac_args(int ldv, int ldz, const void *vels, const void *nlayers, const void *off,
+                   const void *dep, const void *jvels, const void *jdepths) {
+    if (int rc = check_ldv(ldv)) return rc;
+    if (!vels || !nlayers || !jvels) return fail("the Jacobian needs vels, nlayers and jvels");
+    if (ldz > 0 && !jdepths) return fail("the Jacobian needs jdepths when ldz > 0");
+    if (!off || !dep) return fail("the Jacobian needs src_offset and src_depth");
+    return 0;
+}
+
+// The argument checks both normal-equations entries share; timeP and p are checked by the device
+// entry, whose inputs they are.
+int check_normal_args(int ldv, int ldz, int nsrc, const void *vels, const void *nlayers,
+                      const void *off, const void *dep, const void *JtJ, const void *tobs,
+                      const void *Jtr) {
+    if (int rc = check_ldv(ldv)) return rc;
+    if (!vels || !nlayers || !JtJ) return fail("the normal equations need vels, nlayers and JtJ");
+    // empty source arrays may arrive as NULL: with no source there is nothing to read
+    if ((tobs && !Jtr) || (!tobs && Jtr && nsrc > 0)) return fail("tobs and Jtr must be given together");
+    if (nsrc > 0 && (!off || !dep)) return fail("the normal equations need src_offset and src_depth");
+    return 0;
 }
 
 }  // namespace
+}  // extern "C++"
 
 int rtb200_dff_grad_device(const double *d_vels, const double *d_depths, const int *d_nlayers,
                            int B, int ldv, int ldz, const double *d_src_offset,
@@ -1066,22 +1184,15 @@ int rtb200_dff_grad_device(const double *d_vels, const double *d_depths, const i
     if (int rc = check_grad_args(ldv, ldz, d_vels, d_nlayers, d_src_offset, d_src_depth, NSrc, d_w,
                                  d_gvels, d_gdepths))
         return rc;
-    if (NSrc > 0 && (!d_timeP || !d_p)) return fail("the gradient needs the forward's timeP and p");
-    cudaStream_t st = stream ? (cudaStream_t)stream : g.s_comp;
-    const rtb::GradArgs a = grad_args(d_vels, d_depths, d_nlayers, B, ldv, ldz, d_src_offset,
-                                      d_src_depth, NSrc, d_timeP, d_p, d_w, d_gvels, d_gdepths,
-                                      d_dtdr, d_dtdd, kmode);
-    CK(cudaEventRecord(g.ev_k0[0], st));
-    CK(rtb::launch_grad(a, st));
-    CK(cudaEventRecord(g.ev_k1[0], st));
-    g.launches++;
-    if (!stream) {
-        CK(cudaStreamSynchronize(st));
-        float ms = 0.f;
-        CK(cudaEventElapsedTime(&ms, g.ev_k0[0], g.ev_k1[0]));
-        g.kernel_ms = g.total_ms = ms;
-    }
-    return 0;
+    if (int rc = check_forward("the gradient needs", NSrc, d_timeP, d_p)) return rc;
+    const rtb::GradArgs a{deriv_args(d_vels, d_depths, d_nlayers, B, ldv, ldz, d_src_offset, d_src_depth,
+                                     NSrc, d_timeP, d_p, kmode),
+                          d_w, d_gvels, d_gdepths, d_dtdr, d_dtdd};
+    return device_launch(stream, [&](cudaStream_t st) {
+        CK(rtb::launch_grad(a, st));
+        g.launches++;
+        return 0;
+    });
 }
 
 int dff_batch_grad(const double *vels, const double *depths, const int *nlayers, const int *B,
@@ -1096,98 +1207,31 @@ int dff_batch_grad(const double *vels, const double *depths, const int *nlayers,
     if (nb <= 0) return 0;
     if (int rc = check_grad_args(lv, lz, vels, nlayers, src_offset, src_depth, ns, w, gvels, gdepths))
         return rc;
+    // copy in, forward, gradient, copy out; with no source the gradient kernel alone writes zeros
     const size_t Bz = (size_t)nb, S = (size_t)ns;
-    TileCfg cfg{};
-    if (ns > 0)
-        if (int rc = choose_cfg(nb, lv, lz, ns, true, cfg)) return rc;
-    // copy in, forward, gradient, copy out; our buffers are padded to whole tiles as in run_host
-    const size_t M = ns > 0 ? (size_t)cfg.M : 1, Bpad = (Bz + M - 1) / M * M + M;
-    CK(g.vels.reserve(Bpad * lv * 8));
-    CK(g.depths.reserve(Bpad * std::max(lz, 1) * 8));
-    CK(g.nl.reserve(Bpad * 4));
-    CK(g.off.reserve(std::max<size_t>(S, 1) * 8));
-    CK(g.dep.reserve(std::max<size_t>(S, 1) * 8));
-    CK(g.timeP.reserve(std::max<size_t>(Bz * S, 1) * 8));
-    CK(g.pout.reserve(std::max<size_t>(Bz * S, 1) * 8));
-    CK(g.gw.reserve(std::max<size_t>(Bz * S, 1) * 8));
-    CK(g.ggv.reserve(Bz * lv * 8));
-    CK(g.ggz.reserve(std::max<size_t>(Bz * lz, 1) * 8));
-    if (dtdr) CK(g.gdr.reserve(std::max<size_t>(Bz * S, 1) * 8));
-    if (dtdd) CK(g.gdd.reserve(std::max<size_t>(Bz * S, 1) * 8));
+    CK(g.w.reserve(std::max<size_t>(Bz * S, 1) * 8));
+    CK(g.dvels.reserve(Bz * lv * 8));
+    CK(g.ddepths.reserve(std::max<size_t>(Bz * lz, 1) * 8));
+    if (dtdr) CK(g.dtdr.reserve(std::max<size_t>(Bz * S, 1) * 8));
+    if (dtdd) CK(g.dtdd.reserve(std::max<size_t>(Bz * S, 1) * 8));
+    rtb::DerivArgs d;
+    if (int rc = host_forward(vels, depths, nlayers, nb, lv, lz, src_offset, src_depth, ns, g.w.p, w,
+                              Bz * S * 8, d))
+        return rc;
     cudaStream_t st = g.s_comp;
-    if (int rc = scratch_acquire(st)) return rc;
-    CK(cudaMemcpyAsync(g.vels.p, vels, Bz * lv * 8, cudaMemcpyHostToDevice, st));
-    if (lz > 0) CK(cudaMemcpyAsync(g.depths.p, depths, Bz * lz * 8, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(g.nl.p, nlayers, Bz * 4, cudaMemcpyHostToDevice, st));
-    if (ns > 0) {
-        CK(cudaMemcpyAsync(g.off.p, src_offset, S * 8, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(g.dep.p, src_depth, S * 8, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(g.gw.p, w, Bz * S * 8, cudaMemcpyHostToDevice, st));
-    }
-    CK(cudaEventRecord(g.ev_k0[0], st));
-    if (ns > 0) {
-        BatchArgs a{};
-        a.vels = g.vels.as<double>(); a.depths = g.depths.as<double>(); a.nlayers = g.nl.as<int>();
-        a.B = nb; a.ldv = lv; a.ldz = lz; a.kmode = 0;
-        a.src_offset = g.off.as<double>(); a.src_depth = g.dep.as<double>(); a.nsrc = ns;
-        a.timeP = g.timeP.as<double>(); a.p_out = g.pout.as<double>();
-        a.padded = 1;
-        a.sched = next_sched();
-        CK(rtb::launch_batch(a, cfg, st));
-        g.launches++;
-        g.last = cfg;
-    }
-    const rtb::GradArgs ga = grad_args(g.vels.as<double>(), g.depths.as<double>(), g.nl.as<int>(), nb, lv,
-                                       lz, g.off.as<double>(), g.dep.as<double>(), ns, g.timeP.as<double>(),
-                                       g.pout.as<double>(), g.gw.as<double>(), g.ggv.as<double>(),
-                                       g.ggz.as<double>(), dtdr ? g.gdr.as<double>() : nullptr,
-                                       dtdd ? g.gdd.as<double>() : nullptr, 0);
+    const rtb::GradArgs ga{d, g.w.as<double>(), g.dvels.as<double>(), g.ddepths.as<double>(),
+                           dtdr ? g.dtdr.as<double>() : nullptr, dtdd ? g.dtdd.as<double>() : nullptr};
     CK(rtb::launch_grad(ga, st));
     CK(cudaEventRecord(g.ev_k1[0], st));
     g.launches++;
-    CK(cudaMemcpyAsync(gvels, g.ggv.p, Bz * lv * 8, cudaMemcpyDeviceToHost, st));
-    if (lz > 0) CK(cudaMemcpyAsync(gdepths, g.ggz.p, Bz * lz * 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(gvels, g.dvels.p, Bz * lv * 8, cudaMemcpyDeviceToHost, st));
+    if (lz > 0) CK(cudaMemcpyAsync(gdepths, g.ddepths.p, Bz * lz * 8, cudaMemcpyDeviceToHost, st));
     if (ns > 0) {
-        if (timeP) CK(cudaMemcpyAsync(timeP, g.timeP.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
-        if (p_out) CK(cudaMemcpyAsync(p_out, g.pout.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
-        if (dtdr) CK(cudaMemcpyAsync(dtdr, g.gdr.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
-        if (dtdd) CK(cudaMemcpyAsync(dtdd, g.gdd.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
+        if (dtdr) CK(cudaMemcpyAsync(dtdr, g.dtdr.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
+        if (dtdd) CK(cudaMemcpyAsync(dtdd, g.dtdd.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
     }
-    CK(cudaStreamSynchronize(st));
-    if (int rc = scratch_release(st, true)) return rc;
-    float ms = 0.f;
-    if (cudaEventElapsedTime(&ms, g.ev_k0[0], g.ev_k1[0]) == cudaSuccess) g.kernel_ms = g.total_ms = ms;
-    return 0;
+    return host_finish(d, timeP, p_out);
 }
-
-namespace {
-
-// The argument checks both Jacobian entries share; timeP and p are checked by the device entry,
-// whose inputs they are.
-int check_jac_args(int ldv, int ldz, const void *vels, const void *nlayers, const void *off,
-                   const void *dep, const void *jvels, const void *jdepths) {
-    if (ldv < 1) return fail("ldv must be >= 1");
-    if (ldv > 255) return fail("more than 254 interfaces per model are not supported");
-    if (!vels || !nlayers || !jvels) return fail("the Jacobian needs vels, nlayers and jvels");
-    if (ldz > 0 && !jdepths) return fail("the Jacobian needs jdepths when ldz > 0");
-    if (!off || !dep) return fail("the Jacobian needs src_offset and src_depth");
-    return 0;
-}
-
-rtb::JacArgs jac_args(const double *vels, const double *depths, const int *nlayers, int B, int ldv,
-                      int ldz, const double *off, const double *dep, int nsrc, const double *timeP,
-                      const double *p, double *jvels, double *jdepths, double *dtdr, double *dtdd,
-                      int kmode) {
-    rtb::JacArgs a{};
-    a.vels = vels; a.depths = depths; a.nlayers = nlayers;
-    a.B = B; a.ldv = ldv; a.ldz = ldz; a.kmode = kmode;
-    a.src_offset = off; a.src_depth = dep; a.nsrc = nsrc;
-    a.timeP = timeP; a.p = p;
-    a.jvels = jvels; a.jdepths = jdepths; a.dtdr = dtdr; a.dtdd = dtdd;
-    return a;
-}
-
-}  // namespace
 
 int rtb200_dff_jac_device(const double *d_vels, const double *d_depths, const int *d_nlayers,
                           int B, int ldv, int ldz, const double *d_src_offset,
@@ -1202,22 +1246,15 @@ int rtb200_dff_jac_device(const double *d_vels, const double *d_depths, const in
     if (int rc = check_jac_args(ldv, ldz, d_vels, d_nlayers, d_src_offset, d_src_depth, d_jvels,
                                 d_jdepths))
         return rc;
-    if (!d_timeP || !d_p) return fail("the Jacobian needs the forward's timeP and p");
-    cudaStream_t st = stream ? (cudaStream_t)stream : g.s_comp;
-    const rtb::JacArgs a = jac_args(d_vels, d_depths, d_nlayers, B, ldv, ldz, d_src_offset,
-                                    d_src_depth, NSrc, d_timeP, d_p, d_jvels, d_jdepths, d_dtdr,
-                                    d_dtdd, kmode);
-    CK(cudaEventRecord(g.ev_k0[0], st));
-    CK(rtb::launch_jac(a, st));
-    CK(cudaEventRecord(g.ev_k1[0], st));
-    g.launches++;
-    if (!stream) {
-        CK(cudaStreamSynchronize(st));
-        float ms = 0.f;
-        CK(cudaEventElapsedTime(&ms, g.ev_k0[0], g.ev_k1[0]));
-        g.kernel_ms = g.total_ms = ms;
-    }
-    return 0;
+    if (int rc = check_forward("the Jacobian needs", NSrc, d_timeP, d_p)) return rc;
+    const rtb::JacArgs a{deriv_args(d_vels, d_depths, d_nlayers, B, ldv, ldz, d_src_offset, d_src_depth,
+                                    NSrc, d_timeP, d_p, kmode),
+                         d_jvels, d_jdepths, d_dtdr, d_dtdd};
+    return device_launch(stream, [&](cudaStream_t st) {
+        CK(rtb::launch_jac(a, st));
+        g.launches++;
+        return 0;
+    });
 }
 
 int dff_batch_jac(const double *vels, const double *depths, const int *nlayers, const int *B,
@@ -1232,92 +1269,28 @@ int dff_batch_jac(const double *vels, const double *depths, const int *nlayers, 
     if (nb <= 0 || ns <= 0) return 0;
     if (int rc = check_jac_args(lv, lz, vels, nlayers, src_offset, src_depth, jvels, jdepths))
         return rc;
+    // copy in, forward, Jacobian, copy out
     const size_t Bz = (size_t)nb, S = (size_t)ns;
-    TileCfg cfg{};
-    if (int rc = choose_cfg(nb, lv, lz, ns, true, cfg)) return rc;
-    // copy in, forward, Jacobian, copy out; our buffers are padded to whole tiles as in run_host
-    const size_t M = (size_t)cfg.M, Bpad = (Bz + M - 1) / M * M + M;
-    CK(g.vels.reserve(Bpad * lv * 8));
-    CK(g.depths.reserve(Bpad * std::max(lz, 1) * 8));
-    CK(g.nl.reserve(Bpad * 4));
-    CK(g.off.reserve(S * 8));
-    CK(g.dep.reserve(S * 8));
-    CK(g.timeP.reserve(Bz * S * 8));
-    CK(g.pout.reserve(Bz * S * 8));
-    CK(g.ggv.reserve(Bz * S * lv * 8));
-    if (lz > 0) CK(g.ggz.reserve(Bz * S * lz * 8));
-    if (dtdr) CK(g.gdr.reserve(Bz * S * 8));
-    if (dtdd) CK(g.gdd.reserve(Bz * S * 8));
+    CK(g.dvels.reserve(Bz * S * lv * 8));
+    if (lz > 0) CK(g.ddepths.reserve(Bz * S * lz * 8));
+    if (dtdr) CK(g.dtdr.reserve(Bz * S * 8));
+    if (dtdd) CK(g.dtdd.reserve(Bz * S * 8));
+    rtb::DerivArgs d;
+    if (int rc = host_forward(vels, depths, nlayers, nb, lv, lz, src_offset, src_depth, ns, nullptr, nullptr,
+                              0, d))
+        return rc;
     cudaStream_t st = g.s_comp;
-    if (int rc = scratch_acquire(st)) return rc;
-    CK(cudaMemcpyAsync(g.vels.p, vels, Bz * lv * 8, cudaMemcpyHostToDevice, st));
-    if (lz > 0) CK(cudaMemcpyAsync(g.depths.p, depths, Bz * lz * 8, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(g.nl.p, nlayers, Bz * 4, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(g.off.p, src_offset, S * 8, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(g.dep.p, src_depth, S * 8, cudaMemcpyHostToDevice, st));
-    CK(cudaEventRecord(g.ev_k0[0], st));
-    BatchArgs a{};
-    a.vels = g.vels.as<double>(); a.depths = g.depths.as<double>(); a.nlayers = g.nl.as<int>();
-    a.B = nb; a.ldv = lv; a.ldz = lz; a.kmode = 0;
-    a.src_offset = g.off.as<double>(); a.src_depth = g.dep.as<double>(); a.nsrc = ns;
-    a.timeP = g.timeP.as<double>(); a.p_out = g.pout.as<double>();
-    a.padded = 1;
-    a.sched = next_sched();
-    CK(rtb::launch_batch(a, cfg, st));
-    g.launches++;
-    g.last = cfg;
-    const rtb::JacArgs ja = jac_args(g.vels.as<double>(), g.depths.as<double>(), g.nl.as<int>(), nb, lv,
-                                     lz, g.off.as<double>(), g.dep.as<double>(), ns, g.timeP.as<double>(),
-                                     g.pout.as<double>(), g.ggv.as<double>(),
-                                     lz > 0 ? g.ggz.as<double>() : nullptr,
-                                     dtdr ? g.gdr.as<double>() : nullptr,
-                                     dtdd ? g.gdd.as<double>() : nullptr, 0);
+    const rtb::JacArgs ja{d, g.dvels.as<double>(), lz > 0 ? g.ddepths.as<double>() : nullptr,
+                          dtdr ? g.dtdr.as<double>() : nullptr, dtdd ? g.dtdd.as<double>() : nullptr};
     CK(rtb::launch_jac(ja, st));
     CK(cudaEventRecord(g.ev_k1[0], st));
     g.launches++;
-    CK(cudaMemcpyAsync(jvels, g.ggv.p, Bz * S * lv * 8, cudaMemcpyDeviceToHost, st));
-    if (lz > 0) CK(cudaMemcpyAsync(jdepths, g.ggz.p, Bz * S * lz * 8, cudaMemcpyDeviceToHost, st));
-    if (timeP) CK(cudaMemcpyAsync(timeP, g.timeP.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
-    if (p_out) CK(cudaMemcpyAsync(p_out, g.pout.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
-    if (dtdr) CK(cudaMemcpyAsync(dtdr, g.gdr.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
-    if (dtdd) CK(cudaMemcpyAsync(dtdd, g.gdd.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    if (int rc = scratch_release(st, true)) return rc;
-    float ms = 0.f;
-    if (cudaEventElapsedTime(&ms, g.ev_k0[0], g.ev_k1[0]) == cudaSuccess) g.kernel_ms = g.total_ms = ms;
-    return 0;
+    CK(cudaMemcpyAsync(jvels, g.dvels.p, Bz * S * lv * 8, cudaMemcpyDeviceToHost, st));
+    if (lz > 0) CK(cudaMemcpyAsync(jdepths, g.ddepths.p, Bz * S * lz * 8, cudaMemcpyDeviceToHost, st));
+    if (dtdr) CK(cudaMemcpyAsync(dtdr, g.dtdr.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
+    if (dtdd) CK(cudaMemcpyAsync(dtdd, g.dtdd.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
+    return host_finish(d, timeP, p_out);
 }
-
-namespace {
-
-// The argument checks both normal-equations entries share; timeP and p are checked by the device
-// entry, whose inputs they are.
-int check_normal_args(int ldv, int ldz, int nsrc, const void *vels, const void *nlayers,
-                      const void *off, const void *dep, const void *JtJ, const void *tobs,
-                      const void *Jtr) {
-    if (ldv < 1) return fail("ldv must be >= 1");
-    if (ldv > 255) return fail("more than 254 interfaces per model are not supported");
-    if (!vels || !nlayers || !JtJ) return fail("the normal equations need vels, nlayers and JtJ");
-    // empty source arrays may arrive as NULL: with no source there is nothing to read
-    if ((tobs && !Jtr) || (!tobs && Jtr && nsrc > 0)) return fail("tobs and Jtr must be given together");
-    if (nsrc > 0 && (!off || !dep)) return fail("the normal equations need src_offset and src_depth");
-    return 0;
-}
-
-rtb::NormalArgs normal_args(const double *vels, const double *depths, const int *nlayers, int B,
-                            int ldv, int ldz, const double *off, const double *dep, int nsrc,
-                            const double *timeP, const double *p, const double *tobs, double *JtJ,
-                            double *Jtr, int kmode) {
-    rtb::NormalArgs a{};
-    a.vels = vels; a.depths = depths; a.nlayers = nlayers;
-    a.B = B; a.ldv = ldv; a.ldz = ldz; a.kmode = kmode;
-    a.src_offset = off; a.src_depth = dep; a.nsrc = nsrc;
-    a.timeP = timeP; a.p = p; a.tobs = tobs;
-    a.JtJ = JtJ; a.Jtr = Jtr;
-    return a;
-}
-
-}  // namespace
 
 int rtb200_dff_normal_device(const double *d_vels, const double *d_depths, const int *d_nlayers,
                              int B, int ldv, int ldz, const double *d_src_offset,
@@ -1332,28 +1305,21 @@ int rtb200_dff_normal_device(const double *d_vels, const double *d_depths, const
     if (int rc = check_normal_args(ldv, ldz, NSrc, d_vels, d_nlayers, d_src_offset, d_src_depth,
                                    d_JtJ, d_tobs, d_Jtr))
         return rc;
-    if (NSrc > 0 && (!d_timeP || !d_p)) return fail("the normal equations need the forward's timeP and p");
-    cudaStream_t st = stream ? (cudaStream_t)stream : g.s_comp;
+    if (int rc = check_forward("the normal equations need", NSrc, d_timeP, d_p)) return rc;
     const size_t P = (size_t)(ldv + ldz);
-    CK(cudaEventRecord(g.ev_k0[0], st));
-    if (NSrc <= 0) {            // sums over no source
-        CK(cudaMemsetAsync(d_JtJ, 0, (size_t)B * P * P * 8, st));
-        if (d_Jtr) CK(cudaMemsetAsync(d_Jtr, 0, (size_t)B * P * 8, st));
-    } else {
-        const rtb::NormalArgs a = normal_args(d_vels, d_depths, d_nlayers, B, ldv, ldz, d_src_offset,
-                                              d_src_depth, NSrc, d_timeP, d_p, d_tobs, d_JtJ, d_Jtr,
-                                              kmode);
-        CK(rtb::launch_normal(a, st));
-        g.launches++;
-    }
-    CK(cudaEventRecord(g.ev_k1[0], st));
-    if (!stream) {
-        CK(cudaStreamSynchronize(st));
-        float ms = 0.f;
-        CK(cudaEventElapsedTime(&ms, g.ev_k0[0], g.ev_k1[0]));
-        g.kernel_ms = g.total_ms = ms;
-    }
-    return 0;
+    const rtb::NormalArgs a{deriv_args(d_vels, d_depths, d_nlayers, B, ldv, ldz, d_src_offset, d_src_depth,
+                                       NSrc, d_timeP, d_p, kmode),
+                            d_tobs, d_JtJ, d_Jtr};
+    return device_launch(stream, [&](cudaStream_t st) {
+        if (NSrc <= 0) {        // sums over no source
+            CK(cudaMemsetAsync(d_JtJ, 0, (size_t)B * P * P * 8, st));
+            if (d_Jtr) CK(cudaMemsetAsync(d_Jtr, 0, (size_t)B * P * 8, st));
+        } else {
+            CK(rtb::launch_normal(a, st));
+            g.launches++;
+        }
+        return 0;
+    });
 }
 
 int dff_batch_normal(const double *vels, const double *depths, const int *nlayers, const int *B,
@@ -1374,59 +1340,26 @@ int dff_batch_normal(const double *vels, const double *depths, const int *nlayer
         if (Jtr) std::memset(Jtr, 0, Bz * P * 8);
         return 0;
     }
+    // copy in, forward, normal equations, copy out
     const size_t S = (size_t)ns;
-    TileCfg cfg{};
-    if (int rc = choose_cfg(nb, lv, lz, ns, true, cfg)) return rc;
-    // copy in, forward, normal equations, copy out; our buffers are padded to whole tiles as in run_host
-    const size_t M = (size_t)cfg.M, Bpad = (Bz + M - 1) / M * M + M;
-    CK(g.vels.reserve(Bpad * lv * 8));
-    CK(g.depths.reserve(Bpad * std::max(lz, 1) * 8));
-    CK(g.nl.reserve(Bpad * 4));
-    CK(g.off.reserve(S * 8));
-    CK(g.dep.reserve(S * 8));
-    CK(g.timeP.reserve(Bz * S * 8));
-    CK(g.pout.reserve(Bz * S * 8));
-    CK(g.ggv.reserve(Bz * P * P * 8));
+    CK(g.JtJ.reserve(Bz * P * P * 8));
     if (tobs) {
-        CK(g.gdr.reserve(S * 8));
-        CK(g.ggz.reserve(Bz * P * 8));
+        CK(g.tobs.reserve(S * 8));
+        CK(g.Jtr.reserve(Bz * P * 8));
     }
+    rtb::DerivArgs d;
+    if (int rc = host_forward(vels, depths, nlayers, nb, lv, lz, src_offset, src_depth, ns, g.tobs.p, tobs,
+                              S * 8, d))
+        return rc;
     cudaStream_t st = g.s_comp;
-    if (int rc = scratch_acquire(st)) return rc;
-    CK(cudaMemcpyAsync(g.vels.p, vels, Bz * lv * 8, cudaMemcpyHostToDevice, st));
-    if (lz > 0) CK(cudaMemcpyAsync(g.depths.p, depths, Bz * lz * 8, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(g.nl.p, nlayers, Bz * 4, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(g.off.p, src_offset, S * 8, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(g.dep.p, src_depth, S * 8, cudaMemcpyHostToDevice, st));
-    if (tobs) CK(cudaMemcpyAsync(g.gdr.p, tobs, S * 8, cudaMemcpyHostToDevice, st));
-    CK(cudaEventRecord(g.ev_k0[0], st));
-    BatchArgs a{};
-    a.vels = g.vels.as<double>(); a.depths = g.depths.as<double>(); a.nlayers = g.nl.as<int>();
-    a.B = nb; a.ldv = lv; a.ldz = lz; a.kmode = 0;
-    a.src_offset = g.off.as<double>(); a.src_depth = g.dep.as<double>(); a.nsrc = ns;
-    a.timeP = g.timeP.as<double>(); a.p_out = g.pout.as<double>();
-    a.padded = 1;
-    a.sched = next_sched();
-    CK(rtb::launch_batch(a, cfg, st));
-    g.launches++;
-    g.last = cfg;
-    const rtb::NormalArgs na = normal_args(g.vels.as<double>(), g.depths.as<double>(), g.nl.as<int>(), nb,
-                                           lv, lz, g.off.as<double>(), g.dep.as<double>(), ns,
-                                           g.timeP.as<double>(), g.pout.as<double>(),
-                                           tobs ? g.gdr.as<double>() : nullptr, g.ggv.as<double>(),
-                                           tobs ? g.ggz.as<double>() : nullptr, 0);
+    const rtb::NormalArgs na{d, tobs ? g.tobs.as<double>() : nullptr, g.JtJ.as<double>(),
+                             tobs ? g.Jtr.as<double>() : nullptr};
     CK(rtb::launch_normal(na, st));
     CK(cudaEventRecord(g.ev_k1[0], st));
     g.launches++;
-    CK(cudaMemcpyAsync(JtJ, g.ggv.p, Bz * P * P * 8, cudaMemcpyDeviceToHost, st));
-    if (tobs) CK(cudaMemcpyAsync(Jtr, g.ggz.p, Bz * P * 8, cudaMemcpyDeviceToHost, st));
-    if (timeP) CK(cudaMemcpyAsync(timeP, g.timeP.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
-    if (p_out) CK(cudaMemcpyAsync(p_out, g.pout.p, Bz * S * 8, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    if (int rc = scratch_release(st, true)) return rc;
-    float ms = 0.f;
-    if (cudaEventElapsedTime(&ms, g.ev_k0[0], g.ev_k1[0]) == cudaSuccess) g.kernel_ms = g.total_ms = ms;
-    return 0;
+    CK(cudaMemcpyAsync(JtJ, g.JtJ.p, Bz * P * P * 8, cudaMemcpyDeviceToHost, st));
+    if (tobs) CK(cudaMemcpyAsync(Jtr, g.Jtr.p, Bz * P * 8, cudaMemcpyDeviceToHost, st));
+    return host_finish(d, timeP, p_out);
 }
 
 extern "C++" {   // the helpers below include templates
@@ -1970,8 +1903,8 @@ void rtb200_shutdown(void) {
     for (auto &e : g.ev_slot) { if (e) cudaEventDestroy(e); e = nullptr; }
     for (DevBuf *b : {&g.vels, &g.depths, &g.nl, &g.off, &g.dep, &g.tobs, &g.sigma,
                       &g.timeP, &g.pout, &g.logL, &g.arena, &g.voro, &g.vsorted, &g.idxar, &g.arparb,
-                      &g.sched, &g.mh_ll, &g.mh_out, &g.mh_kp, &g.mh_lpr, &g.gw, &g.ggv, &g.ggz,
-                      &g.gdr, &g.gdd})
+                      &g.sched, &g.mh_ll, &g.mh_out, &g.mh_kp, &g.mh_lpr, &g.w, &g.dvels, &g.ddepths,
+                      &g.dtdr, &g.dtdd, &g.JtJ, &g.Jtr})
         b->release();
     for (int i = 0; i < kMaxChunks; ++i) {
         cudaEventDestroy(g.ev_h2d[i]);

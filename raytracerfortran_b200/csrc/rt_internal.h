@@ -42,9 +42,11 @@ struct BatchArgs {
     int          *sched;
 };
 
-// One launch of the gradient kernel (the vector-Jacobian product of the travel times, DESIGN.md
-// section 11).  Every pointer is a device pointer; model and source arrays as in BatchArgs.
-struct GradArgs {
+// What every derivative kernel reads: the models and sources of a batch-kernel launch and what it
+// returned.  Every pointer is a device pointer; model and source arrays as in BatchArgs.  It is
+// the base of GradArgs, JacArgs and NormalArgs, so their fields keep the offsets they would have
+// if each declared these itself.
+struct DerivArgs {
     const double *vels;        // [B][ldv]
     const double *depths;      // [B][ldz]
     const int    *nlayers;     // [B]; kmode: node counts k
@@ -55,6 +57,11 @@ struct GradArgs {
     int           nsrc;
     const double *timeP;       // [B][nsrc] the batch kernel's travel times
     const double *p;           // [B][nsrc] and ray parameters
+};
+
+// One launch of the gradient kernel (the vector-Jacobian product of the travel times, DESIGN.md
+// section 11).
+struct GradArgs : DerivArgs {
     const double *w;           // [B][nsrc] weights of the product
     double       *gvels;       // [B][ldv]  sum_s w dT/dV_i
     double       *gdepths;     // [B][ldz]  sum_s w dT/dz_j
@@ -63,37 +70,17 @@ struct GradArgs {
 };
 
 // One launch of the Jacobian kernel (the per-ray terms the gradient kernel sums, DESIGN.md
-// section 12).  Every pointer is a device pointer; inputs as in GradArgs.
-struct JacArgs {
-    const double *vels;        // [B][ldv]
-    const double *depths;      // [B][ldz]
-    const int    *nlayers;     // [B]; kmode: node counts k
-    int           B, ldv, ldz;
-    int           kmode;
-    const double *src_offset;  // [nsrc]
-    const double *src_depth;   // [nsrc]
-    int           nsrc;
-    const double *timeP;       // [B][nsrc] the batch kernel's travel times
-    const double *p;           // [B][nsrc] and ray parameters
+// section 12).
+struct JacArgs : DerivArgs {
     double       *jvels;       // [B][nsrc][ldv]  dT_bs/dV_i
     double       *jdepths;     // [B][nsrc][ldz]  dT_bs/dz_j (null when ldz = 0)
     double       *dtdr;        // [B][nsrc] or null: dT/d(offset)
     double       *dtdd;        // [B][nsrc] or null: dT/d(depth)
 };
 
-// One launch of the normal-equations kernel (DESIGN.md section 13).  Every pointer is a device
-// pointer; inputs as in JacArgs.  P = ldv + ldz parameter columns, [vels | depths].
-struct NormalArgs {
-    const double *vels;        // [B][ldv]
-    const double *depths;      // [B][ldz]
-    const int    *nlayers;     // [B]; kmode: node counts k
-    int           B, ldv, ldz;
-    int           kmode;
-    const double *src_offset;  // [nsrc]
-    const double *src_depth;   // [nsrc]
-    int           nsrc;
-    const double *timeP;       // [B][nsrc] the batch kernel's travel times
-    const double *p;           // [B][nsrc] and ray parameters
+// One launch of the normal-equations kernel (DESIGN.md section 13).  P = ldv + ldz parameter
+// columns, [vels | depths].
+struct NormalArgs : DerivArgs {
     const double *tobs;        // [nsrc] or null (then Jtr is null)
     double       *JtJ;         // [B][P][P]
     double       *Jtr;         // [B][P] or null

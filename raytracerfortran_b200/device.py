@@ -84,6 +84,25 @@ def _check_grad_shapes(vels, depths, nlayers, src_offset, src_depth, per_ray):
     return B, ldv, ldz, S
 
 
+def _deriv_prologue(fn, vels, depths, nlayers, src_offset, src_depth, timeP, p, per_ray, outputs):
+    """What the derivative wrappers share, every check before the library is loaded: the shapes
+    (per_ray: the [B, NSrc] inputs by name; outputs(B, ldv, ldz, S): the wrapper's own checks, which
+    return its (name, tensor or None, shape) outputs to check), CUDA tensors, the device.  Returns
+    (B, ldv, ldz, S), the device and the 11 leading arguments of the C entry `fn`."""
+    B, ldv, ldz, S = _check_grad_shapes(vels, depths, nlayers, src_offset, src_depth, per_ray)
+    for name, t, shape in outputs(B, ldv, ldz, S):
+        if t is not None and tuple(t.shape) != shape:
+            raise ValueError(f"{name} must be {list(shape)}, got {list(t.shape)}")
+    if not vels.is_cuda:
+        raise ValueError(f"{fn} needs CUDA tensors (there is no CPU path)")
+    dev = vels.device
+    _ensure_device(dev.index if dev.index is not None else torch.cuda.current_device())
+    f64 = torch.float64
+    args = (_ptr(vels, f64), _ptr(depths, f64) if ldz else None, _ptr(nlayers, torch.int32), B, ldv, ldz,
+            _ptr(src_offset, f64), _ptr(src_depth, f64), S, _ptr(timeP, f64), _ptr(p, f64))
+    return (B, ldv, ldz, S), dev, args
+
+
 def dff_grad_device(vels, depths, nlayers, src_offset, src_depth, timeP, p, w, gvels=None,
                     gdepths=None, want_src=False, dtdr=None, dtdd=None, kmode=False, stream=None):
     """Vector-Jacobian product of the travel times dff_batch_device returned (timeP, p [B, NSrc])
@@ -93,15 +112,10 @@ def dff_grad_device(vels, depths, nlayers, src_offset, src_depth, timeP, p, w, g
     gvels[b, i] = sum_s w[b, s] dT[b, s]/dV_i, gdepths likewise for the interfaces (kmode: ziface),
     dtdr / dtdd the per-ray derivatives with respect to the source offset and depth (want_src).
     Asynchronous on `stream` (default: torch's current stream)."""
-    B, ldv, ldz, S = _check_grad_shapes(vels, depths, nlayers, src_offset, src_depth,
-                                        {"timeP": timeP, "p": p, "w": w, "dtdr": dtdr, "dtdd": dtdd})
-    for name, t, shape in (("gvels", gvels, (B, ldv)), ("gdepths", gdepths, (B, ldz))):
-        if t is not None and tuple(t.shape) != shape:
-            raise ValueError(f"{name} must be {list(shape)}, got {list(t.shape)}")
-    if not vels.is_cuda:
-        raise ValueError("dff_grad_device needs CUDA tensors (there is no CPU path)")
-    dev = vels.device
-    _ensure_device(dev.index if dev.index is not None else torch.cuda.current_device())
+    (B, ldv, ldz, S), dev, args = _deriv_prologue(
+        "dff_grad_device", vels, depths, nlayers, src_offset, src_depth, timeP, p,
+        {"timeP": timeP, "p": p, "w": w, "dtdr": dtdr, "dtdd": dtdd},
+        lambda B, ldv, ldz, S: (("gvels", gvels, (B, ldv)), ("gdepths", gdepths, (B, ldz))))
     f64 = torch.float64
     if gvels is None:
         gvels = torch.empty((B, ldv), dtype=f64, device=dev)
@@ -112,10 +126,8 @@ def dff_grad_device(vels, depths, nlayers, src_offset, src_depth, timeP, p, w, g
     if want_src and dtdd is None:
         dtdd = torch.empty((B, S), dtype=f64, device=dev)
     rc = _lib.load().rtb200_dff_grad_device(
-        _ptr(vels, f64), _ptr(depths, f64) if ldz else None, _ptr(nlayers, torch.int32), B, ldv, ldz,
-        _ptr(src_offset, f64), _ptr(src_depth, f64), S, _ptr(timeP, f64), _ptr(p, f64), _ptr(w, f64),
-        _ptr(gvels, f64), _ptr(gdepths, f64) if ldz else None, _ptr(dtdr, f64), _ptr(dtdd, f64),
-        1 if kmode else 0, _stream_handle(stream, dev))
+        *args, _ptr(w, f64), _ptr(gvels, f64), _ptr(gdepths, f64) if ldz else None, _ptr(dtdr, f64),
+        _ptr(dtdd, f64), 1 if kmode else 0, _stream_handle(stream, dev))
     _lib.check(rc)
     return {"gvels": gvels, "gdepths": gdepths, "dtdr": dtdr, "dtdd": dtdd}
 
@@ -129,15 +141,10 @@ def dff_jac_device(vels, depths, nlayers, src_offset, src_depth, timeP, p, jvels
     jvels[b, s, i] = dT[b, s]/dV_i, jdepths[b, s, j] = dT[b, s]/dz_j (kmode: ziface), dtdr / dtdd
     as dff_grad_device returns them (want_src).  Asynchronous on `stream` (default: torch's
     current stream)."""
-    B, ldv, ldz, S = _check_grad_shapes(vels, depths, nlayers, src_offset, src_depth,
-                                        {"timeP": timeP, "p": p, "dtdr": dtdr, "dtdd": dtdd})
-    for name, t, shape in (("jvels", jvels, (B, S, ldv)), ("jdepths", jdepths, (B, S, ldz))):
-        if t is not None and tuple(t.shape) != shape:
-            raise ValueError(f"{name} must be {list(shape)}, got {list(t.shape)}")
-    if not vels.is_cuda:
-        raise ValueError("dff_jac_device needs CUDA tensors (there is no CPU path)")
-    dev = vels.device
-    _ensure_device(dev.index if dev.index is not None else torch.cuda.current_device())
+    (B, ldv, ldz, S), dev, args = _deriv_prologue(
+        "dff_jac_device", vels, depths, nlayers, src_offset, src_depth, timeP, p,
+        {"timeP": timeP, "p": p, "dtdr": dtdr, "dtdd": dtdd},
+        lambda B, ldv, ldz, S: (("jvels", jvels, (B, S, ldv)), ("jdepths", jdepths, (B, S, ldz))))
     f64 = torch.float64
     if jvels is None:
         jvels = torch.empty((B, S, ldv), dtype=f64, device=dev)
@@ -148,9 +155,7 @@ def dff_jac_device(vels, depths, nlayers, src_offset, src_depth, timeP, p, jvels
     if want_src and dtdd is None:
         dtdd = torch.empty((B, S), dtype=f64, device=dev)
     rc = _lib.load().rtb200_dff_jac_device(
-        _ptr(vels, f64), _ptr(depths, f64) if ldz else None, _ptr(nlayers, torch.int32), B, ldv, ldz,
-        _ptr(src_offset, f64), _ptr(src_depth, f64), S, _ptr(timeP, f64), _ptr(p, f64),
-        _ptr(jvels, f64), _ptr(jdepths, f64) if ldz else None, _ptr(dtdr, f64), _ptr(dtdd, f64),
+        *args, _ptr(jvels, f64), _ptr(jdepths, f64) if ldz else None, _ptr(dtdr, f64), _ptr(dtdd, f64),
         1 if kmode else 0, _stream_handle(stream, dev))
     _lib.check(rc)
     return {"jvels": jvels, "jdepths": jdepths, "dtdr": dtdr, "dtdd": dtdd}
@@ -165,28 +170,24 @@ def dff_normal_device(vels, depths, nlayers, src_offset, src_depth, timeP, p, to
     Returns {"JtJ" [B, P, P], "Jtr" [B, P] or None}, P = ldv + ldz: with J the rows dff_jac_device
     writes, [jvels | jdepths], JtJ = J^T J and, given tobs [NSrc], Jtr = J^T (tobs - timeP), each
     sum in source order.  Asynchronous on `stream` (default: torch's current stream)."""
-    B, ldv, ldz, S = _check_grad_shapes(vels, depths, nlayers, src_offset, src_depth,
-                                        {"timeP": timeP, "p": p})
-    P = ldv + ldz
-    if tobs is not None and tuple(tobs.shape) != (S,):
-        raise ValueError(f"tobs must be [NSrc] = [{S}], got {list(tobs.shape)}")
-    if Jtr is not None and tobs is None:
-        raise ValueError("Jtr needs tobs")
-    for name, t, shape in (("JtJ", JtJ, (B, P, P)), ("Jtr", Jtr, (B, P))):
-        if t is not None and tuple(t.shape) != shape:
-            raise ValueError(f"{name} must be {list(shape)}, got {list(t.shape)}")
-    if not vels.is_cuda:
-        raise ValueError("dff_normal_device needs CUDA tensors (there is no CPU path)")
-    dev = vels.device
-    _ensure_device(dev.index if dev.index is not None else torch.cuda.current_device())
+    def outputs(B, ldv, ldz, S):
+        if tobs is not None and tuple(tobs.shape) != (S,):
+            raise ValueError(f"tobs must be [NSrc] = [{S}], got {list(tobs.shape)}")
+        if Jtr is not None and tobs is None:
+            raise ValueError("Jtr needs tobs")
+        P = ldv + ldz
+        return ("JtJ", JtJ, (B, P, P)), ("Jtr", Jtr, (B, P))
+
+    (B, ldv, ldz, S), dev, args = _deriv_prologue(
+        "dff_normal_device", vels, depths, nlayers, src_offset, src_depth, timeP, p,
+        {"timeP": timeP, "p": p}, outputs)
     f64 = torch.float64
+    P = ldv + ldz
     if JtJ is None:
         JtJ = torch.empty((B, P, P), dtype=f64, device=dev)
     if tobs is not None and Jtr is None:
         Jtr = torch.empty((B, P), dtype=f64, device=dev)
     rc = _lib.load().rtb200_dff_normal_device(
-        _ptr(vels, f64), _ptr(depths, f64) if ldz else None, _ptr(nlayers, torch.int32), B, ldv, ldz,
-        _ptr(src_offset, f64), _ptr(src_depth, f64), S, _ptr(timeP, f64), _ptr(p, f64), _ptr(tobs, f64),
-        _ptr(JtJ, f64), _ptr(Jtr, f64), 1 if kmode else 0, _stream_handle(stream, dev))
+        *args, _ptr(tobs, f64), _ptr(JtJ, f64), _ptr(Jtr, f64), 1 if kmode else 0, _stream_handle(stream, dev))
     _lib.check(rc)
     return {"JtJ": JtJ, "Jtr": Jtr}

@@ -118,6 +118,16 @@ def travel_times(vels, depths, nlayers, src_offset, src_depth, kmode=False):
                               src_offset.contiguous(), src_depth.contiguous(), bool(kmode))
 
 
+def _forward_then(deriv, vels, depths, nlayers, src_offset, src_depth, kmode, **kw):
+    """The forward, then `deriv` (a device wrapper) at its timeP and p, without an autograd graph.
+    Returns {"timeP", "p"} and what deriv returns."""
+    with torch.no_grad():
+        args = tuple(t.detach().contiguous() for t in (vels, depths, nlayers, src_offset, src_depth))
+        out = device.dff_batch_device(*args, want_times=True, want_p=True, kmode=bool(kmode))
+        r = deriv(*args, out["timeP"], out["p"], kmode=bool(kmode), **kw)
+    return {"timeP": out["timeP"], "p": out["p"], **r}
+
+
 def jacobian(vels, depths, nlayers, src_offset, src_depth, kmode=False, want_src=True):
     """Travel times and their Jacobian per ray, without an autograd graph (DESIGN.md section 12).
 
@@ -126,11 +136,8 @@ def jacobian(vels, depths, nlayers, src_offset, src_depth, kmode=False, want_src
     jdepths[b, s, j] = dT[b, s]/dz_j, the rows whose sums over s travel_times' backward forms.
     timeP is dff_batch_device's, bit for bit."""
     _check(vels, depths, nlayers, src_offset, src_depth)
-    with torch.no_grad():
-        args = tuple(t.detach().contiguous() for t in (vels, depths, nlayers, src_offset, src_depth))
-        out = device.dff_batch_device(*args, want_times=True, want_p=True, kmode=bool(kmode))
-        r = device.dff_jac_device(*args, out["timeP"], out["p"], want_src=want_src, kmode=bool(kmode))
-    return {"timeP": out["timeP"], "p": out["p"], **r}
+    return _forward_then(device.dff_jac_device, vels, depths, nlayers, src_offset, src_depth, kmode,
+                         want_src=want_src)
 
 
 def normal_equations(vels, depths, nlayers, src_offset, src_depth, tobs=None, kmode=False):
@@ -144,13 +151,8 @@ def normal_equations(vels, depths, nlayers, src_offset, src_depth, tobs=None, km
     _, S = _check(vels, depths, nlayers, src_offset, src_depth)
     if tobs is not None and (tobs.dtype != torch.float64 or tuple(tobs.shape) != (S,)):
         raise ValueError(f"tobs must be a float64 [NSrc] = [{S}] tensor")
-    with torch.no_grad():
-        args = tuple(t.detach().contiguous() for t in (vels, depths, nlayers, src_offset, src_depth))
-        out = device.dff_batch_device(*args, want_times=True, want_p=True, kmode=bool(kmode))
-        r = device.dff_normal_device(*args, out["timeP"], out["p"],
-                                     tobs=None if tobs is None else tobs.detach().contiguous(),
-                                     kmode=bool(kmode))
-    return {"timeP": out["timeP"], "p": out["p"], **r}
+    return _forward_then(device.dff_normal_device, vels, depths, nlayers, src_offset, src_depth, kmode,
+                         tobs=None if tobs is None else tobs.detach().contiguous())
 
 
 def loglhood(vels, depths, nlayers, src_offset, src_depth, tobs, sigma, kmode=False):

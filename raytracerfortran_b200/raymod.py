@@ -107,14 +107,9 @@ def dff_batch(vels, depths, nlayers, src_offset, src_depth, tobs=None, sigma=Non
     return {"timeP": t, "p": p, "logL": ll}
 
 
-def dff_batch_grad(vels, depths, nlayers, src_offset, src_depth, w, want_times=False, want_p=False,
-                   want_src=False):
-    """dff_batch and the gradient of its travel times in one call (DESIGN.md section 11).
-
-    w [B, NSrc] weights the rays.  Returns a dict with "gvels" [B, ldv] = sum_s w dT/dV,
-    "gdepths" [B, ldz] = sum_s w dT/dz, and, on request, "timeP" / "p" [B, NSrc] of the forward
-    and "dtdr" / "dtdd" [B, NSrc], the per-ray derivatives with respect to the source offset and
-    depth (None otherwise)."""
+def _deriv_inputs(vels, depths, nlayers, src_offset, src_depth):
+    """The conversion and checks the derivative wrappers share.  Returns B, ldv, ldz, NSrc and the
+    C entries' first nine arguments (models, shapes, sources)."""
     v = _d(vels)
     z = _d(depths)
     if v.ndim != 2 or z.ndim != 2 or v.shape[0] != z.shape[0]:
@@ -128,6 +123,19 @@ def dff_batch_grad(vels, depths, nlayers, src_offset, src_depth, w, want_times=F
         raise ValueError("ldv must be 1..255 (at most 254 interfaces)")
     if B and (nl.min() < 0 or int(nl.max()) + 1 > ldv or int(nl.max()) > ldz):
         raise ValueError("nlayers exceeds the row length of vels / depths")
+    args = (_p(v), _p(z), nl.ctypes.data_as(_IP), _ci(B), _ci(ldv), _ci(ldz), _p(so), _p(sd), _ci(nsrc))
+    return B, ldv, ldz, nsrc, args
+
+
+def dff_batch_grad(vels, depths, nlayers, src_offset, src_depth, w, want_times=False, want_p=False,
+                   want_src=False):
+    """dff_batch and the gradient of its travel times in one call (DESIGN.md section 11).
+
+    w [B, NSrc] weights the rays.  Returns a dict with "gvels" [B, ldv] = sum_s w dT/dV,
+    "gdepths" [B, ldz] = sum_s w dT/dz, and, on request, "timeP" / "p" [B, NSrc] of the forward
+    and "dtdr" / "dtdd" [B, NSrc], the per-ray derivatives with respect to the source offset and
+    depth (None otherwise)."""
+    B, ldv, ldz, nsrc, args = _deriv_inputs(vels, depths, nlayers, src_offset, src_depth)
     ww = _d(w)
     if ww.shape != (B, nsrc):
         raise ValueError(f"w must be [B, NSrc] = [{B}, {nsrc}], got {list(ww.shape)}")
@@ -136,9 +144,7 @@ def dff_batch_grad(vels, depths, nlayers, src_offset, src_depth, w, want_times=F
     p = np.empty((B, nsrc)) if want_p else None
     dr = np.empty((B, nsrc)) if want_src else None
     dd = np.empty((B, nsrc)) if want_src else None
-    rc = _lib.load().dff_batch_grad(_p(v), _p(z), nl.ctypes.data_as(_IP), _ci(B), _ci(ldv), _ci(ldz),
-                                    _p(so), _p(sd), _ci(nsrc), _p(ww), _p(t), _p(p), _p(gv), _p(gz),
-                                    _p(dr), _p(dd))
+    rc = _lib.load().dff_batch_grad(*args, _p(ww), _p(t), _p(p), _p(gv), _p(gz), _p(dr), _p(dd))
     _lib.check(rc)
     return {"gvels": gv, "gdepths": gz, "timeP": t, "p": p, "dtdr": dr, "dtdd": dd}
 
@@ -150,27 +156,13 @@ def dff_batch_jac(vels, depths, nlayers, src_offset, src_depth, want_times=False
     Returns a dict with "jvels" [B, NSrc, ldv] = dT/dV and "jdepths" [B, NSrc, ldz] = dT/dz per
     ray, and, on request, "timeP" / "p" [B, NSrc] of the forward and "dtdr" / "dtdd" [B, NSrc],
     the per-ray derivatives with respect to the source offset and depth (None otherwise)."""
-    v = _d(vels)
-    z = _d(depths)
-    if v.ndim != 2 or z.ndim != 2 or v.shape[0] != z.shape[0]:
-        raise ValueError("vels and depths must be [B, ldv] and [B, ldz]")
-    nl = np.ascontiguousarray(nlayers, dtype=np.int32)
-    so, sd = _d(src_offset), _d(src_depth)
-    B, ldv, ldz, nsrc = v.shape[0], v.shape[1], z.shape[1], so.size
-    if nl.shape != (B,) or so.ndim != 1 or sd.shape != so.shape:
-        raise ValueError("nlayers must be [B], src_offset and src_depth [NSrc]")
-    if not 1 <= ldv <= 255:
-        raise ValueError("ldv must be 1..255 (at most 254 interfaces)")
-    if B and (nl.min() < 0 or int(nl.max()) + 1 > ldv or int(nl.max()) > ldz):
-        raise ValueError("nlayers exceeds the row length of vels / depths")
+    B, ldv, ldz, nsrc, args = _deriv_inputs(vels, depths, nlayers, src_offset, src_depth)
     jv, jz = np.empty((B, nsrc, ldv)), np.empty((B, nsrc, ldz))
     t = np.empty((B, nsrc)) if want_times else None
     p = np.empty((B, nsrc)) if want_p else None
     dr = np.empty((B, nsrc)) if want_src else None
     dd = np.empty((B, nsrc)) if want_src else None
-    rc = _lib.load().dff_batch_jac(_p(v), _p(z), nl.ctypes.data_as(_IP), _ci(B), _ci(ldv), _ci(ldz),
-                                   _p(so), _p(sd), _ci(nsrc), _p(t), _p(p), _p(jv), _p(jz), _p(dr),
-                                   _p(dd))
+    rc = _lib.load().dff_batch_jac(*args, _p(t), _p(p), _p(jv), _p(jz), _p(dr), _p(dd))
     _lib.check(rc)
     return {"jvels": jv, "jdepths": jz, "timeP": t, "p": p, "dtdr": dr, "dtdd": dd}
 
@@ -183,29 +175,16 @@ def dff_batch_normal(vels, depths, nlayers, src_offset, src_depth, tobs=None, wa
     Returns a dict with "JtJ" [B, P, P] = J^T J, P = ldv + ldz, over the rows dff_batch_jac
     returns ([jvels | jdepths]), "Jtr" [B, P] = J^T (tobs - timeP) when tobs [NSrc] is given, and,
     on request, "timeP" / "p" [B, NSrc] of the forward (None otherwise)."""
-    v = _d(vels)
-    z = _d(depths)
-    if v.ndim != 2 or z.ndim != 2 or v.shape[0] != z.shape[0]:
-        raise ValueError("vels and depths must be [B, ldv] and [B, ldz]")
-    nl = np.ascontiguousarray(nlayers, dtype=np.int32)
-    so, sd = _d(src_offset), _d(src_depth)
-    B, ldv, ldz, nsrc = v.shape[0], v.shape[1], z.shape[1], so.size
-    if nl.shape != (B,) or so.ndim != 1 or sd.shape != so.shape:
-        raise ValueError("nlayers must be [B], src_offset and src_depth [NSrc]")
+    B, ldv, ldz, nsrc, args = _deriv_inputs(vels, depths, nlayers, src_offset, src_depth)
     to = None if tobs is None else _d(tobs)
-    if to is not None and to.shape != so.shape:
+    if to is not None and to.shape != (nsrc,):
         raise ValueError("tobs must be [NSrc]")
-    if not 1 <= ldv <= 255:
-        raise ValueError("ldv must be 1..255 (at most 254 interfaces)")
-    if B and (nl.min() < 0 or int(nl.max()) + 1 > ldv or int(nl.max()) > ldz):
-        raise ValueError("nlayers exceeds the row length of vels / depths")
     P = ldv + ldz
     jtj = np.empty((B, P, P))
     jtr = np.empty((B, P)) if to is not None else None
     t = np.empty((B, nsrc)) if want_times else None
     p = np.empty((B, nsrc)) if want_p else None
-    rc = _lib.load().dff_batch_normal(_p(v), _p(z), nl.ctypes.data_as(_IP), _ci(B), _ci(ldv), _ci(ldz),
-                                      _p(so), _p(sd), _ci(nsrc), _p(to), _p(t), _p(p), _p(jtj), _p(jtr))
+    rc = _lib.load().dff_batch_normal(*args, _p(to), _p(t), _p(p), _p(jtj), _p(jtr))
     _lib.check(rc)
     return {"JtJ": jtj, "Jtr": jtr, "timeP": t, "p": p}
 
