@@ -793,7 +793,8 @@ void orc_sd_step_batch(const int *k, const double *voro, double *logL, double *s
  * idxarRT == 0: birth (arparRT uniform over [minlimarRT, maxlimarRT], logarp = LOG(0.5));
  * else ran_uni_ar >= 0.5: death (idxarRT = 0, arparRT = minlimarRT - 1, logarp = LOG(2)),
  * otherwise perturb (arparRT + pertarsdRT*gauss, logarp = 0).  LOGLHOOD with the AR model of
- * loglhood.f90:171-182; reject iff ran_uni >= EXP(logarp + (logL_new - logL)*beta_mh).
+ * loglhood.f90:171-182 (LOGLHOOD2's constant 1 under ISMPPRIOR = 1, as for the other moves);
+ * reject iff ran_uni >= EXP(logarp + (logL_new - logL)*beta_mh).
  * ar_prior = { pertarsdRT, minlimarRT, maxlimarRT, armxRT }.  Returns 1 / 0 / -1 outside.     */
 int orc_ar_step(int k, const double *node_depth, const double *node_vp, double *logL, double sigma,
                 int *idxar, double *arpar, double u_choice, double u_prop, double gauss,
@@ -820,10 +821,13 @@ int orc_ar_step(int k, const double *node_depth, const double *node_vp, double *
         if ((ar_new - amin) < 0.0 || (amax - ar_new) < 0.0) outside = 1;
     }
     if (outside) return -1;                                      /* :621-625 */
-    double *pred = (double *)malloc(sizeof(double) * (size_t)(nsrc > 0 ? nsrc : 1));
-    orc_loglhood_rt(k, node_vp, node_depth + 1, src_offset, src_depth, nsrc, tobs, sigma, pred);
-    const double ll = orc_loglhood_from_times_ar(pred, tobs, nsrc, sigma, idx_new, ar_new, armx);
-    free(pred);
+    double ll = 1.0;                                             /* ISMPPRIOR = 1: LOGLHOOD2 */
+    if (!g_ismpprior) {
+        double *pred = (double *)malloc(sizeof(double) * (size_t)(nsrc > 0 ? nsrc : 1));
+        orc_loglhood_rt(k, node_vp, node_depth + 1, src_offset, src_depth, nsrc, tobs, sigma, pred);
+        ll = orc_loglhood_from_times_ar(pred, tobs, nsrc, sigma, idx_new, ar_new, armx);
+        free(pred);
+    }
     if (logL_prop) *logL_prop = ll;
     const double logPLratio = logarp + (ll - *logL) * beta;      /* :611 */
     if (u_acc >= exp(logPLratio)) return 0;                      /* :613-615 */
