@@ -143,6 +143,15 @@ int dff_batch_normal(const double *vels, const double *depths, const int *nlayer
                      const double *src_depth, const int *NSrc, const double *tobs, double *timeP,
                      double *p_out, double *JtJ, double *Jtr);
 
+/* dff_batch and the weighted second derivatives of its travel times in one call (host pointers,
+ * scalars by reference): the forward, then rtb200_dff_hess_device with weights w [B][NSrc].
+ * H [B][P][P], P = ldv + ldz; timeP and p_out [B][NSrc] may each be NULL.  No kmode.  Returns 0,
+ * or a non-zero status (see rtb200_last_error()). */
+int dff_batch_hess(const double *vels, const double *depths, const int *nlayers, const int *B,
+                   const int *ldv, const int *ldz, const double *src_offset,
+                   const double *src_depth, const int *NSrc, const double *w, double *timeP,
+                   double *p_out, double *H);
+
 /* LOGLHOOD / LOGLHOOD_RT (loglhood.f90:3-32,35-211) over B chain states, with the model
  * mapping of :127-146: state b has k[b] Voronoi nodes, vp[b][0..k-1] = voro(1:k,2),
  * ziface[b][0..k-2] = ziface(1:k-1); k == 1 becomes two equal velocities over one fake
@@ -250,6 +259,25 @@ int rtb200_dff_normal_device(const double *d_vels, const double *d_depths, const
                              const double *d_src_depth, int NSrc, const double *d_timeP,
                              const double *d_p, const double *d_tobs, double *d_JtJ,
                              double *d_Jtr, int kmode, void *stream);
+
+/* Second derivatives of the travel times with respect to the layered model, weighted and summed
+ * per model (DESIGN.md section 14).  Inputs as for rtb200_dff_grad_device (w [B][NSrc] the
+ * weights), without the source derivatives.  With P = ldv + ldz columns as in
+ * rtb200_dff_normal_device:
+ *   H  [B][P][P]  sum_s w[b][s] d2T_bs / dtheta_i dtheta_j
+ * taken at the forward's p with the implicit function theorem: for a ray of n >= 2 layers
+ * d2T = D + u u^T / X'(p), u = dX/dtheta, X'(p) = sum_i H_i V_i / cos_i^3, D the band of
+ * d2(p R + sum_i H_i cos_i / V_i) at fixed p; a top-layer ray has 2 T / V_0^2 at (0, 0) alone.  The
+ * sum over s, the terms a ray reaches, the zero rows and columns and kmode are as in
+ * rtb200_dff_normal_device, so H is exactly symmetric and reproducible bit for bit.  The exact
+ * Newton matrix of (1/2) |tobs - T|^2 is JtJ - H with w = tobs - timeP.  NSrc = 0 gives zeros;
+ * the source arrays, timeP, p and w may then be NULL.  Stream semantics of
+ * rtb200_dff_batch_device. */
+int rtb200_dff_hess_device(const double *d_vels, const double *d_depths, const int *d_nlayers,
+                           int B, int ldv, int ldz, const double *d_src_offset,
+                           const double *d_src_depth, int NSrc, const double *d_timeP,
+                           const double *d_p, const double *d_w, double *d_H, int kmode,
+                           void *stream);
 
 /* One fixed-dimension Metropolis-Hastings move of B independent chains, entirely on the device:
  * PROPOSAL (prjmh_temper_rf.f90:1386-1447, ENOS = 0: Cauchy step on voro(ivo,iwhich), |.| for a

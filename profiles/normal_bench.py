@@ -113,7 +113,8 @@ def main():
         e["jac_route_within_bound"] = bool(ok.all().item() and ok2.all().item())
         del Ja, ok, ok2, ra
         jv, jz = Jc[:, :, :ldv].contiguous(), Jc[:, :, ldv:].contiguous()
-        del Jc, R
+        del Jc
+        R.clear()           # jac_route_timed fills it again: deleting the name would unbind jac_route's R
         torch.cuda.empty_cache()
 
         def jac():

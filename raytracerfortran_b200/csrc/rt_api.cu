@@ -76,6 +76,7 @@ struct Ctx {
         idxar, arparb, sched, mh_ll, mh_out, mh_kp, mh_lpr,
         // the derivative entries': the gradient's weights; the derivatives with respect to the
         // model (the gradient's sums, the Jacobian's rows) and to the sources; the normal equations
+        // (JtJ also holds the second derivatives' H)
         w, dvels, ddepths, dtdr, dtdd, JtJ, Jtr;
     // The scratch buffers above (vels ... Jtr) are shared by every entry.  Entries that return
     // without synchronising (a caller stream was given) leave an event behind; any later entry that
@@ -1166,6 +1167,17 @@ int check_normal_args(int ldv, int ldz, int nsrc, const void *vels, const void *
     return 0;
 }
 
+// The argument checks both second-derivative entries share; timeP and p are checked by the
+// device entry, whose inputs they are.
+int check_hess_args(int ldv, int nsrc, const void *vels, const void *nlayers, const void *off,
+                    const void *dep, const void *w, const void *H) {
+    if (int rc = check_ldv(ldv)) return rc;
+    if (!vels || !nlayers || !H) return fail("the second derivatives need vels, nlayers and H");
+    // empty source arrays may arrive as NULL: with no source there is nothing to read
+    if (nsrc > 0 && (!off || !dep || !w)) return fail("the second derivatives need src_offset, src_depth and w");
+    return 0;
+}
+
 }  // namespace
 }  // extern "C++"
 
@@ -1359,6 +1371,67 @@ int dff_batch_normal(const double *vels, const double *depths, const int *nlayer
     g.launches++;
     CK(cudaMemcpyAsync(JtJ, g.JtJ.p, Bz * P * P * 8, cudaMemcpyDeviceToHost, st));
     if (tobs) CK(cudaMemcpyAsync(Jtr, g.Jtr.p, Bz * P * 8, cudaMemcpyDeviceToHost, st));
+    return host_finish(d, timeP, p_out);
+}
+
+int rtb200_dff_hess_device(const double *d_vels, const double *d_depths, const int *d_nlayers,
+                           int B, int ldv, int ldz, const double *d_src_offset,
+                           const double *d_src_depth, int NSrc, const double *d_timeP,
+                           const double *d_p, const double *d_w, double *d_H, int kmode,
+                           void *stream) {
+    ApiLock api_lock_;
+    if (int rc = ensure_init()) return rc;
+    g.err.clear();
+    if (B <= 0) return 0;
+    ldz = std::max(ldz, 0);
+    if (int rc = check_hess_args(ldv, NSrc, d_vels, d_nlayers, d_src_offset, d_src_depth, d_w, d_H))
+        return rc;
+    if (int rc = check_forward("the second derivatives need", NSrc, d_timeP, d_p)) return rc;
+    const size_t P = (size_t)(ldv + ldz);
+    const rtb::HessArgs a{deriv_args(d_vels, d_depths, d_nlayers, B, ldv, ldz, d_src_offset, d_src_depth,
+                                     NSrc, d_timeP, d_p, kmode),
+                          d_w, d_H};
+    return device_launch(stream, [&](cudaStream_t st) {
+        if (NSrc <= 0) {        // sums over no source
+            CK(cudaMemsetAsync(d_H, 0, (size_t)B * P * P * 8, st));
+        } else {
+            CK(rtb::launch_hess(a, st));
+            g.launches++;
+        }
+        return 0;
+    });
+}
+
+int dff_batch_hess(const double *vels, const double *depths, const int *nlayers, const int *B,
+                   const int *ldv, const int *ldz, const double *src_offset,
+                   const double *src_depth, const int *NSrc, const double *w, double *timeP,
+                   double *p_out, double *H) {
+    ApiLock api_lock_;
+    if (int rc = ensure_init()) return rc;
+    g.err.clear();
+    g.kernel_ms = g.total_ms = 0.0;
+    const int nb = *B, lv = *ldv, lz = std::max(*ldz, 0), ns = *NSrc;
+    if (nb <= 0) return 0;
+    if (int rc = check_hess_args(lv, ns, vels, nlayers, src_offset, src_depth, w, H)) return rc;
+    const size_t Bz = (size_t)nb, P = (size_t)(lv + lz);
+    if (ns <= 0) {              // sums over no source
+        std::memset(H, 0, Bz * P * P * 8);
+        return 0;
+    }
+    // copy in, forward, second derivatives, copy out (H in the normal equations' scratch)
+    const size_t S = (size_t)ns;
+    CK(g.JtJ.reserve(Bz * P * P * 8));
+    CK(g.w.reserve(Bz * S * 8));
+    rtb::DerivArgs d;
+    if (int rc = host_forward(vels, depths, nlayers, nb, lv, lz, src_offset, src_depth, ns, g.w.p, w,
+                              Bz * S * 8, d))
+        return rc;
+    cudaStream_t st = g.s_comp;
+    const rtb::HessArgs ha{d, g.w.as<double>(), g.JtJ.as<double>()};
+    CK(rtb::launch_hess(ha, st));
+    CK(cudaEventRecord(g.ev_k1[0], st));
+    g.launches++;
+    CK(cudaMemcpyAsync(H, g.JtJ.p, Bz * P * P * 8, cudaMemcpyDeviceToHost, st));
     return host_finish(d, timeP, p_out);
 }
 

@@ -44,7 +44,7 @@ struct BatchArgs {
 
 // What every derivative kernel reads: the models and sources of a batch-kernel launch and what it
 // returned.  Every pointer is a device pointer; model and source arrays as in BatchArgs.  It is
-// the base of GradArgs, JacArgs and NormalArgs, so their fields keep the offsets they would have
+// the base of GradArgs, JacArgs, NormalArgs and HessArgs, so their fields keep the offsets they would have
 // if each declared these itself.
 struct DerivArgs {
     const double *vels;        // [B][ldv]
@@ -84,6 +84,13 @@ struct NormalArgs : DerivArgs {
     const double *tobs;        // [nsrc] or null (then Jtr is null)
     double       *JtJ;         // [B][P][P]
     double       *Jtr;         // [B][P] or null
+};
+
+// One launch of the second-derivative kernel (DESIGN.md section 14).  P = ldv + ldz parameter
+// columns, [vels | depths].
+struct HessArgs : DerivArgs {
+    const double *w;           // [B][nsrc] weights of the rays
+    double       *H;           // [B][P][P]  sum_s w_s d2T_s
 };
 
 // Tile geometry chosen by the host for one launch.
@@ -157,6 +164,7 @@ cudaError_t launch_batch(const BatchArgs &a, const TileCfg &c, cudaStream_t st);
 cudaError_t launch_grad(const GradArgs &a, cudaStream_t st);
 cudaError_t launch_jac(const JacArgs &a, cudaStream_t st);
 cudaError_t launch_normal(const NormalArgs &a, cudaStream_t st);
+cudaError_t launch_hess(const HessArgs &a, cudaStream_t st);
 cudaError_t launch_prep_voro(const int *k, const double *voro, int B, int ldk, double *vels,
                              double *depths, double *sorted, cudaStream_t st);
 cudaError_t launch_propose_voro(const int *k, const double *voro, int B, int ldk, const int *ivo,

@@ -2,7 +2,8 @@
 
 torch is used for device memory and streams only; the work is done by the sm_100a kernels in
 libraytrace_b200.so through rtb200_dff_batch_device and, for derivatives, rtb200_dff_grad_device,
-rtb200_dff_jac_device and rtb200_dff_normal_device (include/raytrace_b200.h).
+rtb200_dff_jac_device, rtb200_dff_normal_device and rtb200_dff_hess_device
+(include/raytrace_b200.h).
 """
 import torch
 
@@ -191,3 +192,28 @@ def dff_normal_device(vels, depths, nlayers, src_offset, src_depth, timeP, p, to
         *args, _ptr(tobs, f64), _ptr(JtJ, f64), _ptr(Jtr, f64), 1 if kmode else 0, _stream_handle(stream, dev))
     _lib.check(rc)
     return {"JtJ": JtJ, "Jtr": Jtr}
+
+
+def dff_hess_device(vels, depths, nlayers, src_offset, src_depth, timeP, p, w, H=None, kmode=False,
+                    stream=None):
+    """Weighted second derivatives of the travel times dff_batch_device returned (timeP, p
+    [B, NSrc]), per model, on the GPU (rtb200_dff_hess_device; DESIGN.md section 14).
+
+    Returns {"H" [B, P, P]}, P = ldv + ldz: H[b] = sum_s w[b, s] d2T[b, s] / dtheta dtheta^T over the
+    columns [vels | depths] of dff_normal_device, each sum in source order; exactly symmetric.
+    Asynchronous on `stream` (default: torch's current stream)."""
+    def outputs(B, ldv, ldz, S):
+        P = ldv + ldz
+        return (("H", H, (B, P, P)),)
+
+    (B, ldv, ldz, S), dev, args = _deriv_prologue(
+        "dff_hess_device", vels, depths, nlayers, src_offset, src_depth, timeP, p,
+        {"timeP": timeP, "p": p, "w": w}, outputs)
+    f64 = torch.float64
+    P = ldv + ldz
+    if H is None:
+        H = torch.empty((B, P, P), dtype=f64, device=dev)
+    rc = _lib.load().rtb200_dff_hess_device(
+        *args, _ptr(w, f64), _ptr(H, f64), 1 if kmode else 0, _stream_handle(stream, dev))
+    _lib.check(rc)
+    return {"H": H}

@@ -19,6 +19,15 @@ Gauss-Newton and linearised-uncertainty computations need.
 
 returns the travel times with the per-model normal equations J^T J and J^T (tobs - T) of those
 rows (rtb200_dff_normal_device), accumulated on the device without writing J.
+
+    S = hessian(vels, depths, nlayers, src_offset, src_depth, w, kmode=False)
+    A = newton_equations(vels, depths, nlayers, src_offset, src_depth, tobs, kmode=False)
+
+hessian returns the travel times with the weighted second derivatives sum_s w_s d2T_s, per model
+(rtb200_dff_hess_device); newton_equations adds them to the normal equations as the exact Newton
+matrix A = J^T J - sum_s (tobs_s - T_s) d2T_s of (1/2) |tobs - T|^2.  Like jacobian and
+normal_equations, both return plain tensors without an autograd graph; solving with them is the
+caller's business.
 """
 import torch
 from torch.autograd.function import once_differentiable
@@ -153,6 +162,42 @@ def normal_equations(vels, depths, nlayers, src_offset, src_depth, tobs=None, km
         raise ValueError(f"tobs must be a float64 [NSrc] = [{S}] tensor")
     return _forward_then(device.dff_normal_device, vels, depths, nlayers, src_offset, src_depth, kmode,
                          tobs=None if tobs is None else tobs.detach().contiguous())
+
+
+def hessian(vels, depths, nlayers, src_offset, src_depth, w, kmode=False):
+    """Travel times and their weighted second derivatives, per model, without an autograd graph
+    (DESIGN.md section 14).
+
+    Returns {"timeP", "p" [B, NSrc], "H" [B, P, P]}, P = ldv + ldz: H[b] = sum_s w[b, s]
+    d2T[b, s] / dtheta dtheta^T over the columns normal_equations uses, at the forward's p,
+    exactly symmetric.  w is [B, NSrc] float64.  timeP is dff_batch_device's, bit for bit."""
+    B, S = _check(vels, depths, nlayers, src_offset, src_depth)
+    if w.dtype != torch.float64 or tuple(w.shape) != (B, S):
+        raise ValueError(f"w must be a float64 [B, NSrc] = [{B}, {S}] tensor")
+    return _forward_then(device.dff_hess_device, vels, depths, nlayers, src_offset, src_depth, kmode,
+                         w=w.detach().contiguous())
+
+
+def newton_equations(vels, depths, nlayers, src_offset, src_depth, tobs, kmode=False):
+    """Travel times, the Gauss-Newton normal equations and the exact Newton matrix of
+    (1/2) |tobs - T|^2, per model, without an autograd graph (DESIGN.md section 14).
+
+    Returns {"timeP", "p" [B, NSrc], "JtJ" [B, P, P], "Jtr" [B, P], "A" [B, P, P]}: one forward,
+    JtJ and Jtr as normal_equations returns them, and A = JtJ - H with H the second derivatives
+    weighted by the residuals r = tobs - timeP, one rounded subtract an entry.  A is exactly
+    symmetric; it need not be positive definite."""
+    _, S = _check(vels, depths, nlayers, src_offset, src_depth)
+    if tobs.dtype != torch.float64 or tuple(tobs.shape) != (S,):
+        raise ValueError(f"tobs must be a float64 [NSrc] = [{S}] tensor")
+    with torch.no_grad():
+        tobs = tobs.detach().contiguous()
+        args = tuple(t.detach().contiguous() for t in (vels, depths, nlayers, src_offset, src_depth))
+        out = device.dff_batch_device(*args, want_times=True, want_p=True, kmode=bool(kmode))
+        T, p = out["timeP"], out["p"]
+        N = device.dff_normal_device(*args, T, p, tobs=tobs, kmode=bool(kmode))
+        H = device.dff_hess_device(*args, T, p, (tobs[None, :] - T).contiguous(), kmode=bool(kmode))["H"]
+        A = N["JtJ"] - H
+    return {"timeP": T, "p": p, "JtJ": N["JtJ"], "Jtr": N["Jtr"], "A": A}
 
 
 def loglhood(vels, depths, nlayers, src_offset, src_depth, tobs, sigma, kmode=False):

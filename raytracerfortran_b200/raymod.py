@@ -189,6 +189,26 @@ def dff_batch_normal(vels, depths, nlayers, src_offset, src_depth, tobs=None, wa
     return {"JtJ": jtj, "Jtr": jtr, "timeP": t, "p": p}
 
 
+def dff_batch_hess(vels, depths, nlayers, src_offset, src_depth, w, want_times=False, want_p=False):
+    """dff_batch and the weighted second derivatives of its travel times in one call (DESIGN.md
+    section 14).
+
+    w [B, NSrc] weights the rays.  Returns a dict with "H" [B, P, P] = sum_s w d2T/dtheta^2,
+    P = ldv + ldz, over the columns dff_batch_normal uses, and, on request, "timeP" / "p"
+    [B, NSrc] of the forward (None otherwise)."""
+    B, ldv, ldz, nsrc, args = _deriv_inputs(vels, depths, nlayers, src_offset, src_depth)
+    ww = _d(w)
+    if ww.shape != (B, nsrc):
+        raise ValueError(f"w must be [B, NSrc] = [{B}, {nsrc}], got {list(ww.shape)}")
+    P = ldv + ldz
+    h = np.empty((B, P, P))
+    t = np.empty((B, nsrc)) if want_times else None
+    p = np.empty((B, nsrc)) if want_p else None
+    rc = _lib.load().dff_batch_hess(*args, _p(ww), _p(t), _p(p), _p(h))
+    _lib.check(rc)
+    return {"H": h, "timeP": t, "p": p}
+
+
 def loglhood_batch(k, voro_vp, ziface, src_offset, src_depth, DobsRT, sdparRT, want_pred=False):
     """LOGLHOOD / LOGLHOOD_RT (loglhood.f90:3-32,35-211) over B chain states.
 
